@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the DyrosDynamicWalk hot path (BASELINE.json metric, configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs 4096] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs 4096] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -74,7 +74,14 @@ def parse():
     ap.add_argument("--ppo-dtype", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--grad-sync", default="peer", choices=["peer", "peer2", "nccl"],
                     help="PPO gradient exchange at N > 1: sum over peer-mapped buffers inside the optimiser's kernels, or one NCCL all-reduce")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed env step returned to rank 0 (obs, rew, reset, "
+                         "time_outs, stacked_rewards) as DIR/<name>.npy, float32 / float64; beyond 64 MiB a fixed, seeded "
+                         "sample of envs (DIR/env_index.npy). The inputs are the same on every run with the same arguments.")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "env"):
+        ap.error("--dump-outputs writes the outputs of the env-step path (--impl ours --workload env)")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -153,6 +160,37 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": max(mx), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+# ------------------------------------------------------------------------------------------------ outputs
+DUMP_BYTES = 64 << 20
+
+
+def step_outputs(out, seed=0):
+    """What DyrosDynamicWalk.step returned, as host arrays (float32; integer buffers as float64, exactly). The env's own
+    buffers, overwritten by the next step: call this before that. If the arrays exceed DUMP_BYTES, the rows of a fixed,
+    seeded sample of envs; `env_index` lists which."""
+    import numpy as np
+    obs, rew, reset, extras = out
+    arrays = {"obs": obs["obs"], "rew": rew, "reset": reset, "time_outs": extras["time_outs"],
+              "stacked_rewards": extras["stacked_rewards"]}
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float64 if v.dtype.kind in "biu" else np.float32) for k, v in arrays.items()}
+    n = len(arrays["rew"])
+    row_bytes = 8 + sum(v.nbytes for v in arrays.values()) // n
+    keep = np.arange(n)
+    if n * row_bytes > DUMP_BYTES - (1 << 16):  # (room for the .npy headers)
+        keep = np.sort(np.random.default_rng(seed).choice(n, (DUMP_BYTES - (1 << 16)) // row_bytes, replace=False))
+    arrays = {k: v[keep] for k, v in arrays.items()}
+    arrays["env_index"] = keep.astype(np.float64)
+    return arrays
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------ CPU oracle port
@@ -269,7 +307,7 @@ def run_ours(a):
     def device_step(i):
         # the public call; the action tensors are resident in HBM and the step's first kernel reads them in place (one
         # CUDA graph per action tensor, captured the second time `step` sees it)
-        env.step(pool[i % len(pool)])
+        return env.step(pool[i % len(pool)])
 
     for i in range(2 * len(pool)):  # every pool entry seen twice: all graphs captured before the warm-up
         device_step(i)
@@ -284,11 +322,12 @@ def run_ours(a):
         for i in range(K):
             env.core.flush_l2(flush, i)
             ev[i][0].record()
-            device_step(W + i)
+            out = device_step(W + i)
             ev[i][1].record()
         barrier()
         t_wall_flush = time.perf_counter() - t_wall0
         cold_ms = sum(s.elapsed_time(e) for s, e in ev)
+        last_outputs = step_outputs(out) if a.dump_outputs and rank == 0 else None
         # ---- (2) back to back (state L2-resident, as in the real rollout loop)
         s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
@@ -467,6 +506,8 @@ def run_ours(a):
         }
         if world == 1 and not a.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(a.cpu_seconds)
+        if last_outputs is not None:
+            write_outputs(a.dump_outputs, last_outputs)
         emit(line)
     if world > 1:
         dist.barrier()

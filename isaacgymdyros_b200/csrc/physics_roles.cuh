@@ -39,6 +39,8 @@ constexpr int LS_SC = 48;  // 4  [qd -> qd*, tau -> u, damping -> 1/D, armature 
 constexpr int LS_Q = 52;   // 1  joint angle
 constexpr int LS = 53;
 constexpr int LS_S = LS_E, LS_R = LS_E + 3;
+constexpr int LS_WP = LS_E + 6;  // 3  from pass 1b on: the parent's angular velocity (pass 3 of a link whose parent is
+                                 //    not the role's previous link: the parent's LS_V may hold dv by then)
 constexpr int A_POSE = 6, A_CIA = 0, A_CPA = 21, A_ACC = 0, A_OM0 = 6, A_ROWS = 6, A_G = 21;
 constexpr int ROWS_PER_LINK = 2;  // contact rows (7 floats each) parked in one leg-chain link's block
 // per-env extra scratch
@@ -291,6 +293,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
       pw_prev = ld3(Lp + LS_A + A_POSE + 9);
     }
     M3 E = ld_m3(L + LS_E);
+    if (k == 0 || par != prev) st3(L + LS_WP, v_prev.w);  // (pass 3 starts its chains where this pass does, and at k = 0)
     const V3 rw = mul(Rw_prev, ld3_f(R + R_R));  // offset of this link's origin from its parent's, world axes
     Rw_prev = mulABt(Rw_prev, E);
     const V3 sw = mul(Rw_prev, ld3_f(R + R_AXIS));  // joint axis, world axes
@@ -499,7 +502,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
     real* L = BLK(i);
     if (par != prev) {
       a_prev = ld6(BLK(par) + LS_A + A_ACC);
-      w_prev = ld3(BLK(par) + LS_V);
+      w_prev = ld3(L + LS_WP);
     }
     const V3 sw = ld3(L + LS_S), rw = ld3(L + LS_R);
     real qd = L[LS_SC];

@@ -4,6 +4,7 @@
 // and its dataflow synchronisation with the dense fp64 oracle (oracle/physics_oracle.py) without a GPU.
 // Never linked into the product.
 #include <barrier>
+#include <chrono>
 #include <thread>
 #include <vector>
 
@@ -15,8 +16,20 @@ void set_error(const char*, ...) {}
 }  // namespace dyros
 using namespace dyros;
 
+// One role held back at one stage marker (sync.mark) of every sub-step: the result must not depend on how far the
+// other roles get meanwhile, i.e. on anything but the stage flags.
+static int g_hold_role = -1, g_hold_mark = -1, g_hold_us = 0;
+extern "C" void dyros_hostemu_hold_role(int role, int mark, int microseconds) {
+  g_hold_role = role;
+  g_hold_mark = mark;
+  g_hold_us = microseconds;
+}
+
 struct HostRoleSync {
-  void mark(int) const {}
+  int role;
+  void mark(int id) const {
+    if (role == g_hold_role && id == g_hold_mark) std::this_thread::sleep_for(std::chrono::microseconds(g_hold_us));
+  }
   void signal(int* f, int v) const { __atomic_store_n(f, v, __ATOMIC_RELEASE); }
   void wait(const int* f, int v) const {
     while (__atomic_load_n(f, __ATOMIC_ACQUIRE) < v) std::this_thread::yield();
@@ -62,7 +75,7 @@ extern "C" int dyros_hostemu_simulate(const DyrosSimDesc* d, const DyrosModelDes
     for (int role = 0; role < DYROS_LANES; ++role)
       th.emplace_back([&, role]() {
         EnvIO mine = io;
-        HostRoleSync sync;
+        HostRoleSync sync{role};
         for (int s = 0; s < p.substeps; ++s) {
           env_stage_inputs(mine, scratch.data(), hot, m, p, role, DYROS_LANES);
           bar.arrive_and_wait();

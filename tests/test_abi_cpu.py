@@ -60,12 +60,10 @@ int main(void){printf("%zu %zu %zu %zu %zu %zu\n", sizeof(DyrosModelDesc), sizeo
 
 
 def test_core_refuses_to_run_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from isaacgymdyros_b200.core import DyrosCore
-    with pytest.raises(native.DyrosError):
-        DyrosCore(4)
+    """In a child process with every CUDA device hidden, so that it runs on GPU machines too."""
+    code = ("import pytest\nfrom isaacgymdyros_b200 import native\nfrom isaacgymdyros_b200.core import DyrosCore\n"
+            "with pytest.raises(native.DyrosError):\n    DyrosCore(4)\n")
+    subprocess.run([sys.executable, "-c", code], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""}, check=True)
 
 
 def test_header_is_plain_c(tmp_path):

@@ -87,6 +87,33 @@ def test_humanoid_lane_program_matches_dense_oracle(kind, seed, program):
         assert (want[3][:, feet, 2] > 0).any()
 
 
+def test_role_program_does_not_depend_on_role_timing():
+    """The roles exchange results through the env's scratch block, ordered by stage flags only. Holding any one role back
+    at any stage marker of physics_roles.cuh lets the others run ahead as far as the flags allow; the result must stay
+    bit for bit the same. (The Humanoid's arms hang off the base while its feet hang off the pelvis: no foot waits for
+    an arm's pass 3, so an arm may run its pass 3 after the base response has overwritten the base's velocity.)"""
+    import ctypes as C
+    from tests.golden_util import load_assets
+    from tests.physics_util import hostemu, random_states
+    t, tocabi = humanoid(), load_assets()[0]
+    cases = [(t, CoreConfig(**HUMANOID_CFG), humanoid_states(2, np.random.default_rng(0), t, "air")),
+             (t, CoreConfig(**HUMANOID_CFG), humanoid_states(2, np.random.default_rng(1), t, "stand")),
+             (tocabi, CoreConfig(), random_states(2, np.random.default_rng(2), tocabi, "mixed"))]
+    hold = hostemu().dyros_hostemu_hold_role
+    try:
+        for tab, cfg, st in cases:
+            free = emulate_substep(tab, cfg, st)
+            for role in range(8):
+                for mark in (0, 16, 17, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12):
+                    hold(role, mark, 2000)
+                    held = emulate_substep(tab, cfg, st)
+                    hold(-1, -1, 0)
+                    for a, b in zip(held, free):
+                        assert np.array_equal(a, b), f"{tab.num_links} links: role {role} held at mark {mark} changes the result"
+    finally:
+        hold(-1, -1, 0)
+
+
 def test_humanoid_stands_on_the_oracle():
     """Zero pose on the ground, zero torques: joint springs (stiffness 2..20) and damping hold the pose for a while and
     the ground reaction approaches the weight (40.8 kg)."""
