@@ -273,6 +273,20 @@ int dyros_sim_set_l2_persistence(DyrosSim* sim, void* base, size_t bytes, void* 
 /* Physics launch geometry chosen at create time: envs per CTA, CTAs, threads per CTA, dynamic shared memory bytes. */
 int dyros_sim_launch_info(DyrosSim* sim, int32_t out[4]);
 
+/* gym.add_heightfield (legged_gym terrain, mesh_type 'heightfield'): the ground of the sim becomes a heightfield instead
+ * of the plane z = 0. Vertex (i, j) sits at (origin.x + i row_scale, origin.y + j column_scale,
+ * origin.z + vertical_scale samples[i, j]); each cell is split along the diagonal (i, j)-(i+1, j+1); outside the
+ * field's x-y rectangle there is no ground (DESIGN.md section 4). The contact friction stays DyrosSimDesc.friction /
+ * contact_friction. `samples` is a caller-owned DEVICE buffer that must stay alive and unchanged while the sim uses it.
+ * NULL switches back to the plane. The launch geometry stays as it is. Not for physics_program 1. */
+typedef struct {
+  const int16_t* samples;     /* (num_rows, num_columns) row-major device array; row index along x, column along y */
+  int32_t num_rows, num_columns;  /* >= 2 each */
+  float row_scale, column_scale, vertical_scale;  /* > 0 (m per sample step / per sample unit) */
+  float origin[3];            /* world position of vertex (0, 0) at sample value 0 (HeightFieldParams.transform.p) */
+} DyrosHeightField;
+int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* field);
+
 /* --- task level (bodies of DyrosDynamicWalk methods) --- */
 int dyros_task_create(DyrosSim* sim, const DyrosTaskDesc* desc, const DyrosTaskBuffers* buf, DyrosTask** out);
 int dyros_task_destroy(DyrosTask* task);

@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
 from typing import Dict, Optional
 
 import numpy as np
@@ -34,6 +34,53 @@ INIT_DOF_POS = [0.0, 0.0, -0.24, 0.6, -0.36, 0.0, 0.0, 0.0, -0.24, 0.6, -0.36, 0
 ARMATURE = [0.614, 0.862, 1.09, 1.09, 1.09, 0.360, 0.614, 0.862, 1.09, 1.09, 1.09, 0.360,
             0.078, 0.078, 0.078, 0.18, 0.18, 0.18, 0.18, 0.0032, 0.0032, 0.0032, 0.0032, 0.0032, 0.0032,
             0.18, 0.18, 0.18, 0.18, 0.0032, 0.0032, 0.0032, 0.0032]
+
+
+@dataclass
+class HeightField:
+    """Heightfield ground (gym.add_heightfield; DESIGN.md section 4): vertex (i, j) sits at
+    origin + (i row_scale, j column_scale, vertical_scale samples[i, j]), row index i along x and column index j along y
+    (Isaac Gym's HeightFieldParams, legged_gym's height_samples[px, py]); each cell is split along its diagonal
+    (i, j)-(i+1, j+1); outside the field's x-y rectangle there is no ground.
+    friction: the ground's coefficient in place of CoreConfig.friction (None: keep it).
+    env_origins: (N, 3) world origins of the envs (None: the usual grid, T:709-718, with z the terrain height there)."""
+    samples: np.ndarray
+    row_scale: float
+    column_scale: float
+    vertical_scale: float
+    origin: tuple = (0.0, 0.0, 0.0)
+    friction: Optional[float] = None
+    env_origins: Optional[np.ndarray] = None
+
+    def validate(self):
+        s = self.samples
+        if not isinstance(s, np.ndarray) or s.dtype != np.int16 or s.ndim != 2 or min(s.shape) < 2:
+            raise native.DyrosError("heightfield: samples must be a 2-D int16 array of at least 2 x 2 (rows along x, "
+                                    f"columns along y); got {getattr(s, 'dtype', type(s))} {getattr(s, 'shape', '')}")
+        for k in ("row_scale", "column_scale", "vertical_scale"):
+            v = getattr(self, k)
+            if not (np.isfinite(v) and v > 0):
+                raise native.DyrosError(f"heightfield: {k} must be positive (got {v})")
+        if len(self.origin) != 3 or not np.all(np.isfinite(self.origin)):
+            raise native.DyrosError(f"heightfield: origin must be 3 finite numbers (got {self.origin})")
+        if self.friction is not None and not (np.isfinite(self.friction) and self.friction >= 0):
+            raise native.DyrosError(f"heightfield: friction must be >= 0 (got {self.friction})")
+
+    def height_at(self, x, y):
+        """Terrain height at world points (x, y) and whether they lie on the field (same triangles as the kernels)."""
+        s = self.samples.astype(np.float64) * self.vertical_scale
+        nr, nc = s.shape
+        u = (np.asarray(x, np.float64) - self.origin[0]) / self.row_scale
+        v = (np.asarray(y, np.float64) - self.origin[1]) / self.column_scale
+        inside = (u >= 0) & (v >= 0) & (u <= nr - 1) & (v <= nc - 1)
+        u, v = np.where(inside, u, 0.0), np.where(inside, v, 0.0)
+        i, j = np.minimum(u.astype(int), nr - 2), np.minimum(v.astype(int), nc - 2)
+        fu, fv = u - i, v - j
+        h00, h11 = s[i, j], s[i + 1, j + 1]
+        lower = fu >= fv
+        gu = np.where(lower, s[i + 1, j] - h00, h11 - s[i, j + 1])
+        gv = np.where(lower, h11 - s[i + 1, j], s[i, j + 1] - h00)
+        return self.origin[2] + h00 + fu * gu + fv * gv, inside
 
 
 @dataclass
@@ -76,6 +123,7 @@ class CoreConfig:
     with_rb_force_tensors: bool = False  # generic apply_rigid_body_force_tensors buffers
     physics_program: str = "roles"       # "roles": one lane per env, warp per role (default); "lanes": 8 lanes per env
     self_collision: bool = True          # create_actor(..., filter 0), T:354: the actor's shapes collide with each other
+    heightfield: Optional[HeightField] = None  # ground: None = the plane z = 0 (gym.add_ground), else gym.add_heightfield
 
 
 def stable_penalty(dt_substep: float, m_ref: float = 0.3):
@@ -191,6 +239,14 @@ class DyrosCore:
         self.lib = native.load()
         self.cfg = cfg or CoreConfig()
         self.N = int(num_envs)
+        hf = self.cfg.heightfield
+        if hf is not None:
+            hf.validate()
+            if self.cfg.physics_program != "roles":
+                raise native.DyrosError("heightfield: only the roles physics program has a heightfield ground (the lanes "
+                                        "program is plane only)")
+            if hf.friction is not None:
+                self.cfg = replace(self.cfg, friction=float(hf.friction))
         self.device = torch.device(device)
         self.tables = tables or ModelTables.load(os.path.join(ASSETS, "tocabi_tables.npz"))
         t = self.tables
@@ -263,10 +319,32 @@ class DyrosCore:
         tb["pert_duration"].fill_(1)
         tb["perturb_timing"].fill_(1)
         tb["motor_constant_scale"].fill_(1.0)
-        tb["env_origins"].copy_(torch.tensor(env_origins(N, cfg.env_spacing)))
+        tb["env_origins"].copy_(torch.tensor(self._env_origins()))
+        if cfg.heightfield is not None:  # start where the first reset puts the root (T:734-735), not above (0, 0)
+            s["root_states"][:, 0:3] = tb["env_origins"]
+            s["root_states"][:, 2] += cfg.initial_height
         tb["total_mass"].fill_(float(np.float32(self.tables.total_mass())))
         tb["obs_hist_head"].fill_(19)
         tb["act_hist_head"].fill_(19)
+
+    def _env_origins(self) -> np.ndarray:
+        """T:709-718; on a heightfield the given origins, or the grid with z the terrain height there."""
+        hf = self.cfg.heightfield
+        if hf is None:
+            return env_origins(self.N, self.cfg.env_spacing)
+        if hf.env_origins is not None:
+            o = np.asarray(hf.env_origins, np.float64)
+            if o.shape != (self.N, 3) or not np.all(np.isfinite(o)):
+                raise native.DyrosError(f"heightfield: env_origins must be a finite ({self.N}, 3) array (got {o.shape})")
+        else:
+            o = env_origins(self.N, self.cfg.env_spacing).astype(np.float64)
+            o[:, 2] = hf.height_at(o[:, 0], o[:, 1])[0]
+        inside = hf.height_at(o[:, 0], o[:, 1])[1]
+        if not inside.all():
+            e = int(np.flatnonzero(~inside)[0])
+            raise native.DyrosError(f"heightfield: the origin of env {e} ({o[e, 0]:.3f}, {o[e, 1]:.3f}) lies outside the "
+                                    f"field; {int((~inside).sum())} of {self.N} envs do")
+        return o.astype(np.float32)
 
     def _pack_state_arena(self):
         """Moves every per-env buffer except obs_buf (written once per step, never read by the step) into ONE
@@ -307,6 +385,16 @@ class DyrosCore:
             setattr(sb, n, self.sim_t[n].data_ptr() if n in self.sim_t else None)
         native.check(self.lib.dyros_sim_create(C.byref(sd), C.byref(md), C.byref(sb), C.byref(self.sim_handle)),
                      "dyros_sim_create")
+        hf = self.cfg.heightfield
+        if hf is not None:
+            # (device copy owned by this object: the sim reads it on every step)
+            self.field_samples = torch.tensor(np.ascontiguousarray(hf.samples), dtype=torch.int16, device=self.device)
+            d = native.DyrosHeightField()
+            d.samples = self.field_samples.data_ptr()
+            d.num_rows, d.num_columns = hf.samples.shape
+            d.row_scale, d.column_scale, d.vertical_scale = hf.row_scale, hf.column_scale, hf.vertical_scale
+            d.origin = (C.c_float * 3)(*hf.origin)
+            native.check(self.lib.dyros_sim_set_heightfield(self.sim_handle, C.byref(d)), "dyros_sim_set_heightfield")
 
     def _create_task(self, seed: int):
         t, cfg = self.tables, self.cfg

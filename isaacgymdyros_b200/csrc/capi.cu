@@ -350,6 +350,57 @@ int dyros_sim_launch_info(DyrosSim* sim, int32_t out[4]) {
   return 0;
 }
 
+int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* f) {
+  SIM_OR_FAIL("dyros_sim_set_heightfield");
+  if (!f) {
+    s->has_field = false;
+    s->field = FieldGround{};
+    return 0;
+  }
+  REQUIRE(s->program == 0, "dyros_sim_set_heightfield: the lanes physics program (physics_program 1) has no heightfield "
+                           "ground; use the roles program (0)");
+  REQUIRE(f->samples, "dyros_sim_set_heightfield: samples is NULL");
+  REQUIRE(f->num_rows >= 2 && f->num_columns >= 2, "dyros_sim_set_heightfield: need at least 2 x 2 samples (got %d x %d)",
+          f->num_rows, f->num_columns);
+  REQUIRE(f->row_scale > 0 && f->column_scale > 0 && f->vertical_scale > 0 && std::isfinite(f->row_scale) &&
+              std::isfinite(f->column_scale) && std::isfinite(f->vertical_scale),
+          "dyros_sim_set_heightfield: row_scale, column_scale and vertical_scale must be positive");
+  REQUIRE(std::isfinite(f->origin[0]) && std::isfinite(f->origin[1]) && std::isfinite(f->origin[2]),
+          "dyros_sim_set_heightfield: origin must be finite");
+  // highest vertex and steepest triangle (for the conservative per-link reach cull), from a host copy of the samples
+  const size_t n = (size_t)f->num_rows * f->num_columns;
+  std::vector<int16_t> h(n);
+  DY_CUDA(cudaSetDevice(s->device));
+  DY_CUDA(cudaMemcpy(h.data(), f->samples, n * sizeof(int16_t), cudaMemcpyDeviceToHost));
+  const double dz = f->vertical_scale;
+  double top = -1e300, gmax = 0;
+  for (size_t k = 0; k < n; ++k) top = std::max(top, dz * h[k]);
+  for (int i = 0; i + 1 < f->num_rows; ++i)
+    for (int j = 0; j + 1 < f->num_columns; ++j) {
+      const size_t c = (size_t)i * f->num_columns + j;
+      const double h00 = dz * h[c], h10 = dz * h[c + f->num_columns], h01 = dz * h[c + 1], h11 = dz * h[c + f->num_columns + 1];
+      for (int t = 0; t < 2; ++t) {  // the two triangles of the cell (physics_roles.cuh field_query)
+        const double sx = (t == 0 ? h10 - h00 : h11 - h01) / f->row_scale, sy = (t == 0 ? h11 - h10 : h01 - h00) / f->column_scale;
+        gmax = std::max(gmax, sx * sx + sy * sy);
+      }
+    }
+  FieldGround g{};
+  g.s = f->samples;
+  g.nr = f->num_rows;
+  g.nc = f->num_columns;
+  g.ox = f->origin[0];
+  g.oy = f->origin[1];
+  g.oz = f->origin[2];
+  g.dx = f->row_scale;
+  g.dy = f->column_scale;
+  g.dz = f->vertical_scale;
+  g.zmax = (float)(f->origin[2] + top) + 1e-4f;                     // (rounded up: the cull stays conservative)
+  g.cull = (float)std::sqrt(1 + gmax) * (1 + 1e-5f);                 // 1 / smallest n_z
+  s->has_field = true;  // (same launch geometry as the plane: the env scratch block is the same size)
+  s->field = g;
+  return 0;
+}
+
 int dyros_task_create(DyrosSim* sim, const DyrosTaskDesc* desc, const DyrosTaskBuffers* buf, DyrosTask** out) {
   Task* t = nullptr;
   int rc = build_task(reinterpret_cast<Sim*>(sim), desc, buf, &t);

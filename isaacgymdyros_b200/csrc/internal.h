@@ -92,6 +92,21 @@ struct DevModel {
   float foot_pt_radius[MAX_FEET][MAX_SOLVER_PTS];
 };
 
+// The ground of the physics kernels' role program (physics_roles.cuh), a compile-time parameter: the plane z = 0 with
+// normal +z, or a heightfield (DESIGN.md section 4).
+struct PlaneGround {
+  static constexpr bool kField = false;
+};
+struct FieldGround {
+  static constexpr bool kField = true;
+  const int16_t* s;        // (nr, nc) samples, row-major: row i along x, column j along y (device memory)
+  int nr, nc;              // >= 2 each
+  float ox, oy, oz;        // transform.p
+  float dx, dy, dz;        // row_scale, column_scale, vertical_scale
+  float zmax;              // height of the highest vertex
+  float cull;              // 1 / (smallest n_z of any triangle) >= 1: see link_ext_wrench
+};
+
 struct SimParams {
   int N;
   float dt;       // dt / substeps: the integration step of one sub-step
@@ -146,6 +161,8 @@ struct Sim {
   int program = 0;           // physics program: 0 = one lane per env, warp per role (physics_roles.cuh); 1 = 8 lanes per env (physics_lanes.cuh)
   int envs_per_block = 0;    // physics kernel: envs per CTA
   size_t phys_smem = 0;      // dynamic shared memory of one physics CTA
+  bool has_field = false;    // ground: false = the plane z = 0, true = the heightfield `field` (dyros_sim_set_heightfield)
+  FieldGround field{};
 };
 
 struct Task {

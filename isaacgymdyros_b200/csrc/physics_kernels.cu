@@ -231,8 +231,10 @@ __device__ __noinline__ void noise_stage_slab(NoiseSlabArgs k, int substep, int 
                            [&](int le, int d) { return envs[le * es + dof_link[d] * LS + LS_Q]; });
 }
 
+// (both kernels are instantiated for each ground, PlaneGround and FieldGround: physics_roles.cuh)
+template <class Ground>
 __global__ void __launch_bounds__(kPhysThreads) k_simulate(DevModel m, SimParams p, DyrosSimBuffers b, const float* __restrict__ push,
-                                                           int apply_wrench, int epb, int es) {
+                                                           int apply_wrench, int epb, int es, Ground gnd) {
   extern __shared__ __align__(16) float smem[];
   PhysCta c = phys_cta_setup(m, p, smem, epb, es);
   const int e0 = blockIdx.x * epb, nenv = min(epb, p.N - e0);
@@ -251,7 +253,7 @@ __global__ void __launch_bounds__(kPhysThreads) k_simulate(DevModel m, SimParams
     cp_async_wait_all();
     __syncthreads();
     io.link_pose = (s + 1 == p.substeps && b.link_pose) ? b.link_pose + (size_t)c.e * m.nl * 12 : nullptr;
-    env_substep_role(io, c.sm, c.flags, s, c.hot, m, p, c.role, sync);
+    env_substep_role(io, c.sm, c.flags, s, c.hot, m, p, c.role, sync, false, gnd);
     __syncthreads();
     // (applied wrenches act over the whole simulate() call, i.e. all of its sub-steps: gym_py.html apply_rigid_body_force_tensors)
     if (s + 1 == p.substeps) slab_store_outputs(m, b, c.hot, envs, es, e0, nenv, threadIdx.x, kPhysThreads);
@@ -270,8 +272,9 @@ __device__ __forceinline__ void io_group_sync() { asm volatile("bar.sync 1, %0;"
 // reads the joint angles, untouched until the roles' last pass), evaluates the torque stage and re-stages damping and
 // armature (F_IO_TAU, consumed by pass 2), so none of this sits on the roles' critical path.
 
+template <class Ground>
 __global__ void __launch_bounds__(kStepThreads) k_step_physics(DevModel m, SimParams p, TK k, int epb, int es, long long* trace,
-                                                                const float* __restrict__ actions) {
+                                                                const float* __restrict__ actions, Ground gnd) {
   extern __shared__ __align__(16) float smem[];
   __shared__ float pro[kSlabMaxEnvs][8];  // per-env scalars of the prologue (stage_prologue_slab)
   if (trace && blockIdx.x == 0 && threadIdx.x == 0) trace[24] = clock64();  // kernel entry (profiling)
@@ -370,7 +373,7 @@ __global__ void __launch_bounds__(kStepThreads) k_step_physics(DevModel m, SimPa
         io.push = s == 0 ? k.b.push_force : nullptr;  // every sub-step of the first simulate of the policy step (T:502 vs T:504)
         io.link_pose = (s + 1 == k.p.skipframe && ss + 1 == p.substeps && k.s.link_pose) ? k.s.link_pose + (size_t)c.e * m.nl * 12 : nullptr;
         sync.mark(13);
-        env_substep_role(io, c.sm, c.flags, epoch, c.hot, m, p, role, sync, true);
+        env_substep_role(io, c.sm, c.flags, epoch, c.hot, m, p, role, sync, true, gnd);
       }
       __syncthreads();
     }
@@ -400,16 +403,22 @@ static int physics_configure_roles(Sim* sim) {
   }
   sim->envs_per_block = epb;
   sim->phys_smem = phys_smem_bytes(sim, epb);
-  DY_CUDA(cudaFuncSetAttribute(k_simulate, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
-  DY_CUDA(cudaFuncSetAttribute(k_step_physics, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_simulate<PlaneGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_step_physics<PlaneGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_simulate<FieldGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_step_physics<FieldGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
   return 0;
 }
 
 static int launch_simulate_roles(Sim* sim, int apply_wrench, const float* push, cudaStream_t s) {
   const int epb = sim->envs_per_block;
   const int grid = (sim->p.N + epb - 1) / epb;
-  k_simulate<<<grid, kPhysThreads, sim->phys_smem, s>>>(sim->m, sim->p, sim->b, push, apply_wrench, epb,
-                                                   env_scratch_floats(sim->m.nl, sim->m.nb));
+  if (sim->has_field)
+    k_simulate<<<grid, kPhysThreads, sim->phys_smem, s>>>(sim->m, sim->p, sim->b, push, apply_wrench, epb, env_scratch_floats(sim->m.nl, sim->m.nb),
+                                                     sim->field);
+  else
+    k_simulate<<<grid, kPhysThreads, sim->phys_smem, s>>>(sim->m, sim->p, sim->b, push, apply_wrench, epb, env_scratch_floats(sim->m.nl, sim->m.nb),
+                                                     PlaneGround());
   DY_LAUNCH_CHECK();
   return 0;
 }
@@ -423,8 +432,12 @@ static int launch_task_physics_roles(Task* t, cudaStream_t s, long long* trace, 
   k.b = t->b;
   k.s = sim->b;
   k.j = t->inj;
-  DY_CUDA(launch_kernel(k_step_physics, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p, k, epb,
-                        env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions));
+  if (sim->has_field)
+    DY_CUDA(launch_kernel(k_step_physics<FieldGround>, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p,
+                          k, epb, env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions, sim->field));
+  else
+    DY_CUDA(launch_kernel(k_step_physics<PlaneGround>, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p,
+                          k, epb, env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions, PlaneGround()));
   return 0;
 }
 

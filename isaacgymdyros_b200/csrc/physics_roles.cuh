@@ -104,6 +104,96 @@ HD void export_pose(const EnvIO& io, int link, const M3& Rw, V3 pw) {
   o[9] = (float)pw.x; o[10] = (float)pw.y; o[11] = (float)pw.z;
 }
 
+// ---- the ground (DESIGN.md section 4), a compile-time parameter of the role program: the plane z = 0 with normal +z,
+//      or a heightfield. Vertex (i, j) of the field sits at (ox + i dx, oy + j dy, oz + dz s[i, j]); each cell is split
+//      along its diagonal (i, j)-(i+1, j+1); outside the field's x-y rectangle there is no ground.
+// (PlaneGround, FieldGround: internal.h)
+
+HD real field_sample(const int16_t* s) {
+#ifdef __CUDA_ARCH__
+  return (real)__ldg(s);  // read-only path: the samples are shared by every env and stay in L2
+#else
+  return (real)*s;
+#endif
+}
+
+// Height h and unit upward normal n of the heightfield at (x, y); false outside the field. Grid coordinates
+// u = (x - ox) / dx, v = (y - oy) / dy; the cell is (floor u, floor v), except that the last row / column of vertices
+// belongs to the cell before it. Inside the cell (fu, fv), a point with fu >= fv (on the diagonal or on the +x side of
+// it) takes the triangle (i, j), (i+1, j), (i+1, j+1); any other the triangle (i, j), (i, j+1), (i+1, j+1).
+HD bool field_query(const FieldGround& g, real x, real y, real& h, V3& n) {
+  const real u = (x - g.ox) / g.dx, v = (y - g.oy) / g.dy;
+  if (!(u >= 0 && v >= 0 && u <= (real)(g.nr - 1) && v <= (real)(g.nc - 1))) return false;
+  int i = (int)u, j = (int)v;
+  i = i < g.nr - 2 ? i : g.nr - 2;
+  j = j < g.nc - 2 ? j : g.nc - 2;
+  const real fu = u - (real)i, fv = v - (real)j;
+  const int16_t* c = g.s + (size_t)i * g.nc + j;
+  const real h00 = g.dz * field_sample(c), h11 = g.dz * field_sample(c + g.nc + 1);
+  real gu, gv;  // height change per grid step along u and along v on the chosen triangle
+  if (fu >= fv) {
+    const real h10 = g.dz * field_sample(c + g.nc);
+    gu = h10 - h00;
+    gv = h11 - h10;
+  } else {
+    const real h01 = g.dz * field_sample(c + 1);
+    gu = h11 - h01;
+    gv = h01 - h00;
+  }
+  h = g.oz + h00 + fu * gu + fv * gv;
+  const real sx = gu / g.dx, sy = gv / g.dy;
+  const real inv = 1 / sqrt(1 + sx * sx + sy * sy);
+  n = v3(-sx * inv, -sy * inv, inv);
+  return true;
+}
+
+// Tangent directions of a contact with ground normal n: t1 = normalize(n_z, 0, -n_x), t2 = n x t1 (world x and y for
+// n = +z).
+HD void field_tangents(V3 n, V3& t1, V3& t2) {
+  const real inv = 1 / sqrt(n.z * n.z + n.x * n.x);
+  t1 = v3(n.z * inv, 0, -n.x * inv);
+  t2 = cross(n, t1);
+}
+
+// Heightfield: the active sole points of foot g (X_PTS, at most MAX_ACTIVE_PTS) from the start-of-step foot pose
+// (X_FOOTPOSE); returns their number and the foot's world rotation. Gap phi = (z_c - h) n_z - r of a candidate sphere
+// (centre c, radius r); active when phi < contact_offset. The ground normal of active point a is kept in LS_WP of the
+// a-th link of the foot's chain (>= 6 links, all in the foot's role): so this runs after the role's pass 3, the last
+// reader of LS_WP, and the env scratch block needs no extra words (the CTA still holds 28 TOCABI envs).
+HD int field_select(const FieldGround& gnd, const DevModel& m, const SimParams& p, real* sm, real* X, int g, real inv_dt,
+                    M3& Rwf) {
+  Rwf = ld_m3(X + X_FOOTPOSE + 12 * g);
+  const V3 pf = ld3(X + X_FOOTPOSE + 12 * g + 9);
+  real* const pts = X + X_PTS + g * MAX_ACTIVE_PTS * PT_WORDS;
+  int nact = 0;
+  real h;
+  V3 n;
+#pragma unroll 1
+  for (int k = 0; k < m.foot_npts[g]; ++k) {
+    const V3 c = pf + mul(Rwf, v3(m.foot_pt_pos[g][k][0], m.foot_pt_pos[g][k][1], m.foot_pt_pos[g][k][2]));
+    if (!field_query(gnd, c.x, c.y, h, n)) continue;
+    real phi = (c.z - h) * n.z - m.foot_pt_radius[g][k];
+    if (phi < p.contact_offset && nact < MAX_ACTIVE_PTS) {
+      real* pt = pts + nact * PT_WORDS;
+      reinterpret_cast<int*>(pt)[0] = k;
+      pt[1] = phi >= 0 ? -phi * inv_dt : fmin_r(-p.erp * phi * inv_dt, p.max_depen_vel);
+      pt[2] = pt[3] = pt[4] = 0;
+      st3(BLK(m.chain[g][nact]) + LS_WP, n);
+      ++nact;
+    }
+  }
+  return nact;
+}
+
+// Heightfield: active sole point `a` of foot g -> its contact location relative to the foot origin, world axes (the
+// sphere's point along -n), and its row directions n, t1, t2.
+HD void field_sole_point(const DevModel& m, const real* sm, const real* X, const M3& Rwf, int g, int a, V3& xa, V3* dirs) {
+  const int k = reinterpret_cast<const int*>(X + X_PTS + (g * MAX_ACTIVE_PTS + a) * PT_WORDS)[0];
+  dirs[0] = ld3(BLK(m.chain[g][a]) + LS_WP);
+  field_tangents(dirs[0], dirs[1], dirs[2]);
+  xa = mul(Rwf, v3(m.foot_pt_pos[g][k][0], m.foot_pt_pos[g][k][1], m.foot_pt_pos[g][k][2])) - m.foot_pt_radius[g][k] * dirs[0];
+}
+
 // ---- penalty ground contact of one location on a link (oracle: PhysicsOracle._external_wrench.add_point);
 //      xw = the location relative to the link origin, world axes; v = [w; u] of the link
 HD void penalty_point(const SimParams& p, real mu, SV v, V3 xw, real depth, float* cf, bool live, SV& fext) {
@@ -115,6 +205,27 @@ HD void penalty_point(const SimParams& p, real mu, SV v, V3 xw, real depth, floa
   real lim = mu * fn / (speed > (real)1e-6 ? speed : (real)1e-6);
   real coef = p.pen_c < lim ? p.pen_c : lim;
   V3 Fw = v3(-coef * vel_w.x, -coef * vel_w.y, fn);
+  if (live) {
+    cf[0] += (float)Fw.x;
+    cf[1] += (float)Fw.y;
+    cf[2] += (float)Fw.z;
+  }
+  fext.w = fext.w + cross(xw, Fw);
+  fext.v = fext.v + Fw;
+}
+// the same against a ground of unit normal n at the contact location: normal force along n damped by v.n, friction on
+// the tangential part of the velocity (= penalty_point for n = +z)
+HD void penalty_point_n(const SimParams& p, real mu, SV v, V3 xw, V3 n, real depth, float* cf, bool live, SV& fext) {
+  if (!(depth > 0)) return;
+  V3 vel_w = v.v + cross(v.w, xw);
+  const real vn = dot(vel_w, n);
+  real fn = p.pen_k * depth - p.pen_c * vn;
+  fn = fn < 0 ? 0 : (fn > p.pen_fmax ? p.pen_fmax : fn);
+  const V3 vt = vel_w - vn * n;
+  real speed = sqrt(dot(vt, vt));
+  real lim = mu * fn / (speed > (real)1e-6 ? speed : (real)1e-6);
+  real coef = p.pen_c < lim ? p.pen_c : lim;
+  V3 Fw = fn * n - coef * vt;
   if (live) {
     cf[0] += (float)Fw.x;
     cf[1] += (float)Fw.y;
@@ -147,8 +258,9 @@ HD ABI link_inertia(const real* X, const float* hot, const DevModel& m, const fl
 
 // External wrench on the link of record R (world axes, about the link origin): applied body wrenches and penalty
 // ground contact.
+template <class Ground>
 HD SV link_ext_wrench(const EnvIO& io, const real* X, const float* hot, const DevModel& m, const SimParams& p,
-                      const float* R, const M3& Rw, V3 pw, SV v) {
+                      const float* R, const M3& Rw, V3 pw, SV v, const Ground& gnd) {
   SV fext = sv_zero();
   V3 nrm = v3(Rw.a[6], Rw.a[7], Rw.a[8]);  // world z in link coordinates
   if (io.rb_force || (io.push && RI(R, R_LINK) == 0)) {  // applied world wrenches at the bodies' COMs (tensors.rst.txt:322-335)
@@ -169,6 +281,39 @@ HD SV link_ext_wrench(const EnvIO& io, const real* X, const float* hot, const De
       fext.w = fext.w + cross(com, F) + T;
       fext.v = fext.v + F;
     }
+  }
+  if constexpr (Ground::kField) {
+    // Cull: a sphere of radius r <= reach touches where (h - z_c) n_z + r > 0, i.e. z_c < h + r / n_z, and its centre is
+    // at most reach - r below the link origin; a cylinder's rim point at most reach below it. So nothing of this link
+    // can touch unless pw.z < zmax + reach * cull.
+    if (pw.z - gnd.zmax < R[R_REACH] * gnd.cull) {
+      const real mu = X[X_MU];
+      real h;
+      V3 n;
+#pragma unroll 1
+      for (int k = RI(R, R_PT0); k < RI(R, R_PT1); ++k) {
+        const V3 xw = mul(Rw, ld3_f(m.pt_pos + 3 * k));
+        const real rad = m.pt_radius[k];
+        const V3 c = pw + xw;
+        if (!field_query(gnd, c.x, c.y, h, n)) continue;
+        penalty_point_n(p, mu, v, xw - rad * n, n, (h - c.z) * n.z + rad, io.contact + 3 * m.pt_body[k], io.live, fext);
+      }
+#pragma unroll 1
+      for (int k = RI(R, R_CYL0); k < RI(R, R_CYL1); ++k) {  // the rim point lowest in WORLD z, as for the plane
+        V3 c = ld3_f(m.cyl_center + 3 * k), a = ld3_f(m.cyl_axis + 3 * k);
+        real rad = m.cyl_size[2 * k], hh = m.cyl_size[2 * k + 1];
+        real az = dot(nrm, a);
+        real s = az >= 0 ? (real)-1 : (real)1;
+        V3 d = neg(nrm - az * a);
+        real dn = sqrt(dot(d, d));
+        V3 rim = c + (s * hh) * a;
+        if (dn > (real)1e-6) rim = rim + (rad / dn) * d;
+        const V3 xw = mul(Rw, rim), q = pw + xw;
+        if (!field_query(gnd, q.x, q.y, h, n)) continue;
+        penalty_point_n(p, mu, v, xw, n, (h - q.z) * n.z, io.contact + 3 * m.cyl_body[k], io.live, fext);
+      }
+    }
+    return fext;
   }
   if (pw.z < R[R_REACH]) {  // nothing of this link can reach z = 0 otherwise
     const real mu = X[X_MU];
@@ -234,9 +379,10 @@ HD void env_store_outputs(const EnvIO& io, const real* sm, const float* hot, con
 // with `io_async` the per-sub-step inputs are staged concurrently by another warp, which publishes F_IO_PRE (push,
 // zeroed contact forces: needed by the force loop), F_IO_TAU (torque, damping, armature: needed by pass 2) and
 // F_IO_DONE (it has finished reading the joint angles, which the last pass overwrites).
-template <class Sync>
+// `gnd`: the ground (PlaneGround or FieldGround).
+template <class Sync, class Ground = PlaneGround>
 HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const float* hot, const DevModel& m,
-                         const SimParams& p, int role, Sync& sync, bool io_async = false) {
+                         const SimParams& p, int role, Sync& sync, bool io_async = false, const Ground& gnd = Ground()) {
   const int nl = m.nl;
   real* X = sm + nl * LS;
   const real dt = p.dt;
@@ -345,7 +491,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
       }
       IA = link_inertia(X, hot, m, R, Rw);
       const V3 h = v3(IA.H.a[7], IA.H.a[2], IA.H.a[3]);  // m c, world axes
-      pA = SV{cross(v.w, mul(IA.I, v.w)), cross(v.w, cross(v.w, h))} - link_ext_wrench(io, X, hot, m, p, R, Rw, pw, v);
+      pA = SV{cross(v.w, mul(IA.I, v.w)), cross(v.w, cross(v.w, h))} - link_ext_wrench(io, X, hot, m, p, R, Rw, pw, v, gnd);
     }
     for (int j = 0; j < RI(R, R_NCHILD); ++j) {
       const int cf = RI(R, R_CHILD0 + j), c = cf & ~REC_FOREIGN;
@@ -467,7 +613,9 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
   int nact = 0;
   const real inv_dt = 1 / dt;
   real* const pts = X + X_PTS + (foot >= 0 ? foot : 0) * MAX_ACTIVE_PTS * PT_WORDS;
-  if (foot >= 0) {
+  if constexpr (Ground::kField) {
+    // (heightfield: selected after pass 3, field_select)
+  } else if (foot >= 0) {
     const int g = foot;
     Rwf = ld_m3(X + X_FOOTPOSE + 12 * g);
     const real pz = X[X_FOOTPOSE + 12 * g + 11];
@@ -521,6 +669,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
   if (foot >= 0) {
     const int g = foot;
     const int clen = m.chain_len[g];
+    if constexpr (Ground::kField) nact = field_select(gnd, m, p, sm, X, g, inv_dt, Rwf);
     SV Y[6];              // Om_lca G
     SV V = ld6(BLK(0) + LS_U);  // base role published v0* with ST_PASS2 (waited for in pass 3)
     SV P = sv_zero();     // accumulated contact impulse on the foot (world axes, about the foot origin)
@@ -557,6 +706,23 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
     }
     // rows of the active points: response cv = Om J and 1 / (J . cv) per direction (world z, x, y), parked in the
     // blocks of the first chain links (ROWS_PER_LINK per link)
+    // (heightfield: rows n, t1, t2 of the point's ground normal)
+    if constexpr (Ground::kField) {
+#pragma unroll 1
+      for (int a = 0; a < nact; ++a) {
+        V3 xa, dirs[3];
+        field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+#pragma unroll
+        for (int d = 0; d < 3; ++d) {
+          SV J{cross(xa, dirs[d]), dirs[d]};
+          SV cv = mul(Om, J);
+          const int row = a * 3 + d;
+          real* rw = BLK(m.chain[g][row / ROWS_PER_LINK]) + LS_A + A_ROWS + (row % ROWS_PER_LINK) * 7;
+          st6(rw, cv);
+          rw[6] = 1 / dot(J, cv);
+        }
+      }
+    } else {
 #pragma unroll 1
     for (int a = 0; a < nact; ++a) {
       const V3 xa = sole_point(g, reinterpret_cast<const int*>(pts + a * PT_WORDS)[0]);
@@ -571,11 +737,45 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
         rw[6] = 1 / dot(J, cv);
       }
     }
+    }
     sync.mark(7);
     // fixed number of sweeps; Gauss-Seidel inside a foot, Jacobi between the feet (coupled through the base)
     const real mu = X[X_MU];
     for (int s = 0; s < p.sweeps; ++s) {
       SV dP = sv_zero();
+      if constexpr (Ground::kField) {
+#pragma unroll 1
+        for (int a = 0; a < nact; ++a) {
+          real* pt = pts + a * PT_WORDS;
+          V3 xa, dirs[3];
+          field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+          const real bias = pt[1];
+          real lam[3] = {pt[2], pt[3], pt[4]};
+#pragma unroll
+          for (int d = 0; d < 3; ++d) {
+            SV J{cross(xa, dirs[d]), dirs[d]};
+            const int row = a * 3 + d;
+            const real* rw = BLK(m.chain[g][row / ROWS_PER_LINK]) + LS_A + A_ROWS + (row % ROWS_PER_LINK) * 7;
+            real vrel = dot(J, V);
+            real nw;
+            if (d == 0) {
+              nw = lam[0] + (bias - vrel) * rw[6];
+              nw = nw > 0 ? nw : 0;
+            } else {
+              real lim = mu * lam[0];
+              nw = lam[d] - vrel * rw[6];
+              nw = nw > lim ? lim : (nw < -lim ? -lim : nw);
+            }
+            real delta = nw - lam[d];
+            lam[d] = nw;
+            V = V + delta * ld6(rw);
+            dP = dP + delta * J;
+          }
+          pt[2] = lam[0];
+          pt[3] = lam[1];
+          pt[4] = lam[2];
+        }
+      } else {
 #pragma unroll 1
       for (int a = 0; a < nact; ++a) {
         real* pt = pts + a * PT_WORDS;
@@ -607,6 +807,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
         pt[3] = lam[1];
         pt[4] = lam[2];
       }
+      }
       P = P + dP;
       if (m.num_feet == 2) {
         // base velocity change caused by this sweep's impulses: Om0 G dP = sum_c dP_c Y_c (double-buffered by sweep parity)
@@ -633,6 +834,15 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
       for (int a = 0; a < nact; ++a) {  // world force over this sub-step: rows (n, t1, t2) = world (z, x, y)
         const real* pt = pts + a * PT_WORDS;
         float* cf = io.contact + 3 * m.foot_pt_body[g][reinterpret_cast<const int*>(pt)[0]];
+        if constexpr (Ground::kField) {  // (lam_n n + lam_1 t1 + lam_2 t2) / dt
+          V3 xa, dirs[3];
+          field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+          const V3 F = (pt[2] * inv_dt) * dirs[0] + (pt[3] * inv_dt) * dirs[1] + (pt[4] * inv_dt) * dirs[2];
+          cf[0] += (float)F.x;
+          cf[1] += (float)F.y;
+          cf[2] += (float)F.z;
+          continue;
+        }
         cf[0] += (float)(pt[3] * inv_dt);
         cf[1] += (float)(pt[4] * inv_dt);
         cf[2] += (float)(pt[2] * inv_dt);

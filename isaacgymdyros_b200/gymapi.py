@@ -14,13 +14,14 @@ the same storage, so refresh_* are no-ops that return True (except rigid_body_st
 from __future__ import annotations
 
 import os
+from dataclasses import replace
 from typing import List, Optional
 
 import numpy as np
 import torch
 
 from . import native
-from .core import ARMATURE, ASSETS, CoreConfig, DyrosCore, stable_penalty
+from .core import ARMATURE, ASSETS, CoreConfig, DyrosCore, HeightField, stable_penalty
 from .model.mjcf import load_mjcf
 from .model.tables import ModelTables, build_tables
 
@@ -78,6 +79,32 @@ class PlaneParams:
         self.dynamic_friction = 1.0
         self.restitution = 0.0
         self.segmentation_id = 0
+
+
+class HeightFieldParams:
+    """gymapi.HeightFieldParams: the samples are (nbRows, nbColumns), row index along x, column index along y; vertex
+    (i, j) at transform.p + (i row_scale, j column_scale, vertical_scale h[i, j]). transform.r must be the identity."""
+    def __init__(self):
+        self.nbRows = 0
+        self.nbColumns = 0
+        self.column_scale = 1.0
+        self.row_scale = 1.0
+        self.vertical_scale = 1.0
+        self.transform = Transform()
+        self.static_friction = 1.0
+        self.dynamic_friction = 1.0
+        self.restitution = 0.0
+        self.segmentation_id = 0
+
+
+class TriangleMeshParams:
+    def __init__(self):
+        self.nb_vertices = 0
+        self.nb_triangles = 0
+        self.transform = Transform()
+        self.static_friction = 1.0
+        self.dynamic_friction = 1.0
+        self.restitution = 0.0
 
 
 class AssetOptions:
@@ -213,6 +240,7 @@ class Sim:
     def __init__(self, compute_device: int, params: SimParams):
         self.compute_device, self.params = compute_device, params
         self.plane: Optional[PlaneParams] = None
+        self.heightfield: Optional[HeightField] = None  # add_heightfield (a sim has one ground: plane or heightfield)
         self.asset: Optional[Asset] = None
         self.envs: List[Env] = []
         self.start_poses: List[Transform] = []
@@ -240,6 +268,12 @@ def _cfg_from_sim(sim: Sim) -> CoreConfig:
     cfg.penalty_stiffness, cfg.penalty_damping = stable_penalty(p.dt / p.substeps)
     if sim.plane is not None:
         cfg.friction = float(sim.plane.dynamic_friction)  # shape friction default 1.0 (SURVEY D2)
+    if sim.heightfield is not None:
+        cfg.friction = float(sim.heightfield.friction)    # combined with the shapes as the plane's
+        # (the envs sit where create_actor put them: their origins are the actors' start positions on the field)
+        pos = np.array([[tf.p.x, tf.p.y, 0.0] for tf in sim.start_poses], np.float64).reshape(-1, 3)
+        pos[:, 2] = sim.heightfield.height_at(pos[:, 0], pos[:, 1])[0]
+        cfg.heightfield = replace(sim.heightfield, env_origins=pos)
     if sim.asset is not None:
         cfg.max_angular_velocity = float(sim.asset.options.max_angular_velocity)
     return cfg
@@ -266,10 +300,39 @@ class Gym:
             sim.core = None
 
     def add_ground(self, sim: Sim, params: PlaneParams):
+        if sim.heightfield is not None:
+            raise native.DyrosError("add_ground: the sim already has a heightfield ground (one ground per sim)")
         n = params.normal
         if (round(n.x, 6), round(n.y, 6), round(n.z, 6)) != (0.0, 0.0, 1.0) or params.distance != 0.0:
             raise native.DyrosError("add_ground: only the z = 0 plane with normal +z is implemented (T:227-235)")
         sim.plane = params
+
+    def add_heightfield(self, sim: Sim, heightSamples, params: HeightFieldParams):
+        """The ground of the sim becomes a heightfield (legged_gym terrain, mesh_type 'heightfield'): int16 samples of
+        shape (nbRows, nbColumns), or their row-major flattening. Outside the field there is no ground."""
+        if sim.plane is not None or sim.heightfield is not None:
+            raise native.DyrosError("add_heightfield: the sim already has a ground (one ground per sim: a plane or a "
+                                    "heightfield)")
+        if sim.core is not None:
+            raise native.DyrosError("add_heightfield: call it before prepare_sim")
+        r = params.transform.r
+        if (round(r.x, 6), round(r.y, 6), round(r.z, 6), round(abs(r.w), 6)) != (0.0, 0.0, 0.0, 1.0):
+            raise native.DyrosError("add_heightfield: only an identity transform.r is implemented (the field is axis-aligned)")
+        a = np.asarray(heightSamples)
+        if a.dtype != np.int16:
+            raise native.DyrosError(f"add_heightfield: samples must be int16 (got {a.dtype})")
+        if a.size != int(params.nbRows) * int(params.nbColumns):
+            raise native.DyrosError(f"add_heightfield: {a.size} samples for nbRows x nbColumns = {params.nbRows} x {params.nbColumns}")
+        p = params.transform.p
+        hf = HeightField(np.ascontiguousarray(a.reshape(int(params.nbRows), int(params.nbColumns))), float(params.row_scale),
+                         float(params.column_scale), float(params.vertical_scale), (p.x, p.y, p.z),
+                         friction=float(params.dynamic_friction))
+        hf.validate()
+        sim.heightfield = hf
+
+    def add_triangle_mesh(self, sim: Sim, vertices, triangles, params: "TriangleMeshParams"):
+        raise native.DyrosError("add_triangle_mesh: triangle-mesh ground is not implemented (it needs a general mesh "
+                                "narrow phase); use add_heightfield (mesh_type 'heightfield') or add_ground")
 
     def load_asset(self, sim: Sim, rootpath: str, filename: str, options: Optional[AssetOptions] = None):
         options = options or AssetOptions()
@@ -417,7 +480,9 @@ class Gym:
             sim.shape_friction.append(1.0)
         sim.shape_friction[env.index] = mu
         if sim.core is not None and "contact_friction" in sim.core.sim_t:
-            plane = float(sim.plane.dynamic_friction) if sim.plane is not None else 1.0
+            ground = sim.heightfield.friction if sim.heightfield is not None else (
+                sim.plane.dynamic_friction if sim.plane is not None else 1.0)
+            plane = float(ground)
             sim.core.sim_t["contact_friction"][env.index] = plane * mu
         return True
 
@@ -478,8 +543,8 @@ class Gym:
         """vec_task.py:196: allocate the tensor-API buffers and build the native sim."""
         if sim.core is not None:
             return True
-        if sim.asset is None or not sim.envs or sim.plane is None:
-            print("*** prepare_sim: need a ground plane, an asset and at least one env")
+        if sim.asset is None or not sim.envs or (sim.plane is None and sim.heightfield is None):
+            print("*** prepare_sim: need a ground (plane or heightfield), an asset and at least one env")
             return False
         N = len(sim.envs)
         if any(len(e.actor_names) != 1 for e in sim.envs):

@@ -44,6 +44,11 @@ SIM_BUFFERS = ["root_states", "dof_state", "net_contact_force", "rigid_body_stat
                "rb_torque", "dof_damping", "dof_armature", "body_mass_scale", "contact_friction", "link_pose", "self_contact_force"]
 
 
+class DyrosHeightField(C.Structure):
+    _fields_ = [("samples", C.c_void_p), ("num_rows", i32), ("num_columns", i32), ("row_scale", f32),
+                ("column_scale", f32), ("vertical_scale", f32), ("origin", f32 * 3)]
+
+
 class DyrosSimBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in SIM_BUFFERS]
 
@@ -152,6 +157,7 @@ SIGNATURES = {
     "dyros_measure_fp32_peak": (_INT, [_INT, _INT, C.POINTER(C.c_double)]),
     "dyros_flush_l2": (_INT, [C.c_void_p, C.c_size_t, _INT, C.c_void_p]),
     "dyros_sim_launch_info": (_INT, [_VP, C.POINTER(C.c_int32 * 4)]),
+    "dyros_sim_set_heightfield": (_INT, [_VP, C.POINTER(DyrosHeightField)]),
     "dyros_task_create": (_INT, [_VP, C.POINTER(DyrosTaskDesc), C.POINTER(DyrosTaskBuffers), C.POINTER(_VP)]),
     "dyros_task_destroy": (_INT, [_VP]),
     "dyros_task_set_noise_injection": (_INT, [_VP, C.POINTER(DyrosNoiseInjection)]),

@@ -13,7 +13,7 @@ from typing import Any, Dict, Optional
 import numpy as np
 import torch
 
-from ..core import CoreConfig, DyrosCore
+from ..core import CoreConfig, DyrosCore, HeightField
 from .spaces import Box
 
 REWARD_NAMES = ["mimic_body_orientation_reward", "qpos_regulation", "qvel_regulation", "contact_force_penalty",
@@ -73,6 +73,13 @@ def core_config_from_cfg(cfg: Dict[str, Any]) -> CoreConfig:
                    # T:354; `selfCollision: False` drops the self-collision pass, e.g. to time the step without it)
                    self_collision=env.get("selfCollision", True),
                    physics_program=env.get("physicsProgram", "roles"))  # (ours too: DESIGN.md section 4, "Two programs")
+    # (not a key of the reference's yaml either: the reference's terrain code, T:203-270, builds the field and calls
+    # gym.add_heightfield; here the field comes with the cfg. DESIGN.md section 4, "Ground")
+    hf = env.get("heightfield")
+    if hf is not None:
+        c.heightfield = HeightField(np.asarray(hf["samples"]), float(hf["row_scale"]), float(hf["column_scale"]),
+                                    float(hf["vertical_scale"]), tuple(hf.get("origin", (0.0, 0.0, 0.0))),
+                                    friction=hf.get("friction"), env_origins=hf.get("env_origins"))
     ap = task.get("randomization_params", {}).get("actor_params", {}).get("humanoid", {})
     dp = ap.get("dof_properties", {})
     if "damping" in dp:
