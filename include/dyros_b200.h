@@ -291,6 +291,24 @@ int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* field);
 int dyros_task_create(DyrosSim* sim, const DyrosTaskDesc* desc, const DyrosTaskBuffers* buf, DyrosTask** out);
 int dyros_task_destroy(DyrosTask* task);
 int dyros_task_set_noise_injection(DyrosTask* task, const DyrosNoiseInjection* inj);
+/* Terrain curriculum (legged_gym's _update_terrain_curriculum; DESIGN.md section 4, "Curriculum"). Every reset of env e,
+ * fused or staged or through dyros_task_reset_idx, first moves the env one level up when its root has walked farther than
+ * move_up_distance from env_origins[e] in x-y, else one level down when it walked less than |target_vel[e]| *
+ * move_down_scale; a level past the top is redrawn uniformly over [0, num_levels) (reset_f column 30), a level below 0
+ * stays 0. env_origins[e] then becomes origins[levels[e], types[e]] and the root is placed there. The end-of-step pass
+ * writes the mean of `levels` over all envs to level_mean. All pointers are caller-owned DEVICE memory that must stay
+ * alive while the task uses them. NULL switches the curriculum off. Call before a CUDA graph of the step is captured:
+ * captured launches keep the setting they were captured with. */
+typedef struct {
+  const float* origins;      /* (num_levels, num_types, 3) world origin of each sub-terrain */
+  int32_t* levels;           /* (N) terrain level of each env, in [0, num_levels); updated on every reset */
+  const int32_t* types;      /* (N) terrain type (column) of each env, in [0, num_types) */
+  int32_t num_levels, num_types;  /* >= 1 each */
+  float move_up_distance;    /* terrain_length / 2 */
+  float move_down_scale;     /* episode length (s) * 0.5 */
+  float* level_mean;         /* (1) mean level after each step's resets; may be NULL */
+} DyrosTerrainCurriculum;
+int dyros_task_set_terrain_curriculum(DyrosTask* task, const DyrosTerrainCurriculum* curriculum);
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream);      /* VT:307 + T:449-502 */
 /* T:504-530 in one launch: skipframe x (substep torque, gym.simulate, sensor noise); what dyros_task_step uses. */
 int dyros_task_physics(DyrosTask* task, void* stream);

@@ -84,6 +84,36 @@ class HeightField:
 
 
 @dataclass
+class TerrainCurriculum:
+    """Envs on a grid of sub-terrains and the terrain curriculum (legged_gym's _update_terrain_curriculum; DESIGN.md
+    section 4, "Curriculum"): env e starts at origins[levels[e], types[e]]. With `curriculum`, every reset moves it one
+    level up when it walked farther than move_up_distance from its origin, one level down when it walked less than
+    |target_vel| * move_down_scale; past the top level it lands on a random one. The update runs in the reset stage of
+    the task kernels (dyros_task_set_terrain_curriculum).
+    origins: (num_levels, num_types, 3) world origins of the sub-terrains; types, levels: (N,) integers."""
+    origins: np.ndarray
+    types: np.ndarray
+    levels: np.ndarray
+    move_up_distance: float      # terrain_length / 2
+    move_down_scale: float       # episode length (s) * 0.5
+    curriculum: bool = True      # False: the envs keep their initial sub-terrain (no level updates)
+
+    def validate(self, n: int):
+        o = np.asarray(self.origins)
+        if o.ndim != 3 or o.shape[2] != 3 or min(o.shape[:2]) < 1 or not np.all(np.isfinite(o)):
+            raise native.DyrosError(f"terrain curriculum: origins must be a finite (levels, types, 3) array (got {o.shape})")
+        for k, hi in (("types", o.shape[1]), ("levels", o.shape[0])):
+            v = np.asarray(getattr(self, k))
+            if v.shape != (n,) or not np.issubdtype(v.dtype, np.integer) or v.min() < 0 or v.max() >= hi:
+                raise native.DyrosError(f"terrain curriculum: {k} must be ({n},) integers in [0, {hi}) "
+                                        f"(got {v.dtype} {v.shape})")
+        for k in ("move_up_distance", "move_down_scale"):
+            v = getattr(self, k)
+            if not (np.isfinite(v) and v >= 0):
+                raise native.DyrosError(f"terrain curriculum: {k} must be >= 0 (got {v})")
+
+
+@dataclass
 class CoreConfig:
     """Values of cfg/task/DyrosDynamicWalk.yaml that reach the kernels (SURVEY Appendix A1) plus the
     named model options of SURVEY D2."""
@@ -124,6 +154,7 @@ class CoreConfig:
     physics_program: str = "roles"       # "roles": one lane per env, warp per role (default); "lanes": 8 lanes per env
     self_collision: bool = True          # create_actor(..., filter 0), T:354: the actor's shapes collide with each other
     heightfield: Optional[HeightField] = None  # ground: None = the plane z = 0 (gym.add_ground), else gym.add_heightfield
+    terrain_curriculum: Optional[TerrainCurriculum] = None  # env origins on sub-terrains (+ level updates on reset)
 
 
 def stable_penalty(dt_substep: float, m_ref: float = 0.3):
@@ -247,6 +278,11 @@ class DyrosCore:
                                         "program is plane only)")
             if hf.friction is not None:
                 self.cfg = replace(self.cfg, friction=float(hf.friction))
+        tc = self.cfg.terrain_curriculum
+        if tc is not None:
+            if not with_task:
+                raise native.DyrosError("terrain curriculum: needs the task (its reset stage moves the envs)")
+            tc.validate(int(num_envs))
         self.device = torch.device(device)
         self.tables = tables or ModelTables.load(os.path.join(ASSETS, "tocabi_tables.npz"))
         t = self.tables
@@ -319,6 +355,13 @@ class DyrosCore:
         tb["pert_duration"].fill_(1)
         tb["perturb_timing"].fill_(1)
         tb["motor_constant_scale"].fill_(1.0)
+        tc = cfg.terrain_curriculum
+        if tc is not None:
+            tb["terrain_origins"] = torch.tensor(np.asarray(tc.origins, np.float32), device=dev).contiguous()
+            tb["terrain_types"] = torch.tensor(np.asarray(tc.types, np.int32), device=dev)
+            tb["terrain_levels"] = torch.tensor(np.asarray(tc.levels, np.int32), device=dev)
+            if tc.curriculum:
+                tb["terrain_level_mean"] = torch.tensor(float(np.mean(tc.levels)), dtype=torch.float32, device=dev)
         tb["env_origins"].copy_(torch.tensor(self._env_origins()))
         if cfg.heightfield is not None:  # start where the first reset puts the root (T:734-735), not above (0, 0)
             s["root_states"][:, 0:3] = tb["env_origins"]
@@ -328,8 +371,17 @@ class DyrosCore:
         tb["act_hist_head"].fill_(19)
 
     def _env_origins(self) -> np.ndarray:
-        """T:709-718; on a heightfield the given origins, or the grid with z the terrain height there."""
-        hf = self.cfg.heightfield
+        """T:709-718; on a heightfield the given origins, or the grid with z the terrain height there; with a terrain
+        curriculum origins[levels, types] (every sub-terrain origin must then lie on the field)."""
+        hf, tc = self.cfg.heightfield, self.cfg.terrain_curriculum
+        if tc is not None:
+            table = np.asarray(tc.origins, np.float32)
+            if hf is not None:
+                inside = hf.height_at(table[..., 0], table[..., 1])[1]
+                if not inside.all():
+                    l, t = np.argwhere(~inside)[0]
+                    raise native.DyrosError(f"terrain curriculum: the origin of sub-terrain ({l}, {t}) lies outside the field")
+            return table[np.asarray(tc.levels), np.asarray(tc.types)]
         if hf is None:
             return env_origins(self.N, self.cfg.env_spacing)
         if hf.env_origins is not None:
@@ -433,6 +485,16 @@ class DyrosCore:
             setattr(tbuf, n, self.task_t[n].data_ptr() if n in self.task_t else None)
         native.check(self.lib.dyros_task_create(self.sim_handle, C.byref(td), C.byref(tbuf), C.byref(self.task_handle)),
                      "dyros_task_create")
+        tc = cfg.terrain_curriculum
+        if tc is not None and tc.curriculum:
+            tb = self.task_t
+            d = native.DyrosTerrainCurriculum()
+            d.origins, d.levels, d.types = (tb[k].data_ptr() for k in ("terrain_origins", "terrain_levels", "terrain_types"))
+            d.num_levels, d.num_types = tb["terrain_origins"].shape[:2]
+            d.move_up_distance, d.move_down_scale = tc.move_up_distance, tc.move_down_scale
+            d.level_mean = tb["terrain_level_mean"].data_ptr()
+            native.check(self.lib.dyros_task_set_terrain_curriculum(self.task_handle, C.byref(d)),
+                         "dyros_task_set_terrain_curriculum")
 
     def close(self):
         if getattr(self, "task_handle", None) and self.task_handle.value:

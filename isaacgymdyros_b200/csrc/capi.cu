@@ -425,6 +425,38 @@ int dyros_task_set_noise_injection(DyrosTask* task, const DyrosNoiseInjection* i
   }
   return 0;
 }
+int dyros_task_set_terrain_curriculum(DyrosTask* task, const DyrosTerrainCurriculum* c) {
+  TASK_OR_FAIL("dyros_task_set_terrain_curriculum");
+  if (!c) {
+    t->cur = DyrosTerrainCurriculum{};
+    return 0;
+  }
+  REQUIRE(c->origins && c->levels && c->types, "dyros_task_set_terrain_curriculum: origins, levels and types must be given");
+  REQUIRE(c->num_levels >= 1 && c->num_types >= 1, "dyros_task_set_terrain_curriculum: need num_levels >= 1 and num_types >= 1 "
+          "(got %d, %d)", c->num_levels, c->num_types);
+  REQUIRE(std::isfinite(c->move_up_distance) && c->move_up_distance >= 0 && std::isfinite(c->move_down_scale) &&
+              c->move_down_scale >= 0,
+          "dyros_task_set_terrain_curriculum: move_up_distance and move_down_scale must be finite and >= 0");
+  // the kernel indexes origins with levels / types: check them once here, from host copies
+  const int N = t->p.N;
+  const size_t no = (size_t)c->num_levels * c->num_types * 3;
+  std::vector<int32_t> lv(N), ty(N);
+  std::vector<float> org(no);
+  DY_CUDA(cudaSetDevice(t->sim->device));
+  DY_CUDA(cudaMemcpy(lv.data(), c->levels, N * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  DY_CUDA(cudaMemcpy(ty.data(), c->types, N * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  DY_CUDA(cudaMemcpy(org.data(), c->origins, no * sizeof(float), cudaMemcpyDeviceToHost));
+  for (int e = 0; e < N; ++e) {
+    REQUIRE(lv[e] >= 0 && lv[e] < c->num_levels, "dyros_task_set_terrain_curriculum: level %d of env %d outside [0, %d)",
+            lv[e], e, c->num_levels);
+    REQUIRE(ty[e] >= 0 && ty[e] < c->num_types, "dyros_task_set_terrain_curriculum: type %d of env %d outside [0, %d)",
+            ty[e], e, c->num_types);
+  }
+  for (size_t i = 0; i < no; ++i)
+    REQUIRE(std::isfinite(org[i]), "dyros_task_set_terrain_curriculum: origins must be finite");
+  t->cur = *c;
+  return 0;
+}
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream) {
   TASK_OR_FAIL("dyros_task_prologue");
   if (!actions) {

@@ -147,7 +147,8 @@ struct TaskParams {
   const float* init_dof_pos;
   const float* armature_base;
   uint64_t* step_counter;       // device, Philox epoch; bumped once per step by the cross-env pass
-  unsigned long long* tail;     // device [4]: fixed-point sums of the two gate means, CTA ticket of the fused post-physics launch
+  unsigned long long* tail;     // device [4]: fixed-point sums of the two gate means, CTA ticket of the fused post-physics
+                                // launch, sum of the terrain levels (curriculum)
   unsigned* scan_state;         // device [2 + ceil(N/1024)]: tile ticket, tiles finished, per-tile counts of the id compaction
 };
 
@@ -170,6 +171,7 @@ struct Task {
   TaskParams p;
   DyrosTaskBuffers b;
   DyrosNoiseInjection inj;
+  DyrosTerrainCurriculum cur{};  // dyros_task_set_terrain_curriculum; levels == NULL: off
   void* dev_blob = nullptr;
 };
 

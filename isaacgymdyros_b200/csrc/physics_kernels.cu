@@ -432,6 +432,7 @@ static int launch_task_physics_roles(Task* t, cudaStream_t s, long long* trace, 
   k.b = t->b;
   k.s = sim->b;
   k.j = t->inj;
+  k.c = t->cur;
   if (sim->has_field)
     DY_CUDA(launch_kernel(k_step_physics<FieldGround>, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p,
                           k, epb, env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions, sim->field));

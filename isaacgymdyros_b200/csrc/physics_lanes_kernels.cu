@@ -447,6 +447,7 @@ int launch_task_physics_lanes(Task* t, cudaStream_t s, long long* trace, bool pd
   k.b = t->b;
   k.s = sim->b;
   k.j = t->inj;
+  k.c = t->cur;
   DY_CUDA(launch_kernel(k_step_physics_lanes, dim3(grid), dim3(physics_step_threads_lanes(sim)), sim->phys_smem, s, pdl, sim->m, sim->p, k, epb,
                         env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions));
   return 0;

@@ -188,6 +188,30 @@ __device__ void stage_compute_reward(const TK& k, int e, int lane, const TermSha
   if (lane == 0) reward_scalar(k, e, sums);
 }
 
+// Terrain curriculum of one resetting env (legged_gym _update_terrain_curriculum; DESIGN.md section 4, "Curriculum"),
+// one thread: the new level from the root and the target_vel of the ending episode, then the env's new origin.
+__device__ __forceinline__ void stage_terrain_level(const TK& k, int e, uint64_t step) {
+  const DyrosTerrainCurriculum& C = k.c;
+  const float* root = k.s.root_states + (size_t)e * 13;
+  float* org = k.b.env_origins + (size_t)e * 3;
+  const float dx = root[0] - org[0], dy = root[1] - org[1];
+  const float d = sqrtf(dx * dx + dy * dy);
+  const float tvx = k.b.target_vel[(size_t)e * 2], tvy = k.b.target_vel[(size_t)e * 2 + 1];
+  const bool up = d > C.move_up_distance;
+  const bool down = !up && d < sqrtf(tvx * tvx + tvy * tvy) * C.move_down_scale;
+  int lvl = C.levels[e] + (up ? 1 : 0) - (down ? 1 : 0);
+  if (lvl >= C.num_levels) {  // past the top: a uniform level, from reset_f column 30
+    const float u = k.j.reset_f ? k.j.reset_f[(size_t)e * 32 + 30] : u01(draw4(k.p.seed, step, e, kSiteResetF, 7).z);
+    lvl = min((int)(u * (float)C.num_levels), C.num_levels - 1);
+  }
+  lvl = max(lvl, 0);
+  C.levels[e] = lvl;
+  const float* o = C.origins + ((size_t)lvl * C.num_types + C.types[e]) * 3;
+  org[0] = o[0];
+  org[1] = o[1];
+  org[2] = o[2];
+}
+
 // T:598-669, T:720-748 (+ DR re-draw of damping/armature, VT:519-733 / gymutil.py:584-619)
 __device__ void stage_reset_env(const TK& k, int e, int lane) {
   const TaskParams& P = k.p;
@@ -243,6 +267,10 @@ __device__ void stage_reset_env(const TK& k, int e, int lane) {
     k.b.action_torque_pre[(size_t)e * 12 + lane] = 0.f;                                            // T:636
   }
   if (lane < 3) k.b.quat_bias[(size_t)e * 3 + lane] = uf(12 + lane) * 6.28f / 150.f - (float)(3.14 / 150);  // T:616
+  if (k.c.levels) {  // before the root and target_vel are overwritten below
+    if (lane == 0) stage_terrain_level(k, e, step);
+    __syncwarp();
+  }
   if (lane < 13) {                                                                 // T:734-735
     float v = 0.f;
     if (lane < 3) v = k.b.env_origins[(size_t)e * 3 + lane];
@@ -492,6 +520,7 @@ __device__ __forceinline__ bool gate_open(const TaskParams& P, long long s0, lon
 constexpr int kPostWarps = 4;
 __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tail) {
   __shared__ long long gate_acc[2][kPostWarps];
+  __shared__ int level_acc[kPostWarps];
   pdl_launch_dependents();
   pdl_wait();
   const TaskParams& P = k.p;
@@ -670,10 +699,12 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     const uint64_t epoch = *P.step_counter;
     if (tail) {
       const bool gate = P.perturb != 0;
+      const bool lmean = k.c.levels && k.c.level_mean;  // mean terrain level: an integer sum, order-free like the gate's
       if (gate && lane == 0) {
         gate_acc[0][w] = gate_term0(ell);  // (post-reset values, as k_crossenv reads them)
         gate_acc[1][w] = gate_term1(crm);
       }
+      if (lmean && lane == 0) level_acc[w] = k.c.levels[e];  // (post-reset level: written by this thread)
       asm volatile("bar.sync 1, %0;" ::"r"(live_warps * 32) : "memory");
       if (threadIdx.x == 0) {
         if (gate) {
@@ -684,14 +715,20 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
           }
           atomicAdd(P.tail + 0, (unsigned long long)a);
           atomicAdd(P.tail + 1, (unsigned long long)b);
-          __threadfence();  // the sums before the ticket
         }
+        if (lmean) {
+          long long l = 0;
+          for (int i = 0; i < live_warps; ++i) l += level_acc[i];
+          atomicAdd(P.tail + 3, (unsigned long long)l);
+        }
+        if (gate || lmean) __threadfence();  // the sums before the ticket
         if (atomicAdd(P.tail + 2, 1ull) == gridDim.x - 1) {  // every CTA has published its sums and taken its epoch copy
           __threadfence();
           if (gate) {
             const long long s0 = (long long)atomicExch(P.tail + 0, 0ull), s1 = (long long)atomicExch(P.tail + 1, 0ull);
             if (gate_open(P, s0, s1)) *k.b.perturb_start = 1;  // T:489-490 (sticky)
           }
+          if (lmean) *k.c.level_mean = (float)((double)(long long)atomicExch(P.tail + 3, 0ull) / P.N);
           P.tail[2] = 0;
           *P.step_counter = epoch + 1;
         }
@@ -764,7 +801,7 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
 }
 
 // Cross-env pass: (a) reset_buf.nonzero() -> ascending ids (T:554) by warp ballot + prefix scan, multi-CTA;
-// (b) the curriculum gate means of T:489 (order-free fixed-point sums); (c) Philox epoch bump.
+// (b) the curriculum gate means of T:489 (order-free fixed-point sums) and the mean terrain level; (c) Philox epoch bump.
 //
 // Compaction: a CTA takes a tile of kScanTile consecutive envs (tile index = an atomic ticket, so a tile only ever waits
 // for tiles whose CTAs are already running); thread t reads reset_buf[tile * kScanTile + t] (coalesced), a warp ballot
@@ -783,6 +820,7 @@ __device__ __forceinline__ unsigned ld_acquire_gpu_u32(const unsigned* p) {
 __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, int do_gate, int do_bump) {
   __shared__ int warp_cnt[kScanTile / 32];
   __shared__ long long red[2][kScanTile / 32];
+  __shared__ int level_red[kScanTile / 32];
   __shared__ int s_tile, s_prefix;
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int N = k.p.N, ntiles = (N + kScanTile - 1) / kScanTile;
@@ -800,6 +838,8 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
   const int rank = __popc(bal & ((1u << lane) - 1u));
   long long s0 = (gate && valid) ? gate_term0(k.b.epi_len_log[e]) : 0;  // fixed-point terms: see gate_term0 / gate_term1
   long long s1 = (gate && valid) ? gate_term1(k.b.contact_reward_mean[e]) : 0;
+  const bool lmean = do_gate && k.c.levels && k.c.level_mean;  // mean terrain level (as k_post_fused: an integer sum)
+  int lv = (lmean && valid) ? k.c.levels[e] : 0;
   if (gate) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
@@ -807,10 +847,15 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
       s1 += __shfl_xor_sync(kFull, s1, o);
     }
   }
+  if (lmean) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lv += __shfl_xor_sync(kFull, lv, o);
+  }
   if (lane == 0) {
     warp_cnt[w] = __popc(bal);
     red[0][w] = s0;
     red[1][w] = s1;
+    level_red[w] = lv;
   }
   __syncthreads();
   if (w == 0) {
@@ -850,6 +895,12 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
         atomicAdd(k.p.tail + 1, (unsigned long long)b);
       }
     }
+    if (lmean) {
+      long long l = level_red[lane];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) l += __shfl_xor_sync(kFull, l, o);
+      if (lane == 0) atomicAdd(k.p.tail + 3, (unsigned long long)l);
+    }
   }
   __syncthreads();
   if (flag) {
@@ -869,6 +920,7 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
         const long long a = (long long)atomicExch(k.p.tail + 0, 0ull), b = (long long)atomicExch(k.p.tail + 1, 0ull);
         if (gate_open(k.p, a, b)) *k.b.perturb_start = 1;  // T:489-490 (sticky)
       }
+      if (lmean) *k.c.level_mean = (float)((double)(long long)atomicExch(k.p.tail + 3, 0ull) / N);
       if (do_bump) *k.p.step_counter = *k.p.step_counter + 1;
     }
   }
@@ -918,6 +970,7 @@ static inline TK make_tk(Task* t) {
   k.b = t->b;
   k.s = t->sim->b;
   k.j = t->inj;
+  k.c = t->cur;
   return k;
 }
 static inline int env_grid(int N) { return (N + kWarpsPerBlock - 1) / kWarpsPerBlock; }

@@ -12,6 +12,7 @@ struct TK {
   DyrosTaskBuffers b;
   DyrosSimBuffers s;
   DyrosNoiseInjection j;
+  DyrosTerrainCurriculum c;  // levels == NULL: no curriculum
 };
 
 // JU:374-395 with x_dot_0 = x_dot_f = 0.0 (T:458-461), reference operation order. The terms that depend on the knot

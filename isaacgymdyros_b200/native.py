@@ -94,6 +94,11 @@ class DyrosTaskDesc(C.Structure):
                 ("left_foot_body", i32), ("right_foot_body", i32), ("pelvis_body", i32), ("seed", u64)]
 
 
+class DyrosTerrainCurriculum(C.Structure):
+    _fields_ = [("origins", C.c_void_p), ("levels", C.c_void_p), ("types", C.c_void_p), ("num_levels", i32),
+                ("num_types", i32), ("move_up_distance", f32), ("move_down_scale", f32), ("level_mean", C.c_void_p)]
+
+
 NOISE_FIELDS = ["qpos_normal", "vel_u", "reset_f", "reset_i", "pert_i", "pert_f", "dr_u"]
 
 
@@ -161,6 +166,7 @@ SIGNATURES = {
     "dyros_task_create": (_INT, [_VP, C.POINTER(DyrosTaskDesc), C.POINTER(DyrosTaskBuffers), C.POINTER(_VP)]),
     "dyros_task_destroy": (_INT, [_VP]),
     "dyros_task_set_noise_injection": (_INT, [_VP, C.POINTER(DyrosNoiseInjection)]),
+    "dyros_task_set_terrain_curriculum": (_INT, [_VP, C.POINTER(DyrosTerrainCurriculum)]),
     "dyros_task_prologue": (_INT, [_VP, _VP, _VP]),
     "dyros_task_physics": (_INT, [_VP, _VP]),
     "dyros_task_physics_kernel": (_INT, [_VP, _VP]),

@@ -13,7 +13,9 @@ from typing import Any, Dict, Optional
 import numpy as np
 import torch
 
-from ..core import CoreConfig, DyrosCore, HeightField
+from .. import terrain as terrain_gen
+from ..core import CoreConfig, DyrosCore, HeightField, TerrainCurriculum
+from ..native import DyrosError
 from .spaces import Box
 
 REWARD_NAMES = ["mimic_body_orientation_reward", "qpos_regulation", "qvel_regulation", "contact_force_penalty",
@@ -57,7 +59,9 @@ def _default_cfg(num_envs: int, randomize: bool, perturbation: bool) -> Dict[str
     }
 
 
-def core_config_from_cfg(cfg: Dict[str, Any]) -> CoreConfig:
+def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generator] = None) -> CoreConfig:
+    """`generator` draws the envs' initial terrain levels when cfg["env"]["terrain"] is set (default: a CPU generator
+    seeded with 0)."""
     env, sim, task = cfg["env"], cfg["sim"], cfg.get("task", {})
     px = sim.get("physx", {})
     c = CoreConfig(dt=sim["dt"], substeps=sim.get("substeps", 1), control_freq_inv=env.get("controlFrequencyInv", 1),
@@ -80,6 +84,17 @@ def core_config_from_cfg(cfg: Dict[str, Any]) -> CoreConfig:
         c.heightfield = HeightField(np.asarray(hf["samples"]), float(hf["row_scale"]), float(hf["column_scale"]),
                                     float(hf["vertical_scale"]), tuple(hf.get("origin", (0.0, 0.0, 0.0))),
                                     friction=hf.get("friction"), env_origins=hf.get("env_origins"))
+    # (not a key of the reference's yaml either: its TerrainCfg, terrain_cfg.py:2-21, switched on. DESIGN.md section 4,
+    # "Curriculum")
+    tr = env.get("terrain")
+    if tr is not None:
+        tcfg = terrain_gen.TerrainConfig.from_dict(tr)
+        if tcfg.mesh_type in ("plane", "none"):
+            pass  # the plane z = 0, as without the key
+        elif hf is not None:
+            raise DyrosError('cfg["env"]: give either "heightfield" or "terrain", not both')
+        else:
+            _terrain_config(c, tcfg, int(env["numEnvs"]), generator)
     ap = task.get("randomization_params", {}).get("actor_params", {}).get("humanoid", {})
     dp = ap.get("dof_properties", {})
     if "damping" in dp:
@@ -98,6 +113,20 @@ def core_config_from_cfg(cfg: Dict[str, Any]) -> CoreConfig:
     if pg is not None:
         c.dr_pd_gain_range = tuple(pg["range"])
     return c
+
+
+def _terrain_config(c: CoreConfig, tcfg: "terrain_gen.TerrainConfig", n: int, generator: Optional[torch.Generator]):
+    """The generated field and the envs' sub-terrains (legged_gym's _get_env_origins): env e gets type
+    floor(e / (N / num_cols)) and a random initial level, in [0, max_init_terrain_level] with the curriculum, in
+    [0, num_rows) without."""
+    field, origins = terrain_gen.generate(tcfg)
+    g = generator if generator is not None else torch.Generator().manual_seed(0)
+    top = min(tcfg.max_init_terrain_level, tcfg.num_rows - 1) if tcfg.curriculum else tcfg.num_rows - 1
+    levels = torch.randint(0, top + 1, (n,), device=g.device, generator=g).cpu().numpy().astype(np.int32)
+    types = np.floor(np.arange(n) / (n / tcfg.num_cols)).astype(np.int32)
+    c.heightfield = field
+    c.terrain_curriculum = TerrainCurriculum(origins, types, levels, move_up_distance=tcfg.terrain_length / 2,
+                                             move_down_scale=c.episode_length_s * 0.5, curriculum=tcfg.curriculum)
 
 
 class DyrosDynamicWalk:
@@ -136,13 +165,13 @@ class DyrosDynamicWalk:
         self.max_episode_length_s = env["episodeLength"]
         self.death_cost, self.initial_height = env["deathCost"], env["initialHieght"]
         self.perturb = env["perturbation"]
-        self.core_cfg = core_config_from_cfg(cfg)
+        self.gen = torch.Generator(device=self.device)
+        self.gen.manual_seed(seed + rank)
+        self.core_cfg = core_config_from_cfg(cfg, self.gen)  # (draws the initial terrain levels, if any, from self.gen)
         self.dt, self.skipframe = self.core_cfg.dt, self.control_freq_inv
         self.dt_policy = self.dt * self.skipframe
         self.max_episode_length = self.max_episode_length_s / (self.dt * self.skipframe)  # T:35
         self.core = DyrosCore(self.num_environments, self.device, self.core_cfg, seed=seed, rank=rank)
-        self.gen = torch.Generator(device=self.device)
-        self.gen.manual_seed(seed + rank)
         self._bind_buffers()
         self._initial_randoms()
         self.extras: Dict[str, Any] = {}
@@ -188,6 +217,10 @@ class DyrosDynamicWalk:
         self.dof_vel = s["dof_state"].view(N, 33, 2)[..., 1]
         self.contact_forces = s["net_contact_force"].view(N, 38, 3)
         self.stacked_rewards = t["stacked_rewards"]
+        # terrain (cfg["env"]["terrain"]): level (row) and type (column) of each env's sub-terrain, the sub-terrain
+        # origins; with the curriculum the reset stage updates terrain_levels and terrain_level_mean
+        self.terrain_levels, self.terrain_types = t.get("terrain_levels"), t.get("terrain_types")
+        self.terrain_origins, self.terrain_level_mean = t.get("terrain_origins"), t.get("terrain_level_mean")
         for k in ("actions", "actions_pre", "time", "target_vel", "motor_constant_scale", "qpos_noise", "qvel_noise",
                   "qpos_bias", "quat_bias", "epi_len", "epi_len_log", "contact_reward_mean", "total_mass"):
             setattr(self, k, t[k])
@@ -243,6 +276,8 @@ class DyrosDynamicWalk:
         self.extras["time_outs"] = self.timeout_buf.to(self.rl_device)
         self.extras["stacked_rewards"] = self.stacked_rewards
         self.extras["reward_names"] = REWARD_NAMES
+        if self.terrain_level_mean is not None:  # legged_gym's episode log; written by the step's kernels
+            self.extras.setdefault("episode", {})["terrain_level"] = self.terrain_level_mean
         self.obs_dict["obs"] = self._obs_out()
         return self.obs_dict, self.rew_buf.to(self.rl_device), self.reset_buf.to(self.rl_device), self.extras
 

@@ -1,10 +1,13 @@
-"""What a heightfield ground costs: the fused DyrosDynamicWalk step at 4096 envs (default task, CUDA graph) on four
+"""What a heightfield ground costs: the fused DyrosDynamicWalk step at 4096 envs (default task, CUDA graph) on six
 grounds, timed alternately in one process with the L2 flushed between timed steps (dyros_flush_l2, as bench.py does):
-  plane   the plane z = 0 (the default build path)
-  flat    a heightfield of zeros (same contacts as the plane, heightfield code path)
-  rough   uniform heights in [-5 cm, +5 cm] at 0.1 m spacing
-  stairs  5 cm steps every 0.3 m along x (0.05 m spacing)
-Every field covers the default env grid (T:709-718); the envs stand on it at their origins. Also prints the per-phase
+  plane      the plane z = 0 (the default build path)
+  flat       a heightfield of zeros (same contacts as the plane, heightfield code path)
+  rough      uniform heights in [-5 cm, +5 cm] at 0.1 m spacing
+  stairs     5 cm steps every 0.3 m along x (0.05 m spacing)
+  generated  the terrain generator's default grid (isaacgymdyros_b200/terrain.py: 10 levels x 20 types of 8 m, 0.1 m
+             spacing), envs fixed on their sub-terrains (terrain curriculum: False)
+  curriculum the same field with the terrain curriculum: levels move on every reset
+The first four fields cover the default env grid (T:709-718); the envs stand on them at their origins. Also prints the per-phase
 clock64() breakdown of the physics kernel (CTA 0, per role; marks of physics_roles.cuh, as tools/trace_physics.py)
 and the card's name and power limit. TOCABI's roles: 0 torso + left arm, 1 head + right arm + base, 2 left leg,
 3 right leg (only the two legs have contact phases).
@@ -65,11 +68,13 @@ def main():
     N = a.envs
     name, power = card()
     print(f"card: {name}; power limit, max SM clock: {power}", flush=True)
-    kinds = ["plane", "flat", "rough", "stairs"]
+    kinds = ["plane", "flat", "rough", "stairs", "generated", "curriculum"]
     envs = {}
     for k in kinds:
         cfg = default_cfg(N)
-        if k != "plane":
+        if k in ("generated", "curriculum"):
+            cfg["env"]["terrain"] = {"curriculum": k == "curriculum"}
+        elif k != "plane":
             cfg["env"]["heightfield"] = field(k, N)
         envs[k] = DyrosDynamicWalk(cfg, "cuda:0")
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda:0")
@@ -82,7 +87,7 @@ def main():
     torch.cuda.synchronize()
     times = {k: [] for k in kinds}
     for r in range(a.rounds):
-        for k in kinds:  # alternating: the four grounds see the same machine state
+        for k in kinds:  # alternating: the grounds see the same machine state
             env = envs[k]
             ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.steps)]
             for i in range(a.steps):
