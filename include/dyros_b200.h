@@ -128,7 +128,7 @@ typedef struct {
 /* Per-env task state (names = the reference attributes, T:87-195; internal integers are int32). */
 typedef struct {
   /* VecTask API buffers (VT:242-255) */
-  float* obs_buf;            /* (N,487) */
+  float* obs_buf;            /* (N,487); (N,487+P) with a height scan of P points (dyros_task_set_height_scan) */
   float* rew_buf;            /* (N) */
   int64_t* reset_buf;        /* (N) */
   int64_t* timeout_buf;      /* (N) */
@@ -309,6 +309,25 @@ typedef struct {
   float* level_mean;         /* (1) mean level after each step's resets; may be NULL */
 } DyrosTerrainCurriculum;
 int dyros_task_set_terrain_curriculum(DyrosTask* task, const DyrosTerrainCurriculum* curriculum);
+/* Height scan (legged_gym's measure_heights; DESIGN.md section 4, "Height scan"): the observation row gains P columns,
+ * obs[e, 487 + k] = clip(root_z - base_offset - h_k, -1, 1) * scale. h_k is the terrain height under point k, the point
+ * (points[k].x, points[k].y, 0) of the base's yaw frame carried to the world: rotated by the yaw of the root quaternion,
+ * shifted by the root's x-y. On a heightfield h_k is the lowest of the three samples legged_gym reads at the clamped
+ * cell index (not the triangle the physics touches); on the plane it is 0. The heights are those of the root the rest
+ * of the row describes (post-reset for an env reset in the step). measured_heights, if given, receives h_k in m.
+ * The field is the sim's at each launch (dyros_sim_set_heightfield). From this call on, obs_buf and every later
+ * dyros_task_set_obs_buf target must hold N*(487+P) floats, and dyros_task_pack_results writes the wider rows. Call
+ * before a CUDA graph of the step is captured: captured launches keep the setting they were captured with. NULL
+ * switches the scan off (rows of 487 floats again). All pointers are caller-owned DEVICE memory that must stay alive
+ * while the task uses them. */
+typedef struct {
+  const float* points;       /* (P,2) x, y in the base's yaw frame (m) */
+  int32_t num_points;        /* P, 1..1024 */
+  float base_offset;         /* 0.5 */
+  float scale;               /* obs_scales.height_measurements, 5.0 */
+  float* measured_heights;   /* (N,P) h_k in m; may be NULL */
+} DyrosHeightScan;
+int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* scan);
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream);      /* VT:307 + T:449-502 */
 /* T:504-530 in one launch: skipframe x (substep torque, gym.simulate, sensor noise); what dyros_task_step uses. */
 int dyros_task_physics(DyrosTask* task, void* stream);
@@ -342,11 +361,13 @@ int dyros_task_post_step(DyrosTask* task, void* stream);
 /* Number of kernel launches dyros_task_step enqueues (for bench.py's gpu_launches). */
 int dyros_task_step_launches(DyrosTask* task);
 /* What VecTask.step returns (VT:336-344: obs_dict["obs"], rew_buf, reset_buf, extras["time_outs"]) gathered into ONE
- * contiguous device block `dst` of N*(487*4 + 4 + 8 + 8) bytes, 16-byte aligned:
- * obs (N,487) f32 | rew (N) f32 | reset (N) i64 | time_outs (N) i64. A host-side
+ * contiguous device block `dst`, 16-byte aligned, with W = 487 (+ P with a height scan):
+ * obs (N,W) f32 | rew (N) f32 | [4 bytes of padding if N*(W+1) is odd] | reset (N) i64 | time_outs (N) i64,
+ * i.e. the i64 part starts at N*(W+1)*4 rounded up to a multiple of 8 (N*488*4 without a scan). A host-side
  * caller then moves the block with a single device->host copy on its own stream while the next step runs. */
 int dyros_task_pack_results(DyrosTask* task, void* dst, void* stream);
-/* Re-points the observation buffer (DyrosTaskBuffers.obs_buf, (N,487) f32, 16-byte aligned) for the launches enqueued
+/* Re-points the observation buffer (DyrosTaskBuffers.obs_buf, (N,487) f32, or (N,487+P) with a height scan; 16-byte
+ * aligned) for the launches enqueued
  * from now on; launches already enqueued or captured in a CUDA graph keep the pointer they were given. With obs_buf
  * set to a result block, dyros_task_pack_results on that block only adds rew / reset / time_outs. */
 int dyros_task_set_obs_buf(DyrosTask* task, float* obs_buf);

@@ -20,6 +20,10 @@ from .model.tables import ModelTables, role_programs
 
 ASSETS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "assets")
 ND, NB, NA = 33, 38, 13
+NOBS = 487  # columns of an observation row without a height scan
+# height scan (legged_gym's measure_heights): obs = clip(root_z - BASE_OFFSET - h, -1, 1) * SCALE
+HEIGHT_SCAN_BASE_OFFSET, HEIGHT_SCAN_SCALE = 0.5, 5.0  # _get_heights / compute_observations, obs_scales.height_measurements
+MAX_HEIGHT_POINTS = 1024
 
 # T:58-70 (before the /9 and /3), T:296-301, T:95-100, T:366-371
 KP = [2000.0, 5000.0, 4000.0, 3700.0, 3200.0, 3200.0, 2000.0, 5000.0, 4000.0, 3700.0, 3200.0, 3200.0,
@@ -155,6 +159,18 @@ class CoreConfig:
     self_collision: bool = True          # create_actor(..., filter 0), T:354: the actor's shapes collide with each other
     heightfield: Optional[HeightField] = None  # ground: None = the plane z = 0 (gym.add_ground), else gym.add_heightfield
     terrain_curriculum: Optional[TerrainCurriculum] = None  # env origins on sub-terrains (+ level updates on reset)
+    # (P, 2) points of the height scan in the base's yaw frame (legged_gym's height_points; DESIGN.md section 4, "Height
+    # scan"), or None: each observation row gains P terrain heights around the base, on any ground
+    height_scan: Optional[np.ndarray] = None
+
+
+def validate_height_points(points) -> np.ndarray:
+    """(P, 2) finite float32 points, 1 <= P <= 1024, or DyrosError."""
+    p = np.asarray(points, np.float64)
+    if p.ndim != 2 or p.shape[1] != 2 or not 1 <= p.shape[0] <= MAX_HEIGHT_POINTS or not np.all(np.isfinite(p)):
+        raise native.DyrosError(f"height scan: points must be a finite (P, 2) array with 1 <= P <= {MAX_HEIGHT_POINTS} "
+                                f"(got shape {p.shape})")
+    return np.ascontiguousarray(p, np.float32)
 
 
 def stable_penalty(dt_substep: float, m_ref: float = 0.3):
@@ -283,6 +299,13 @@ class DyrosCore:
             if not with_task:
                 raise native.DyrosError("terrain curriculum: needs the task (its reset stage moves the envs)")
             tc.validate(int(num_envs))
+        self.height_points = None
+        if self.cfg.height_scan is not None:
+            if not with_task:
+                raise native.DyrosError("height scan: needs the task (its observation kernels measure the heights)")
+            self.height_points = validate_height_points(self.cfg.height_scan)
+        self.num_height_points = 0 if self.height_points is None else len(self.height_points)
+        self.obs_width = NOBS + self.num_height_points  # columns of obs_buf
         self.device = torch.device(device)
         self.tables = tables or ModelTables.load(os.path.join(ASSETS, "tocabi_tables.npz"))
         t = self.tables
@@ -340,6 +363,10 @@ class DyrosCore:
             tb[name] = torch.zeros(full, dtype=getattr(torch, dt), device=dev)
         if cfg.dr_pd_gain_range is not None:
             tb["pd_gain_scale"] = torch.ones(N, 2, device=dev)
+        if self.height_points is not None:  # wider rows; measured_heights (N, P) = legged_gym's self.measured_heights
+            tb["obs_buf"] = z(N, self.obs_width)
+            tb["measured_heights"] = z(N, self.num_height_points)
+            tb["height_points"] = torch.tensor(self.height_points, device=dev)
         mocap = np.load(os.path.join(ASSETS, "mocap_walk.npy"))
         obs_norm = np.load(os.path.join(ASSETS, "obs_norm.npy"))
         tb["mocap_data"] = torch.tensor(mocap, device=dev).contiguous()
@@ -399,9 +426,9 @@ class DyrosCore:
         return o.astype(np.float32)
 
     def _pack_state_arena(self):
-        """Moves every per-env buffer except obs_buf (written once per step, never read by the step) into ONE
-        contiguous allocation, 256-byte aligned views: the range dyros_sim_set_l2_persistence can pin in L2."""
-        items = [(d, k) for d in (self.sim_t, self.task_t) for k in d if k != "obs_buf"]
+        """Moves every per-env buffer except obs_buf and measured_heights (written once per step, never read by the step)
+        into ONE contiguous allocation, 256-byte aligned views: the range dyros_sim_set_l2_persistence can pin in L2."""
+        items = [(d, k) for d in (self.sim_t, self.task_t) for k in d if k not in ("obs_buf", "measured_heights")]
         al = lambda n: (n + 255) & ~255
         total = sum(al(d[k].numel() * d[k].element_size()) for d, k in items)
         self.state_arena = torch.zeros(total, dtype=torch.uint8, device=self.device)
@@ -495,6 +522,12 @@ class DyrosCore:
             d.level_mean = tb["terrain_level_mean"].data_ptr()
             native.check(self.lib.dyros_task_set_terrain_curriculum(self.task_handle, C.byref(d)),
                          "dyros_task_set_terrain_curriculum")
+        if self.height_points is not None:
+            d = native.DyrosHeightScan()
+            d.points, d.num_points = self.task_t["height_points"].data_ptr(), self.num_height_points
+            d.base_offset, d.scale = HEIGHT_SCAN_BASE_OFFSET, HEIGHT_SCAN_SCALE
+            d.measured_heights = self.task_t["measured_heights"].data_ptr()
+            native.check(self.lib.dyros_task_set_height_scan(self.task_handle, C.byref(d)), "dyros_task_set_height_scan")
 
     def close(self):
         if getattr(self, "task_handle", None) and self.task_handle.value:
@@ -549,12 +582,21 @@ class DyrosCore:
     def set_obs_buf(self, obs: torch.Tensor):
         """Observation buffer of the launches enqueued from now on (dyros_task_set_obs_buf); `obs` may be the head of a
         result block, pack_results on that block then only adds rew / reset / time_outs."""
-        if obs.device != self.device or not obs.is_contiguous() or obs.numel() * obs.element_size() < self.N * 487 * 4:
-            raise native.DyrosError(f"set_obs_buf needs a contiguous block of {self.N * 487 * 4} bytes on {self.device}")
+        need = self.N * self.obs_width * 4
+        if obs.device != self.device or not obs.is_contiguous() or obs.numel() * obs.element_size() < need:
+            raise native.DyrosError(f"set_obs_buf needs a contiguous block of {need} bytes on {self.device}")
         native.check(self.lib.dyros_task_set_obs_buf(self.task_handle, C.c_void_p(obs.data_ptr())), "dyros_task_set_obs_buf")
 
+    def result_offsets(self):
+        """Byte offsets of rew, reset and time_outs in a pack_results block, and its size: obs (N, obs_width) f32 |
+        rew (N) f32 | reset (N) i64 | time_outs (N) i64, the i64 part 8-byte aligned."""
+        N = self.N
+        rew = N * self.obs_width * 4
+        rst = (rew + N * 4 + 7) & ~7
+        return rew, rst, rst + N * 8, rst + N * 16
+
     def result_bytes(self) -> int:
-        return self.N * (487 * 4 + 4 + 8 + 8)
+        return self.result_offsets()[3]
 
     def step_launches(self) -> int:
         return int(self.lib.dyros_task_step_launches(self.task_handle))

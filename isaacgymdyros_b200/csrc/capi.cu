@@ -457,6 +457,25 @@ int dyros_task_set_terrain_curriculum(DyrosTask* task, const DyrosTerrainCurricu
   t->cur = *c;
   return 0;
 }
+int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* sc) {
+  TASK_OR_FAIL("dyros_task_set_height_scan");
+  if (!sc) {
+    t->scan = DyrosHeightScan{};
+    return 0;
+  }
+  REQUIRE(sc->points && (reinterpret_cast<uintptr_t>(sc->points) & 7) == 0,
+          "dyros_task_set_height_scan: points is NULL or not 8-byte aligned");
+  REQUIRE(sc->num_points >= 1 && sc->num_points <= 1024, "dyros_task_set_height_scan: num_points %d outside [1, 1024]",
+          sc->num_points);
+  REQUIRE(std::isfinite(sc->base_offset) && std::isfinite(sc->scale),
+          "dyros_task_set_height_scan: base_offset and scale must be finite");
+  std::vector<float> pts((size_t)sc->num_points * 2);
+  DY_CUDA(cudaSetDevice(t->sim->device));
+  DY_CUDA(cudaMemcpy(pts.data(), sc->points, pts.size() * sizeof(float), cudaMemcpyDeviceToHost));
+  for (float v : pts) REQUIRE(std::isfinite(v), "dyros_task_set_height_scan: points must be finite");
+  t->scan = *sc;
+  return 0;
+}
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream) {
   TASK_OR_FAIL("dyros_task_prologue");
   if (!actions) {

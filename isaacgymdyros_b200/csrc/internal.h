@@ -107,6 +107,22 @@ struct FieldGround {
   float cull;              // 1 / (smallest n_z of any triangle) >= 1: see link_ext_wrench
 };
 
+// The height scan of the observation kernels (DESIGN.md section 4, "Height scan"), a compile-time parameter of
+// k_post_fused and k_compute_observations like the ground of the physics kernels: none (rows of NOBS floats), or P
+// terrain heights around the base appended to each row.
+struct NoScan {
+  static constexpr bool kOn = false;
+};
+struct HeightScan {
+  static constexpr bool kOn = true;
+  const float2* points;    // (P) x-y in the base's yaw frame (device memory)
+  int P;                   // 1..1024
+  float base_offset, scale;
+  float* measured;         // (N, P) heights in m, or NULL
+  int has_field;           // 0: the plane z = 0 (every height 0)
+  FieldGround f;           // the sim's heightfield when has_field
+};
+
 struct SimParams {
   int N;
   float dt;       // dt / substeps: the integration step of one sub-step
@@ -172,7 +188,9 @@ struct Task {
   DyrosTaskBuffers b;
   DyrosNoiseInjection inj;
   DyrosTerrainCurriculum cur{};  // dyros_task_set_terrain_curriculum; levels == NULL: off
+  DyrosHeightScan scan{};        // dyros_task_set_height_scan; num_points == 0: off
   void* dev_blob = nullptr;
+  int obs_width() const { return NOBS + scan.num_points; }
 };
 
 // launchers (task_kernels.cu)
@@ -187,7 +205,7 @@ int launch_reset_idx(Task* t, const int64_t* env_ids, int count, cudaStream_t s)
 int launch_compute_observations(Task* t, cudaStream_t s);
 int launch_late_update(Task* t, cudaStream_t s);
 int launch_post_fused(Task* t, cudaStream_t s, bool pdl = false, bool tail = false);
-int launch_pack_results(Task* t, float* dst, cudaStream_t s);
+int launch_pack_results(Task* t, float* dst, cudaStream_t s);  // rows of t->obs_width() floats
 // launchers (physics_kernels.cu)
 int physics_configure(Sim* sim);  // chooses envs_per_block / shared memory, sets the kernel attributes
 int launch_simulate(Sim* sim, int apply_wrench, const float* push_force, cudaStream_t s);

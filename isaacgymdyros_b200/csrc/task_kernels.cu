@@ -316,8 +316,58 @@ __device__ void stage_reset_env(const TK& k, int e, int lane) {
   }
 }
 
-// T:750-796 (history kept as rings, see DyrosTaskBuffers)
-__device__ void stage_compute_observations(const TK& k, int e, int lane) {
+// Width of an observation row: NOBS, plus the P heights of a height scan
+__host__ __device__ constexpr int obs_width(const NoScan&) { return NOBS; }
+__host__ __device__ inline int obs_width(const HeightScan& sc) { return NOBS + sc.P; }
+
+// Height scan of one env (DESIGN.md section 4, "Height scan": legged_gym's _get_heights, quat_apply_yaw and the height
+// term of compute_observations), one warp: lane l takes points l, l + 32, ...; the sample gathers of up to kScanBatch
+// points per lane (all of them for P <= 256) are issued before the first is used. (x, y, z) is the root's position,
+// (qz, qw) the z and w components of its quaternion, `ob` the env's observation row (columns NOBS + k are written).
+constexpr int kScanBatch = 8;
+__device__ __forceinline__ void stage_height_scan(const HeightScan& sc, int e, int lane, float x, float y, float z,
+                                                  float qz, float qw, float* ob) {
+  const float n = fmaxf(sqrtf(qz * qz + qw * qw), 1e-9f);  // TU normalize of the quaternion with x = y = 0
+  const float yz = qz / n, yw = qw / n;
+  const float zb = z - sc.base_offset;
+  const FieldGround& f = sc.f;
+  float* mh = sc.measured ? sc.measured + (size_t)e * sc.P : nullptr;
+  for (int k0 = 0; k0 < sc.P; k0 += kWarp * kScanBatch) {
+    int s0[kScanBatch], s1[kScanBatch], s2[kScanBatch];
+#pragma unroll
+    for (int b = 0; b < kScanBatch; ++b) {
+      const int k = min(k0 + lane + b * kWarp, sc.P - 1);  // (past the end: a repeat of the last point, not stored)
+      const float2 p = __ldg(sc.points + k);
+      // TU quat_apply((0, 0, yz, yw), (p.x, p.y, 0)) = v + w t + cross(xyz, t), t = cross(xyz, v) * 2; the left-out
+      // terms have a zero factor and add exact zeros
+      const float tx = -(yz * p.y) * 2.0f, ty = (yz * p.x) * 2.0f;
+      const float wx = ((p.x + yw * tx) - yz * ty) + x;
+      const float wy = ((p.y + yw * ty) + yz * tx) + y;
+      s0[b] = s1[b] = s2[b] = 0;
+      if (sc.has_field) {  // cell index trunc((w - p) / scale), clamped to the field: off it, the edge's samples
+        const int px = (int)fminf(fmaxf((wx - f.ox) / f.dx, 0.0f), (float)(f.nr - 2));
+        const int py = (int)fminf(fmaxf((wy - f.oy) / f.dy, 0.0f), (float)(f.nc - 2));
+        const int16_t* c = f.s + (size_t)px * f.nc + py;
+        s0[b] = __ldg(c);
+        s1[b] = __ldg(c + f.nc);
+        s2[b] = __ldg(c + 1);
+      }
+    }
+#pragma unroll
+    for (int b = 0; b < kScanBatch; ++b) {
+      const int k = k0 + lane + b * kWarp;
+      if (k < sc.P) {
+        const float h = sc.has_field ? f.oz + f.dz * (float)min(min(s0[b], s1[b]), s2[b]) : 0.0f;  // plane: 0
+        ob[NOBS + k] = fminf(fmaxf(zb - h, -1.0f), 1.0f) * sc.scale;
+        if (mh) mh[k] = h;
+      }
+    }
+  }
+}
+
+// T:750-796 (history kept as rings, see DyrosTaskBuffers), then the height scan if there is one
+template <class Scan>
+__device__ void stage_compute_observations(const TK& k, int e, int lane, const Scan& sc) {
   const TaskParams& P = k.p;
   const float* root = k.s.root_states + (size_t)e * 13;
   float time = k.b.time[e];
@@ -354,7 +404,9 @@ __device__ void stage_compute_observations(const TK& k, int e, int lane) {
   }
   __syncwarp();
   if (lane == 0) k.b.obs_hist_head[e] = head;
-  float* ob = k.b.obs_buf + (size_t)e * NOBS;
+  float* ob;
+  if constexpr (Scan::kOn) ob = k.b.obs_buf + (size_t)e * obs_width(sc);
+  else ob = k.b.obs_buf + (size_t)e * NOBS;  // (spelt out: the default instantiation keeps its instruction stream)
   const float* ah = k.b.action_history + (size_t)e * NSLOT * NA;
   int ahead = k.b.act_hist_head[e];
   // gather: all loads first (the compiler cannot reorder them across the stores itself), then the stores
@@ -382,6 +434,7 @@ __device__ void stage_compute_observations(const TK& k, int e, int lane) {
     int o = lane + it * kWarp;
     if (o < NOBS) ob[o] = vals[it];
   }
+  if constexpr (Scan::kOn) stage_height_scan(sc, e, lane, root[0], root[1], root[2], root[5], root[6], ob);
 }
 
 // T:560-563 (loads of all four copies are issued before the first store)
@@ -456,9 +509,10 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_reset_idx(TK k, const i
   if (e < 0 || e >= k.p.N) return;
   stage_reset_env(k, (int)e, lane);
 }
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_compute_observations(TK k) {
+template <class Scan>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_compute_observations(TK k, Scan sc) {
   ENV_LANE();
-  stage_compute_observations(k, e, lane);
+  stage_compute_observations(k, e, lane, sc);
 }
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_late_update(TK k) {
   ENV_LANE();
@@ -517,8 +571,10 @@ __device__ __forceinline__ bool gate_open(const TaskParams& P, long long s0, lon
 }
 
 // 4 warps per CTA, 7 CTAs per SM: 4096 envs (1024 CTAs) are resident on 148 SMs in ONE wave at <= 73 registers per thread
+// (instantiated without and with the height scan, which runs last, from the post-reset root of the observation stage)
 constexpr int kPostWarps = 4;
-__global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tail) {
+template <class Scan>
+__global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tail, Scan sc) {
   __shared__ long long gate_acc[2][kPostWarps];
   __shared__ int level_acc[kPostWarps];
   pdl_launch_dependents();
@@ -777,7 +833,7 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
       if (lane == 0) k.b.obs_hist_head[e] = head;
     }
     {
-      float* ob = k.b.obs_buf + E * NOBS;
+      float* ob = k.b.obs_buf + E * obs_width(sc);
 #pragma unroll
       for (int i = 0; i < NHIS; ++i) {                                                 // T:789-791
         const bool newest = start || i == NHIS - 1;                                    // (T:786-787: at an episode start every slot holds this frame)
@@ -796,6 +852,11 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     if (lane == P.lfoot || lane == P.rfoot) {                                          // the rows the reward reads
       float* o = k.b.contact_forces_pre + E * NB * 3 + 3 * lane;
       o[0] = fA0; o[1] = fA1; o[2] = fA2;
+    }
+    // ================================================================ height scan (DESIGN.md section 4)
+    if constexpr (Scan::kOn) {
+      const float rx = __shfl_sync(kFull, in.root, 0), ry = __shfl_sync(kFull, in.root, 1), rz = __shfl_sync(kFull, in.root, 2);
+      stage_height_scan(sc, e, lane, rx, ry, rz, quat[2], quat[3], k.b.obs_buf + E * obs_width(sc));
     }
   }
 }
@@ -928,13 +989,13 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
 
 
 // ------------------------------------------------------------------ results of a step -> one contiguous block
-// Layout of `dst`: obs (N,487) f32 | rew (N) f32 | reset (N) i64 | time_outs (N) i64 (the i64 part starts at
-// N*488*4, a multiple of 8). The host-facing
+// Layout of `dst`: obs (N,W) f32 | rew (N) f32 | reset (N) i64 | time_outs (N) i64, W = NOBS (+ P with a height scan);
+// the i64 part starts at N*(W+1)*4 rounded up to a multiple of 8 (N*488*4 for W = NOBS). The host-facing
 // step (DyrosDynamicWalk.step_async) hands this block to the copy engine as ONE device->host transfer on a second
 // stream, so the next step may overwrite obs_buf / rew_buf / reset_buf / timeout_buf (VT:336-344) while the block is still in flight.
-__global__ void __launch_bounds__(256) k_pack_results(TK k, float* __restrict__ dst) {
+__global__ void __launch_bounds__(256) k_pack_results(TK k, float* __restrict__ dst, int W) {
   const int N = k.p.N;
-  const size_t n_obs = (size_t)N * 487;
+  const size_t n_obs = (size_t)N * W;
   const size_t tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (size_t)gridDim.x * blockDim.x;
   const size_t n4 = n_obs / 4;  // obs_buf and dst are 16-byte aligned (torch allocations)
   const float4* src4 = reinterpret_cast<const float4*>(k.b.obs_buf);
@@ -955,7 +1016,7 @@ __global__ void __launch_bounds__(256) k_pack_results(TK k, float* __restrict__ 
     for (size_t i = n4 * 4 + tid; i < n_obs; i += nth) dst[i] = k.b.obs_buf[i];
   }
   float* rew = dst + n_obs;
-  long long* rst = reinterpret_cast<long long*>(dst + n_obs + N);
+  long long* rst = reinterpret_cast<long long*>(dst + ((n_obs + N + 1) & ~(size_t)1));
   for (size_t e = tid; e < (size_t)N; e += nth) {
     rew[e] = k.b.rew_buf[e];
     rst[e] = k.b.reset_buf[e];
@@ -973,6 +1034,17 @@ static inline TK make_tk(Task* t) {
   k.c = t->cur;
   return k;
 }
+static inline HeightScan make_scan(const Task* t) {
+  HeightScan sc;
+  sc.points = reinterpret_cast<const float2*>(t->scan.points);
+  sc.P = t->scan.num_points;
+  sc.base_offset = t->scan.base_offset;
+  sc.scale = t->scan.scale;
+  sc.measured = t->scan.measured_heights;
+  sc.has_field = t->sim->has_field ? 1 : 0;  // the sim's ground at this launch (dyros_sim_set_heightfield)
+  sc.f = t->sim->field;
+  return sc;
+}
 static inline int env_grid(int N) { return (N + kWarpsPerBlock - 1) / kWarpsPerBlock; }
 #define LAUNCH_ENV(kern, ...)                                                    \
   kern<<<env_grid(t->p.N), kWarpsPerBlock * 32, 0, s>>>(make_tk(t), ##__VA_ARGS__); \
@@ -985,19 +1057,28 @@ int launch_sensor_noise(Task* t, int substep, cudaStream_t s) { LAUNCH_ENV(k_sen
 int launch_epilogue(Task* t, cudaStream_t s) { LAUNCH_ENV(k_epilogue) }
 int launch_check_termination(Task* t, cudaStream_t s) { LAUNCH_ENV(k_check_termination) }
 int launch_compute_reward(Task* t, cudaStream_t s) { LAUNCH_ENV(k_compute_reward) }
-int launch_compute_observations(Task* t, cudaStream_t s) { LAUNCH_ENV(k_compute_observations) }
+int launch_compute_observations(Task* t, cudaStream_t s) {
+  if (t->scan.num_points) { LAUNCH_ENV(k_compute_observations<HeightScan>, make_scan(t)) }
+  LAUNCH_ENV(k_compute_observations<NoScan>, NoScan())
+}
 int launch_late_update(Task* t, cudaStream_t s) { LAUNCH_ENV(k_late_update) }
 int configure_task_kernels() {
   DY_CUDA(prefer_max_smem_carveout(k_prologue)); DY_CUDA(prefer_max_smem_carveout(k_substep_torque));
   DY_CUDA(prefer_max_smem_carveout(k_sensor_noise)); DY_CUDA(prefer_max_smem_carveout(k_epilogue));
   DY_CUDA(prefer_max_smem_carveout(k_check_termination)); DY_CUDA(prefer_max_smem_carveout(k_compute_reward));
-  DY_CUDA(prefer_max_smem_carveout(k_compute_observations)); DY_CUDA(prefer_max_smem_carveout(k_late_update));
+  DY_CUDA(prefer_max_smem_carveout(k_compute_observations<NoScan>));
+  DY_CUDA(prefer_max_smem_carveout(k_compute_observations<HeightScan>)); DY_CUDA(prefer_max_smem_carveout(k_late_update));
   DY_CUDA(prefer_max_smem_carveout(k_reset_idx)); DY_CUDA(prefer_max_smem_carveout(k_pack_results));
-  DY_CUDA(prefer_max_smem_carveout(k_post_fused)); DY_CUDA(prefer_max_smem_carveout(k_crossenv));
+  DY_CUDA(prefer_max_smem_carveout(k_post_fused<NoScan>)); DY_CUDA(prefer_max_smem_carveout(k_post_fused<HeightScan>));
+  DY_CUDA(prefer_max_smem_carveout(k_crossenv));
   return 0;
 }
 int launch_post_fused(Task* t, cudaStream_t s, bool pdl, bool tail) {
-  DY_CUDA(launch_kernel(k_post_fused, dim3((t->p.N + kPostWarps - 1) / kPostWarps), dim3(kPostWarps * 32), 0, s, pdl, make_tk(t), (int)tail));
+  const dim3 grid((t->p.N + kPostWarps - 1) / kPostWarps), block(kPostWarps * 32);
+  if (t->scan.num_points)
+    DY_CUDA(launch_kernel(k_post_fused<HeightScan>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t)));
+  else
+    DY_CUDA(launch_kernel(k_post_fused<NoScan>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan()));
   return 0;
 }
 int launch_reset_idx(Task* t, const int64_t* env_ids, int count, cudaStream_t s) {
@@ -1010,7 +1091,7 @@ int launch_reset_idx(Task* t, const int64_t* env_ids, int count, cudaStream_t s)
 }
 int launch_pack_results(Task* t, float* dst, cudaStream_t s) {
   // a multiple of the SM count; 8 MB at N = 4096: ~13 float4 per thread
-  k_pack_results<<<148 * 4, 256, 0, s>>>(make_tk(t), dst);
+  k_pack_results<<<148 * 4, 256, 0, s>>>(make_tk(t), dst, t->obs_width());
   DY_LAUNCH_CHECK();
   return 0;
 }

@@ -53,7 +53,8 @@ class DyrosSimBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in SIM_BUFFERS]
 
 
-# (name, torch dtype name, trailing shape); N is prepended unless the shape starts with None
+# (name, torch dtype name, trailing shape); N is prepended unless the shape starts with None. (obs_buf is (N, 487 + P)
+# with a height scan of P points: DyrosCore._alloc)
 TASK_BUFFERS = [
     ("obs_buf", "float32", (487,)), ("rew_buf", "float32", ()), ("reset_buf", "int64", ()),
     ("timeout_buf", "int64", ()), ("progress_buf", "int64", ()), ("randomize_buf", "int64", ()),
@@ -97,6 +98,11 @@ class DyrosTaskDesc(C.Structure):
 class DyrosTerrainCurriculum(C.Structure):
     _fields_ = [("origins", C.c_void_p), ("levels", C.c_void_p), ("types", C.c_void_p), ("num_levels", i32),
                 ("num_types", i32), ("move_up_distance", f32), ("move_down_scale", f32), ("level_mean", C.c_void_p)]
+
+
+class DyrosHeightScan(C.Structure):
+    _fields_ = [("points", C.c_void_p), ("num_points", i32), ("base_offset", f32), ("scale", f32),
+                ("measured_heights", C.c_void_p)]
 
 
 NOISE_FIELDS = ["qpos_normal", "vel_u", "reset_f", "reset_i", "pert_i", "pert_f", "dr_u"]
@@ -167,6 +173,7 @@ SIGNATURES = {
     "dyros_task_destroy": (_INT, [_VP]),
     "dyros_task_set_noise_injection": (_INT, [_VP, C.POINTER(DyrosNoiseInjection)]),
     "dyros_task_set_terrain_curriculum": (_INT, [_VP, C.POINTER(DyrosTerrainCurriculum)]),
+    "dyros_task_set_height_scan": (_INT, [_VP, C.POINTER(DyrosHeightScan)]),
     "dyros_task_prologue": (_INT, [_VP, _VP, _VP]),
     "dyros_task_physics": (_INT, [_VP, _VP]),
     "dyros_task_physics_kernel": (_INT, [_VP, _VP]),

@@ -337,6 +337,10 @@ class PeerGrads:
 
 class PPOTrainer:
     def __init__(self, env, cfg: Optional[PPOConfig] = None, rank: int = 0, world: int = 1):
+        if env.num_obs != NOBS:
+            raise ValueError(f"PPOTrainer: the on-device networks take the reference's {NOBS} observation columns; this env "
+                             f"has {env.num_obs} (a height scan, terrain measure_heights, adds its heights to each row). "
+                             "Train it with a policy of that input width instead")
         self.env, self.cfg = env, cfg or PPOConfig()
         self.rank, self.world = rank, world
         self.lib = native.load()

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from .. import terrain as terrain_gen
-from ..core import CoreConfig, DyrosCore, HeightField, TerrainCurriculum
+from ..core import NOBS, CoreConfig, DyrosCore, HeightField, TerrainCurriculum
 from ..native import DyrosError
 from .spaces import Box
 
@@ -59,6 +59,18 @@ def _default_cfg(num_envs: int, randomize: bool, perturbation: bool) -> Dict[str
     }
 
 
+def height_scan_points(cfg: Dict[str, Any]) -> Optional[np.ndarray]:
+    """(P, 2) points of the height scan that cfg["env"]["terrain"] asks for (measure_heights), or None."""
+    tr = cfg["env"].get("terrain")
+    return None if tr is None else terrain_gen.height_points(terrain_gen.TerrainConfig.from_dict(tr))
+
+
+def num_observations(cfg: Dict[str, Any]) -> int:
+    """Columns of an observation row: the reference's 487 (T:36-44), plus P heights with measure_heights."""
+    p = height_scan_points(cfg)
+    return NOBS + (0 if p is None else len(p))
+
+
 def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generator] = None) -> CoreConfig:
     """`generator` draws the envs' initial terrain levels when cfg["env"]["terrain"] is set (default: a CPU generator
     seeded with 0)."""
@@ -95,6 +107,7 @@ def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generato
             raise DyrosError('cfg["env"]: give either "heightfield" or "terrain", not both')
         else:
             _terrain_config(c, tcfg, int(env["numEnvs"]), generator)
+        c.height_scan = terrain_gen.height_points(tcfg)  # (any ground, the plane too)
     ap = task.get("randomization_params", {}).get("actor_params", {}).get("humanoid", {})
     dp = ap.get("dof_properties", {})
     if "damping" in dp:
@@ -141,6 +154,7 @@ class DyrosDynamicWalk:
         env["numActions"] = self.num_action
         if (self.num_single_step_obs, self.num_action, self.num_obs_his, self.num_obs_skip) != (37, 13, 10, 2):
             raise ValueError("the fused observation kernel is specialised to 37/13/10/2 (DyrosDynamicWalk.yaml:15-20)")
+        env["numObservations"] = num_observations(cfg)  # + the measured heights (legged_gym's measure_heights)
         # VT:50-97 (Env.__init__)
         dev = sim_device.split(":")
         if dev[0].lower() not in ("cuda", "gpu"):
@@ -172,6 +186,8 @@ class DyrosDynamicWalk:
         self.dt_policy = self.dt * self.skipframe
         self.max_episode_length = self.max_episode_length_s / (self.dt * self.skipframe)  # T:35
         self.core = DyrosCore(self.num_environments, self.device, self.core_cfg, seed=seed, rank=rank)
+        assert self.core.obs_width == self.num_observations
+        self.num_height_points = self.core.num_height_points
         self._bind_buffers()
         self._initial_randoms()
         self.extras: Dict[str, Any] = {}
@@ -221,6 +237,9 @@ class DyrosDynamicWalk:
         # origins; with the curriculum the reset stage updates terrain_levels and terrain_level_mean
         self.terrain_levels, self.terrain_types = t.get("terrain_levels"), t.get("terrain_types")
         self.terrain_origins, self.terrain_level_mean = t.get("terrain_origins"), t.get("terrain_level_mean")
+        # height scan (terrain measure_heights): (N, P) terrain heights in m under the points of height_points, of the
+        # root the observation describes (obs_buf columns 487.. hold them scaled); None without the scan
+        self.measured_heights, self.height_points = t.get("measured_heights"), t.get("height_points")
         for k in ("actions", "actions_pre", "time", "target_vel", "motor_constant_scale", "qpos_noise", "qvel_noise",
                   "qpos_bias", "quat_bias", "epi_len", "epi_len_log", "contact_reward_mean", "total_mass"):
             setattr(self, k, t[k])
@@ -455,9 +474,10 @@ class _HostPipe:
         self.host = [torch.empty(nbytes, dtype=torch.uint8).pin_memory() for _ in range(self.DEPTH)]
         self.packed = [torch.cuda.Event() for _ in range(self.DEPTH)]
         self.landed = [torch.cuda.Event() for _ in range(self.DEPTH)]
-        o, r, t = N * 487 * 4, N * 488 * 4, N * 488 * 4 + N * 8
-        self.views = [({"obs": h[:o].view(torch.float32).view(N, 487)}, h[o:r].view(torch.float32),
-                       h[r:t].view(torch.int64), h[t:].view(torch.int64)) for h in self.host]
+        o, r, t, end = env.core.result_offsets()
+        W = env.core.obs_width
+        self.views = [({"obs": h[:o].view(torch.float32).view(N, W)}, h[o:o + N * 4].view(torch.float32),
+                       h[r:t].view(torch.int64), h[t:end].view(torch.int64)) for h in self.host]
         self.graphs: Dict[Any, torch.cuda.CUDAGraph] = {}
         self.count = 0
 

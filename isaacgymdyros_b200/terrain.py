@@ -9,7 +9,7 @@ Randomness comes from numpy.random.default_rng(seed): the same seed gives the sa
 from __future__ import annotations
 
 from dataclasses import dataclass, field, fields
-from typing import List
+from typing import List, Optional
 
 import numpy as np
 
@@ -34,6 +34,13 @@ class TerrainConfig:
     num_cols: int = 20                   # types
     # smooth slope, rough slope, stairs up, stairs down, discrete obstacles
     terrain_proportions: List[float] = field(default_factory=lambda: [0.1, 0.1, 0.35, 0.25, 0.2])
+    # height scan (DESIGN.md section 4, "Height scan"), on any mesh_type. Off by default here (legged_gym: on), because it
+    # widens the observation from 487 to 487 + len(x) * len(y) columns
+    measure_heights: bool = False
+    measured_points_x: List[float] = field(default_factory=lambda: [-0.8, -0.7, -0.6, -0.5, -0.4, -0.3, -0.2, -0.1, 0.,
+                                                                    0.1, 0.2, 0.3, 0.4, 0.5, 0.6, 0.7, 0.8])
+    measured_points_y: List[float] = field(default_factory=lambda: [-0.5, -0.4, -0.3, -0.2, -0.1, 0., 0.1, 0.2, 0.3,
+                                                                    0.4, 0.5])
     seed: int = 0
 
     @classmethod
@@ -114,6 +121,22 @@ def _sub_terrain(cfg: TerrainConfig, rng, choice: float, difficulty: float, shap
     else:  # choice < cum[4] = 1 (+ the 0.001 of the curriculum's last column: obstacles too)
         _discrete_obstacles(h, rng, obstacle_height, 1.0, 2.0, 20, 3.0, hs, vs)
     return h
+
+
+def height_points(cfg: TerrainConfig) -> Optional[np.ndarray]:
+    """legged_gym's _init_height_points: (P, 2) float32 points in the base's yaw frame, point k = (x[k // ny], y[k % ny])
+    (torch.meshgrid(x, y) in "ij" order, flattened); None without measure_heights."""
+    if not cfg.measure_heights:
+        return None
+    x = np.asarray(cfg.measured_points_x, np.float64)
+    y = np.asarray(cfg.measured_points_y, np.float64)
+    for k, v in (("measured_points_x", x), ("measured_points_y", y)):
+        if v.ndim != 1 or len(v) < 1 or not np.all(np.isfinite(v)):
+            raise DyrosError(f"terrain: {k} must be a non-empty list of finite numbers (got {getattr(cfg, k)!r})")
+    if len(x) * len(y) > 1024:
+        raise DyrosError(f"terrain: at most 1024 height points (got {len(x)} x {len(y)} = {len(x) * len(y)})")
+    gx, gy = np.meshgrid(x.astype(np.float32), y.astype(np.float32), indexing="ij")
+    return np.ascontiguousarray(np.stack([gx.ravel(), gy.ravel()], 1), np.float32)
 
 
 def validate(cfg: TerrainConfig):

@@ -1,5 +1,5 @@
 """What a heightfield ground costs: the fused DyrosDynamicWalk step at 4096 envs (default task, CUDA graph) on six
-grounds, timed alternately in one process with the L2 flushed between timed steps (dyros_flush_l2, as bench.py does):
+grounds, and what the height scan adds on the generated terrain, timed alternately in one process with the L2 flushed between timed steps (dyros_flush_l2, as bench.py does):
   plane      the plane z = 0 (the default build path)
   flat       a heightfield of zeros (same contacts as the plane, heightfield code path)
   rough      uniform heights in [-5 cm, +5 cm] at 0.1 m spacing
@@ -7,9 +7,11 @@ grounds, timed alternately in one process with the L2 flushed between timed step
   generated  the terrain generator's default grid (isaacgymdyros_b200/terrain.py: 10 levels x 20 types of 8 m, 0.1 m
              spacing), envs fixed on their sub-terrains (terrain curriculum: False)
   curriculum the same field with the terrain curriculum: levels move on every reset
+  scan       the curriculum row with measure_heights (legged_gym's 187-point height scan appended to the observation)
 The first four fields cover the default env grid (T:709-718); the envs stand on them at their origins. Also prints the per-phase
 clock64() breakdown of the physics kernel (CTA 0, per role; marks of physics_roles.cuh, as tools/trace_physics.py)
-and the card's name and power limit. TOCABI's roles: 0 torso + left arm, 1 head + right arm + base, 2 left leg,
+and the card's name and power limit, and times the fused post-physics launch alone (dyros_task_post_step, L2 flushed
+before each) for the curriculum and scan rows: the kernel the scan runs in. TOCABI's roles: 0 torso + left arm, 1 head + right arm + base, 2 left leg,
 3 right leg (only the two legs have contact phases).
 Usage: python tools/terrain_step_time.py [--envs 4096] [--steps 60] [--rounds 5] [--out FILE.json]"""
 import argparse
@@ -68,12 +70,12 @@ def main():
     N = a.envs
     name, power = card()
     print(f"card: {name}; power limit, max SM clock: {power}", flush=True)
-    kinds = ["plane", "flat", "rough", "stairs", "generated", "curriculum"]
+    kinds = ["plane", "flat", "rough", "stairs", "generated", "curriculum", "scan"]
     envs = {}
     for k in kinds:
         cfg = default_cfg(N)
-        if k in ("generated", "curriculum"):
-            cfg["env"]["terrain"] = {"curriculum": k == "curriculum"}
+        if k in ("generated", "curriculum", "scan"):
+            cfg["env"]["terrain"] = {"curriculum": k != "generated", "measure_heights": k == "scan"}
         elif k != "plane":
             cfg["env"]["heightfield"] = field(k, N)
         envs[k] = DyrosDynamicWalk(cfg, "cuda:0")
@@ -97,6 +99,19 @@ def main():
                 ev[i][1].record()
             torch.cuda.synchronize()
             times[k] += [e0.elapsed_time(e1) for e0, e1 in ev]
+    # the post-physics launch alone (after the step timings: it advances the envs without physics)
+    post = {k: [] for k in ("curriculum", "scan")}
+    for r in range(a.rounds):
+        for k in post:
+            core = envs[k].core
+            ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.steps)]
+            for i in range(a.steps):
+                core.flush_l2(flush, i)
+                ev[i][0].record()
+                core.post_step()
+                ev[i][1].record()
+            torch.cuda.synchronize()
+            post[k] += [e0.elapsed_time(e1) for e0, e1 in ev]
     # phase breakdown: clock64() marks of the physics launch of CTA 0 (a separate, traced launch)
     phases = {}
     for k in kinds:
@@ -121,6 +136,8 @@ def main():
                              "p90": round(float(np.percentile(t, 90)), 4),
                              "round_medians": [round(float(np.median(t[i * a.steps:(i + 1) * a.steps])), 4) for i in range(a.rounds)],
                              "Menv_steps_per_s": round(N / np.median(t) / 1e3, 2)}
+    res["post_step_ms"] = {k: {"median": round(float(np.median(v)), 4), "p10": round(float(np.percentile(v, 10)), 4),
+                               "p90": round(float(np.percentile(v, 90)), 4)} for k, v in post.items()}
     print(json.dumps(res, indent=1))
     if a.out:
         with open(a.out, "w") as f:
