@@ -66,6 +66,11 @@ constexpr int X_MU = X_PTS + MAX_FEET * MAX_ACTIVE_PTS * PT_WORDS;  // 4 (1 used
 constexpr int X_CV = X_MU + 4;                         // MAX_CSLOTS * 8: velocity-product acceleration of the links whose block
                                                        // receives their contribution to the parent (A_CPA overlaps A_C)
 constexpr int X_MASS = X_CV + MAX_CSLOTS * 8;          // nb per-body mass scales (last: sized by the model)
+// the words of the scratch block that the kernels' slab copies fill and read back (physics_cta.cuh)
+struct LanesScratch {
+  static constexpr int link = LB, q = B_Q, qd = B_QD, tau = B_SC, damping = B_SC + 1, armature = B_SC + 2;
+  static constexpr int mu = X_MU, mass = X_MASS, root = X_ROOT, push = X_PUSH;
+};
 
 HD int env_scratch_floats(int nl, int nb) {
   int n = nl * LB + X_MASS + nb;

@@ -55,6 +55,11 @@ constexpr int PT_WORDS = 5;                          // active sole point: candi
 constexpr int X_PTS = X_OML + 21;                    // MAX_FEET * MAX_ACTIVE_PTS * PT_WORDS
 constexpr int X_MU = X_PTS + MAX_FEET * MAX_ACTIVE_PTS * PT_WORDS;    // 1  friction coefficient of this env's ground contacts
 constexpr int X_MASS = X_MU + 1;                     // nb per-body mass scales (last: sized by the model)
+// the words of the scratch block that the kernels' slab copies fill and read back (physics_cta.cuh)
+struct RolesScratch {
+  static constexpr int link = LS, q = LS_Q, qd = LS_SC, tau = LS_SC + 1, damping = LS_SC + 2, armature = LS_SC + 3;
+  static constexpr int mu = X_MU, mass = X_MASS, root = X_ROOT, push = X_PUSH;
+};
 
 HD int env_scratch_floats(int nl, int nb) {
   int n = nl * LS + X_MASS + nb;

@@ -1025,15 +1025,6 @@ __global__ void __launch_bounds__(256) k_pack_results(TK k, float* __restrict__ 
 }
 
 // ------------------------------------------------------------------ launchers
-static inline TK make_tk(Task* t) {
-  TK k;
-  k.p = t->p;
-  k.b = t->b;
-  k.s = t->sim->b;
-  k.j = t->inj;
-  k.c = t->cur;
-  return k;
-}
 static inline HeightScan make_scan(const Task* t) {
   HeightScan sc;
   sc.points = reinterpret_cast<const float2*>(t->scan.points);

@@ -14,6 +14,16 @@ struct TK {
   DyrosNoiseInjection j;
   DyrosTerrainCurriculum c;  // levels == NULL: no curriculum
 };
+// (host) the argument of every task kernel and of the fused physics step
+inline TK make_tk(const Task* t) {
+  TK k;
+  k.p = t->p;
+  k.b = t->b;
+  k.s = t->sim->b;
+  k.j = t->inj;
+  k.c = t->cur;
+  return k;
+}
 
 // JU:374-395 with x_dot_0 = x_dot_f = 0.0 (T:458-461), reference operation order. The terms that depend on the knot
 // times only (tt^2, tt^3 and the reference's literal 0/tt, 0/tt^2) are computed by cubic_knots once per env: a zero
