@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define DYROS_ABI_VERSION 3  /* 3: DyrosTaskBuffers.reset_seq, DyrosSimDesc.physics_program; 2: contact_friction, pd_gain_scale, dr_friction_*, dr_pd_gain_*, pack_results, set_obs_buf, post_step */
+#define DYROS_ABI_VERSION 3  /* 3: DyrosTaskBuffers.reset_seq, DyrosSimDesc.physics_program (later additions within 3, a no-op for zero-initialised structs: DyrosPpoNet.inputs, DyrosPpoBuffers.obs_dim); 2: contact_friction, pd_gain_scale, dr_friction_*, dr_pd_gain_*, pack_results, set_obs_buf, post_step */
 #define DYROS_MAX_LINKS 40
 #define DYROS_MAX_BODIES 48
 #define DYROS_LANES 4 /* roles (warps) per env group in the physics kernel */
@@ -383,7 +383,7 @@ typedef struct {
   float reward_scale;         /* reward_shaper.scale_value, PPO:64 */
   int32_t value_bootstrap;    /* PPO:61 */
   uint64_t seed;              /* Philox key of the action noise */
-  float* obs;                 /* (N,H,487) A2C:639 */
+  float* obs;                 /* (N,H,W) fp32 rows, W = obs_dim (the fp32 path; the packed path keeps bf16 rows) A2C:639 */
   float* actions;             /* (N,H,13) */
   float* mus;                 /* (N,H,13) */
   float* neglogp;             /* (N,H) */
@@ -397,6 +397,8 @@ typedef struct {
   float* ep_stats;            /* (3) sums over finished episodes: reward, length, count (A2C:676-677) */
   int32_t* step;              /* (1) slot of the next rollout step, 0..H-1 */
   uint64_t* global_step;      /* (1) rollout steps so far (Philox counter) */
+  int32_t obs_dim;            /* W, columns of an observation row: 487 + P with a height scan of P points; 0 means 487.
+                               * Appended in ABI 3: a zero-initialised struct keeps the 487 layout. Negative: refused. */
 } DyrosPpoBuffers;
 /* get_action_values + the experience_buffer updates of one rollout step (A2C:633-647, MD:28-58): samples the actions
  * from N(mu, exp(logstd)), computes their neglogp (MD:60-63), records obs / done / mu / value / action / neglogp at slot
@@ -420,15 +422,20 @@ int dyros_ppo_adam(float* params, const float* grads, float* exp_avg, float* exp
                    float eps, float lr0, float lr_min, int lr_max_steps, void* stream);
 
 
-/* ---- packed bf16 path of the two MLPs (network_builder_dyros.py:129-216: separate 487-H-H actor and critic): one batch-2
+/* ---- packed bf16 path of the two MLPs (network_builder_dyros.py:129-216: separate W-H-H actor and critic): one batch-2
  * problem in GEMM layout, net 0 = actor, net 1 = critic. The caller runs the 8 batched GEMMs of a minibatch with a
  * library (3 forward: x W0^T, h0 W1^T, h1 Wh^T; 5 backward); these entry points are everything between them. Weights
  * and activations bf16 (where the reference trains under fp16 autocast + GradScaler, PPO:59), biases, bias gradients,
  * master parameters, Adam moments fp32. The flat master layout (dyros_ppo_adam's buffers) is, per net,
- * [W0 (H x 487), b0 (H), W1 (H x H), b1 (H), Wh (nout x H), bh (nout)], nout = 13 (actor) then 1 (critic). */
+ * [W0 (H x W), b0 (H), W1 (H x H), b1 (H), Wh (nout x H), bh (nout)], nout = 13 (actor) then 1 (critic).
+ * W is the input width and K0 = round_up(W, 8) the padded one: a GEMM's rows must be a multiple of 8 elements for the
+ * library's tensor-core kernels (an odd leading dimension falls back to its slow align-1 kernels), so W0 and the bf16
+ * observation rows x_step / x_roll are K0 wide, with columns W..K0-1 zero. W = 487: K0 = 488; W = 674: K0 = 680. */
 typedef struct DyrosPpoNet {
   int32_t hidden;        /* H, a multiple of 8 (256: PPO:28-35) */
-  void* w0;              /* bf16 [2][H][488]: 487 inputs padded to 488 (column 487 is zero) */
+  int32_t inputs;        /* W; 0 means 487. Added in ABI 3 in the padding before w0: sizeof and every other offset are
+                          * unchanged, and a zero-initialised struct keeps the 487 layout. Negative: refused. */
+  void* w0;              /* bf16 [2][H][K0]: W inputs padded to K0 (columns W..K0-1 are zero) */
   float* b0;             /* [2][H] */
   void* w1;              /* bf16 [2][H][H] */
   float* b1;             /* [2][H] */
@@ -441,8 +448,8 @@ typedef struct DyrosPpoNet {
   float* gb1;            /* zeroed by dyros_ppo_unpack_grads */
   float* gbh;
 } DyrosPpoNet;
-/* obs (N,487) fp32 -> bf16 rows of width 488: x_step (N,488) for this step's policy forward and, if x_roll is given,
- * row e*H + *step of the env-major rollout store (N*H,488). */
+/* obs (N,W) fp32 -> bf16 rows of width K0 (W = b->obs_dim, columns W..K0-1 written as zero): x_step (N,K0) for this
+ * step's policy forward and, if x_roll is given, row e*H + *step of the env-major rollout store (N*H,K0). */
 int dyros_ppo_cast_obs(const DyrosPpoBuffers* b, const float* obs, void* x_step, void* x_roll, void* stream);
 /* t [2][rows][H] bf16 = relu(t + bias [2][H]) in place (the hidden layers' activation, network_builder_dyros.py:132-146). */
 int dyros_ppo_bias_relu(void* t, const float* bias, int rows, int hidden, void* stream);

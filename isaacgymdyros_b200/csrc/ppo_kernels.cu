@@ -1,7 +1,8 @@
 // On-device PPO pieces around the env step (SURVEY 8f-1): the bodies of the rollout bookkeeping, GAE, the clipped
 // surrogate / value loss gradient and the two Adam optimisers of the reference's rl_games fork, as sm_100a kernels.
-// The two 487-256-256-{13,1} MLPs stay library GEMMs (torch / cuBLAS); everything elementwise around them is here, so
-// that one rollout step and one minibatch update are each a handful of launches inside a CUDA graph.
+// The two W-256-256-{13,1} MLPs stay library GEMMs (torch / cuBLAS); everything elementwise around them is here, so
+// that one rollout step and one minibatch update are each a handful of launches inside a CUDA graph. W is the input width:
+// the reference's 487 observation columns, or more with a height scan (DyrosPpoBuffers.obs_dim, DyrosPpoNet.inputs).
 // Citations: A2C = learning/rl_games_custom/a2c_common_dyros.py, AG = learning/rl_games_custom/a2c_continuous_seperate.py,
 // MD = learning/rl_games_custom/models_dyros.py, PPO = cfg/train/DyrosDynamicWalkPPO.yaml (reference tree). The loss
 // formulas of rl_games 1.1.4 (common_losses.actor_loss / critic_loss, torch_ext.policy_kl; pinned by
@@ -15,7 +16,9 @@
 
 namespace dyros {
 
-constexpr int PPO_NA = 13, PPO_NOBS = 487;
+constexpr int PPO_NA = 13, PPO_NOBS = 487;  // PPO_NOBS: the input width that obs_dim / inputs = 0 stand for
+static inline int ppo_width(int w) { return w ? w : PPO_NOBS; }
+static inline int ppo_padded_width(int w) { return (w + 7) & ~7; }  // K0: GEMM rows a multiple of 8 (DESIGN.md section 9)
 
 // ---------------------------------------------------------------- rollout: act + record (A2C:629-647, MD:28-58)
 // One warp per env. Samples a = mu + sigma * N(0,1) (Philox, counter = (env, global step)), its negative log
@@ -25,7 +28,7 @@ constexpr int PPO_NA = 13, PPO_NOBS = 487;
 __global__ void __launch_bounds__(256) k_ppo_act(DyrosPpoBuffers b, const float* __restrict__ mu, const float* __restrict__ value,
                                                  const float* __restrict__ logstd, const float* __restrict__ obs,
                                                  const long long* __restrict__ reset_buf, float* __restrict__ actions_env,
-                                                 const float* __restrict__ inject_normal) {
+                                                 const float* __restrict__ inject_normal, int W) {
   const int lane = threadIdx.x & 31, e = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (e >= b.N) return;
   const int n = *b.step;
@@ -59,9 +62,9 @@ __global__ void __launch_bounds__(256) k_ppo_act(DyrosPpoBuffers b, const float*
     b.values[row] = value[e];
     b.dones[row] = reset_buf[e] != 0 ? 1.f : 0.f;  // self.dones BEFORE the step (A2C:640)
   }
-  const float* src = obs + (size_t)e * PPO_NOBS;
-  float* dst = b.obs + row * PPO_NOBS;
-  for (int i = lane; i < PPO_NOBS; i += 32) dst[i] = src[i];
+  const float* src = obs + (size_t)e * W;
+  float* dst = b.obs + row * W;
+  for (int i = lane; i < W; i += 32) dst[i] = src[i];
 }
 
 // after the env step: shaped reward with the time-out bootstrap (A2C:654-661), episode statistics (A2C:663-684)
@@ -226,26 +229,27 @@ __global__ void k_ppo_adam_finish(float* norm2, int* t_dev, float* lr_dev, float
 
 
 // ================================================================ packed bf16 path (DESIGN.md section 9, "update v2")
-// The two MLPs as ONE batch-2 problem in GEMM layout (net 0 = actor, net 1 = critic): W0 [2][H][488] (487 inputs padded
-// to a multiple of 8: cuBLAS falls back to its slow align-1 kernels for an odd leading dimension), W1 [2][H][H],
+// The two MLPs as ONE batch-2 problem in GEMM layout (net 0 = actor, net 1 = critic): W0 [2][H][K0] (W inputs padded
+// to K0, a multiple of 8: cuBLAS falls back to its slow align-1 kernels for an odd leading dimension), W1 [2][H][H],
 // Wh [2][16][H] (13 / 1 rows used, the rest stay zero), bf16, biases fp32. The 8 GEMMs of a minibatch (3 forward, 5
 // backward) are batched library calls; everything between them is here: 5 kernels instead of ~60 framework launches
 // (casts, bias adds, ReLU masks, bf16 column sums for the bias gradients).
-constexpr int PPO_K0 = 488, PPO_HEAD = 16;
+constexpr int PPO_HEAD = 16;
 typedef __nv_bfloat16 bf16;
 __device__ __forceinline__ float bf2f(bf16 x) { return __bfloat162float(x); }
 
-// obs (N,487) fp32 -> bf16 rows of width 488 (last column 0): the policy's input of this step and, when x_roll is
-// given, the same row at slot *step of the env-major rollout store (row e*H + n). One warp per env.
-__global__ void __launch_bounds__(256) k_ppo_cast_obs(const float* __restrict__ obs, int N, bf16* __restrict__ x_step,
+// obs (N,W) fp32 -> bf16 rows of width K0 (columns W..K0-1 zero): the policy's input of this step and, when x_roll is
+// given, the same row at slot *step of the env-major rollout store (row e*H + n). One warp per env; lane i of a pass
+// reads the pair 2i, 2i+1, so a warp's loads cover 64 consecutive floats of the row.
+__global__ void __launch_bounds__(256) k_ppo_cast_obs(const float* __restrict__ obs, int N, int W, int K0, bf16* __restrict__ x_step,
                                                       bf16* __restrict__ x_roll, const int* __restrict__ step, int H) {
   const int lane = threadIdx.x & 31, e = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (e >= N) return;
-  const float* src = obs + (size_t)e * PPO_NOBS;
-  __nv_bfloat162* a = reinterpret_cast<__nv_bfloat162*>(x_step + (size_t)e * PPO_K0);
-  __nv_bfloat162* r = x_roll ? reinterpret_cast<__nv_bfloat162*>(x_roll + ((size_t)e * H + *step) * PPO_K0) : nullptr;
-  for (int i = lane; i < PPO_K0 / 2; i += 32) {
-    const float lo = src[2 * i], hi = 2 * i + 1 < PPO_NOBS ? src[2 * i + 1] : 0.f;
+  const float* src = obs + (size_t)e * W;
+  __nv_bfloat162* a = reinterpret_cast<__nv_bfloat162*>(x_step + (size_t)e * K0);
+  __nv_bfloat162* r = x_roll ? reinterpret_cast<__nv_bfloat162*>(x_roll + ((size_t)e * H + *step) * K0) : nullptr;
+  for (int i = lane; i < K0 / 2; i += 32) {
+    const float lo = 2 * i < W ? src[2 * i] : 0.f, hi = 2 * i + 1 < W ? src[2 * i + 1] : 0.f;
     const __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     a[i] = v;
     if (r) r[i] = v;
@@ -431,8 +435,9 @@ __global__ void __launch_bounds__(256) k_ppo_loss_grad_packed(DyrosPpoBuffers b,
   }
 }
 
-// master layout of the flat fp32 buffers (ppo.py FlatActorCritic): per net [W0 (H x 487), b0 (H), W1 (H x H), b1 (H),
-// Wh (nout x H), bh (nout)], actor (nout 13) then critic (nout 1)
+// master layout of the flat fp32 buffers (ppo.py FlatActorCritic): per net [W0 (H x W), b0 (H), W1 (H x H), b1 (H),
+// Wh (nout x H), bh (nout)], actor (nout 13) then critic (nout 1). The kernels below visit the master block's rows x cols
+// only, so the padding columns W..K0-1 of the packed W0 are never written and stay zero.
 struct PpoSeg {
   int master_off, rows, cols;  // the master block
   int dst_cols;                // leading dimension of the packed matrix (0: a bias vector)
@@ -442,12 +447,12 @@ struct PpoSeg {
 struct PpoSegs {
   PpoSeg s[12];
 };
-static PpoSegs ppo_segments(int hidden) {
+static PpoSegs ppo_segments(int hidden, int W) {
   PpoSegs S;
   int off = 0, k = 0;
   for (int net = 0; net < 2; ++net) {
     const int nout = net == 0 ? PPO_NA : 1;
-    S.s[k++] = PpoSeg{off, hidden, PPO_NOBS, PPO_K0, 0, net}; off += hidden * PPO_NOBS;
+    S.s[k++] = PpoSeg{off, hidden, W, ppo_padded_width(W), 0, net}; off += hidden * W;
     S.s[k++] = PpoSeg{off, 1, hidden, 0, 1, net}; off += hidden;
     S.s[k++] = PpoSeg{off, hidden, hidden, hidden, 2, net}; off += hidden * hidden;
     S.s[k++] = PpoSeg{off, 1, hidden, 0, 3, net}; off += hidden;
@@ -458,7 +463,7 @@ static PpoSegs ppo_segments(int hidden) {
 }
 __device__ __forceinline__ size_t ppo_packed_index(const PpoSeg& g, int hidden, int r, int c) {
   switch (g.which) {
-    case 0: return ((size_t)g.net * hidden + r) * PPO_K0 + c;
+    case 0: return ((size_t)g.net * hidden + r) * g.dst_cols + c;
     case 2: return ((size_t)g.net * hidden + r) * hidden + c;
     case 4: return ((size_t)g.net * PPO_HEAD + r) * hidden + c;
     case 5: return (size_t)g.net * PPO_HEAD + c;
@@ -758,9 +763,10 @@ extern "C" {
 int dyros_ppo_act(const DyrosPpoBuffers* b, const float* mu, const float* value, const float* logstd, const float* obs,
                   const int64_t* reset_buf, float* actions_env, const float* inject_normal, void* stream) {
   PPO_CHECK(b && mu && value && logstd && obs && reset_buf && actions_env, "dyros_ppo_act: null argument");
+  PPO_CHECK(b->obs_dim >= 0, "dyros_ppo_act: DyrosPpoBuffers.obs_dim < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
   k_ppo_act<<<(b->N + 7) / 8, 256, 0, (cudaStream_t)stream>>>(*b, mu, value, logstd, obs, reinterpret_cast<const long long*>(reset_buf),
-                                                              actions_env, inject_normal);
+                                                              actions_env, inject_normal, ppo_width(b->obs_dim));
   DY_LAUNCH_CHECK();
   return 0;
 }
@@ -810,9 +816,11 @@ static bool ppo_net_ok(const DyrosPpoNet* n) {
 }
 int dyros_ppo_cast_obs(const DyrosPpoBuffers* b, const float* obs, void* x_step, void* x_roll, void* stream) {
   PPO_CHECK(b && obs && x_step, "dyros_ppo_cast_obs: null argument");
+  PPO_CHECK(b->obs_dim >= 0, "dyros_ppo_cast_obs: DyrosPpoBuffers.obs_dim < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
-  k_ppo_cast_obs<<<(b->N + 7) / 8, 256, 0, (cudaStream_t)stream>>>(obs, b->N, static_cast<bf16*>(x_step), static_cast<bf16*>(x_roll),
-                                                                   b->step, b->H);
+  const int W = ppo_width(b->obs_dim);
+  k_ppo_cast_obs<<<(b->N + 7) / 8, 256, 0, (cudaStream_t)stream>>>(obs, b->N, W, ppo_padded_width(W), static_cast<bf16*>(x_step),
+                                                                   static_cast<bf16*>(x_roll), b->step, b->H);
   DY_LAUNCH_CHECK();
   return 0;
 }
@@ -853,16 +861,19 @@ int dyros_ppo_loss_grad_packed(const DyrosPpoBuffers* b, int row0, int mb, const
 }
 int dyros_ppo_pack_params(const DyrosPpoNet* net, const float* flat, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && flat, "dyros_ppo_pack_params: bad argument");
+  PPO_CHECK(net->inputs >= 0, "dyros_ppo_pack_params: DyrosPpoNet.inputs < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
-  k_ppo_pack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden), *net, flat);
+  k_ppo_pack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, flat);
   DY_LAUNCH_CHECK();
   return 0;
 }
 int dyros_ppo_unpack_grads(const DyrosPpoNet* net, float* flat_grad, float* norm2_accum, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && net->gw0 && net->gw1 && net->gwh && net->gb0 && net->gb1 && net->gbh && flat_grad,
             "dyros_ppo_unpack_grads: bad argument");
+  PPO_CHECK(net->inputs >= 0, "dyros_ppo_unpack_grads: DyrosPpoNet.inputs < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
-  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden), *net, flat_grad, norm2_accum, nullptr, 0);
+  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, flat_grad,
+                                                               norm2_accum, nullptr, 0);
   DY_LAUNCH_CHECK();
   return 0;
 }
@@ -871,12 +882,13 @@ int dyros_ppo_adam_packed(const DyrosPpoNet* net, float* params, const float* gr
                           float max_norm, int norm_done, float* norm2_scratch, float* lr_dev, int32_t* step_dev, float beta1, float beta2,
                           float eps, float lr0, float lr_min, int lr_max_steps, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && params && grads && exp_avg && exp_avg_sq && norm2_scratch && lr_dev && step_dev, "dyros_ppo_adam_packed: bad argument");
+  PPO_CHECK(net->inputs >= 0, "dyros_ppo_adam_packed: DyrosPpoNet.inputs < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
   cudaStream_t s = (cudaStream_t)stream;
-  const int H = net->hidden, n_actor = H * PPO_NOBS + H + H * H + H + PPO_NA * H + PPO_NA;
+  const int H = net->hidden, W = ppo_width(net->inputs), n_actor = H * W + H + H * H + H + PPO_NA * H + PPO_NA;
   // norm2 holds the squared norm of the UNSCALED actor gradients (sum over ranks); the kernel scales it
   if (max_norm > 0.f && !norm_done) k_ppo_gradnorm<<<148, 256, 0, s>>>(grads, n_actor, 1.f, norm2_scratch);
-  k_ppo_adam_pack<<<dim3(64, 12), 256, 0, s>>>(ppo_segments(H), *net, params, grads, exp_avg, exp_avg_sq, grad_scale, max_norm, norm2_scratch,
+  k_ppo_adam_pack<<<dim3(64, 12), 256, 0, s>>>(ppo_segments(H, W), *net, params, grads, exp_avg, exp_avg_sq, grad_scale, max_norm, norm2_scratch,
                                               lr_dev, step_dev, beta1, beta2, eps);
   k_ppo_adam_finish<<<1, 1, 0, s>>>(norm2_scratch, step_dev, lr_dev, lr0, lr_min, lr_max_steps);
   DY_LAUNCH_CHECK();
@@ -893,8 +905,9 @@ int dyros_ppo_unpack_grads_peers(const DyrosPpoNet* net, const DyrosPpoPeers* pe
   PPO_CHECK(ppo_net_ok(net) && net->gw0 && net->gw1 && net->gwh && net->gb0 && net->gb1 && net->gbh && ppo_peers_ok(peers),
             "dyros_ppo_unpack_grads_peers: bad argument");
   PPO_CHECK(peers->grad[peers->rank][1] == peers->grad[peers->rank][0] + peers->stride, "dyros_ppo_unpack_grads_peers: the rank's two buffers must be `stride` apart");
+  PPO_CHECK(net->inputs >= 0, "dyros_ppo_unpack_grads_peers: DyrosPpoNet.inputs < 0 (0 means 487)");
   if (configure_ppo_kernels()) return 1;
-  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden), *net, peers->grad[peers->rank][0], nullptr, peers->epoch,
+  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, peers->grad[peers->rank][0], nullptr, peers->epoch,
                                                                (size_t)peers->stride);
   DY_LAUNCH_CHECK();
   return 0;

@@ -116,11 +116,11 @@ class DyrosPpoBuffers(C.Structure):
     _fields_ = [("N", i32), ("H", i32), ("gamma", f32), ("tau", f32), ("e_clip", f32), ("critic_coef", f32),
                 ("reward_scale", f32), ("value_bootstrap", i32), ("seed", u64)] + [
         (n, C.c_void_p) for n in ("obs", "actions", "mus", "neglogp", "values", "rewards", "dones", "advantages", "returns",
-                                  "cur_reward", "cur_length", "ep_stats", "step", "global_step")]
+                                  "cur_reward", "cur_length", "ep_stats", "step", "global_step")] + [("obs_dim", i32)]
 
 
 class DyrosPpoNet(C.Structure):
-    _fields_ = [("hidden", i32)] + [(n, C.c_void_p) for n in ("w0", "b0", "w1", "b1", "wh", "bh", "gw0", "gw1", "gwh", "gb0", "gb1", "gbh")]
+    _fields_ = [("hidden", i32), ("inputs", i32)] + [(n, C.c_void_p) for n in ("w0", "b0", "w1", "b1", "wh", "bh", "gw0", "gw1", "gwh", "gb0", "gb1", "gbh")]
 
 
 class DyrosPpoPeers(C.Structure):

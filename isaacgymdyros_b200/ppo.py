@@ -7,10 +7,12 @@ the rollout buffers, GAE, the loss gradient and both optimisers are kernels of l
 one rollout step and one minibatch update are each ONE CUDA graph, and with several ranks the only traffic is one NCCL
 all-reduce of the flat 1.54 MB gradient bucket per minibatch (AG:161-203) plus a few scalars per epoch.
 
-The two 487-256-256-{13,1} MLPs are library GEMMs (torch / cuBLAS); parameters, gradients and Adam moments live in flat
-fp32 buffers. Two network paths:
+The two W-256-256-{13,1} MLPs are library GEMMs (torch / cuBLAS); parameters, gradients and Adam moments live in flat
+fp32 buffers. W = PPOConfig.num_obs, the env's observation width: the reference's 487, or 674 with the default height scan
+(terrain measure_heights). Both networks see the whole row. Two network paths:
   * `mixed_precision="bf16"` (default; the reference trains under fp16 autocast + GradScaler, PPO:59): `PackedNets` --
-    actor and critic as ONE batch-2 problem in GEMM layout (bf16 weights, input width padded 487 -> 488), 8 batched
+    actor and critic as ONE batch-2 problem in GEMM layout (bf16 weights, input width padded to K0 = round_up(W, 8):
+    487 -> 488, 674 -> 680), 8 batched
     GEMMs per minibatch with hand-written backward and the library's own kernels in between (csrc/ppo_kernels.cu,
     "packed bf16 path"): 21 launches per minibatch instead of 79;
   * `mixed_precision="fp32"`: torch autograd on views of the flat buffers (what the tests pin against the oracle)."""
@@ -60,11 +62,13 @@ class PPOConfig:
     seed: int = 42
     use_cuda_graph: bool = True
     graph_span: str = "mini_epoch"          # one CUDA graph per "minibatch" update, or one for all minibatches of a "mini_epoch"
+    num_obs: int = NOBS                     # input width of both networks = the env's num_obs (network_builder_dyros.py
+                                            # takes it from the observation space); 674 with the default height scan
 
 
-def layer_shapes(units=(256, 256)):
+def layer_shapes(units=(256, 256), num_obs=NOBS):
     """(name, out, in) of the actor and the critic (network_builder_dyros.py:129-216, `separate: True`)."""
-    dims = [NOBS] + list(units)
+    dims = [num_obs] + list(units)
     actor = [(f"actor_mlp.{i}", dims[i + 1], dims[i]) for i in range(len(units))] + [("mu", NA, dims[-1])]
     critic = [(f"critic_mlp.{i}", dims[i + 1], dims[i]) for i in range(len(units))] + [("value", 1, dims[-1])]
     return actor, critic
@@ -76,7 +80,7 @@ class FlatActorCritic:
 
     def __init__(self, device, cfg: PPOConfig):
         self.cfg, self.device = cfg, torch.device(device)
-        actor, critic = layer_shapes(cfg.units)
+        actor, critic = layer_shapes(cfg.units, cfg.num_obs)
         self.n_actor = sum(o * i + o for _, o, i in actor)
         self.n = self.n_actor + sum(o * i + o for _, o, i in critic)
         self.flat = torch.zeros(self.n, device=device)
@@ -201,14 +205,16 @@ class FlatActorCritic:
 
 class PackedNets:
     """bf16 compute copies of the flat master parameters in GEMM layout (include/dyros_b200.h DyrosPpoNet) and the
-    forward / backward of both networks as batch-2 GEMMs. Activations of the last `forward` are kept for `backward`."""
-    K0, HEAD = 488, 16
+    forward / backward of both networks as batch-2 GEMMs. Activations of the last `forward` are kept for `backward`.
+    K0 = round_up(num_obs, 8) is the padded input width of W0 and of the bf16 observation rows (columns num_obs.. zero)."""
+    HEAD = 16
 
     def __init__(self, net: FlatActorCritic, lib):
         if len(net.cfg.units) != 2 or net.cfg.units[0] != net.cfg.units[1] or net.cfg.units[0] % 8:
             raise ValueError("the packed path holds two hidden layers of equal width (a multiple of 8), PPO:28-35")
         self.net, self.lib, dev = net, lib, net.device
         Hd = self.hidden = net.cfg.units[0]
+        self.K0 = (net.cfg.num_obs + 7) // 8 * 8
         zb = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)
         zf = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)
         self.w0, self.w1, self.wh = zb(2, Hd, self.K0), zb(2, Hd, Hd), zb(2, self.HEAD, Hd)
@@ -216,7 +222,7 @@ class PackedNets:
         self.gw0, self.gw1, self.gwh = zb(2, Hd, self.K0), zb(2, Hd, Hd), zb(2, self.HEAD, Hd)
         self.gb0, self.gb1, self.gbh = zf(2, Hd), zf(2, Hd), zf(2, self.HEAD)
         d = native.DyrosPpoNet()
-        d.hidden = Hd
+        d.hidden, d.inputs = Hd, net.cfg.num_obs
         for k in ("w0", "b0", "w1", "b1", "wh", "bh", "gw0", "gw1", "gwh", "gb0", "gb1", "gbh"):
             setattr(d, k, getattr(self, k).data_ptr())
         self.desc = d
@@ -245,7 +251,7 @@ class PackedNets:
         return b
 
     def forward(self, x: torch.Tensor):
-        """x (rows, 488) bf16 -> head output (2, rows, 16) bf16 WITHOUT the head bias (the consumers add `bh`)."""
+        """x (rows, K0) bf16 -> head output (2, rows, 16) bf16 WITHOUT the head bias (the consumers add `bh`)."""
         rows = x.shape[0]
         b, s, lib = self._buffers(rows), self._stream, self.lib
         xe = x.unsqueeze(0).expand(2, rows, self.K0)
@@ -270,7 +276,7 @@ class PackedNets:
         torch.bmm(b["d1"], self.w1, out=b["d0"])
         native.check(lib.dyros_ppo_relu_bwd(C.c_void_p(b["d0"].data_ptr()), C.c_void_p(b["h0"].data_ptr()),
                                             C.c_void_p(self.gb0.data_ptr()), rows, self.hidden, s), "relu_bwd")
-        torch.bmm(b["d0"].transpose(1, 2), xe, out=self.gw0)                              # (2,H,488)
+        torch.bmm(b["d0"].transpose(1, 2), xe, out=self.gw0)                              # (2,H,K0)
 
     def mu_value(self, out: torch.Tensor):
         """fp32 (rows,13) mu and (rows) value of a head output (tests, the bootstrap value of the last observation)."""
@@ -337,11 +343,12 @@ class PeerGrads:
 
 class PPOTrainer:
     def __init__(self, env, cfg: Optional[PPOConfig] = None, rank: int = 0, world: int = 1):
-        if env.num_obs != NOBS:
-            raise ValueError(f"PPOTrainer: the on-device networks take the reference's {NOBS} observation columns; this env "
+        cfg = cfg or PPOConfig()
+        if env.num_obs != cfg.num_obs:
+            raise ValueError(f"PPOTrainer: the networks take PPOConfig.num_obs = {cfg.num_obs} observation columns; this env "
                              f"has {env.num_obs} (a height scan, terrain measure_heights, adds its heights to each row). "
-                             "Train it with a policy of that input width instead")
-        self.env, self.cfg = env, cfg or PPOConfig()
+                             f"Train it with PPOConfig(num_obs={env.num_obs})")
+        self.env, self.cfg = env, cfg
         self.rank, self.world = rank, world
         self.lib = native.load()
         c, dev = self.cfg, env.device
@@ -360,15 +367,16 @@ class PPOTrainer:
             raise ValueError("grad_sync: 'peer', 'peer2' or 'nccl'")
         self.peers: Optional[PeerGrads] = (PeerGrads(self.net.n, dev, rank, world)
                                            if world > 1 and self.packed is not None and c.grad_sync in ("peer", "peer2") else None)
-        if self.packed is not None:  # the rollout's observations are kept as the bf16 rows the GEMMs read (N*H x 488)
-            self.x_step = z(N, PackedNets.K0, dt=torch.bfloat16)
-            self.x_roll = z(N * H, PackedNets.K0, dt=torch.bfloat16)
-        self.buf = {"obs": z(N, H, NOBS) if self.packed is None else z(1), "actions": z(N, H, NA), "mus": z(N, H, NA), "neglogp": z(N, H), "values": z(N, H),
+        if self.packed is not None:  # the rollout's observations are kept as the bf16 rows the GEMMs read (N*H x K0)
+            self.x_step = z(N, self.packed.K0, dt=torch.bfloat16)
+            self.x_roll = z(N * H, self.packed.K0, dt=torch.bfloat16)
+        self.buf = {"obs": z(N, H, c.num_obs) if self.packed is None else z(1), "actions": z(N, H, NA), "mus": z(N, H, NA), "neglogp": z(N, H), "values": z(N, H),
                     "rewards": z(N, H), "dones": z(N, H), "advantages": z(N, H), "returns": z(N, H), "cur_reward": z(N),
                     "cur_length": z(N), "ep_stats": z(3), "step": z(1, dt=torch.int32), "global_step": z(1, dt=torch.int64)}
         pb = native.DyrosPpoBuffers()
         pb.N, pb.H, pb.gamma, pb.tau, pb.e_clip, pb.critic_coef = N, H, c.gamma, c.tau, c.e_clip, c.critic_coef
         pb.reward_scale, pb.value_bootstrap, pb.seed = c.reward_scale, int(c.value_bootstrap), c.seed + 7919 * (rank + 1)
+        pb.obs_dim = c.num_obs
         for k, t in self.buf.items():
             setattr(pb, k, t.data_ptr())
         self.pb = pb
@@ -512,7 +520,7 @@ class PPOTrainer:
             return self._minibatch_packed(i)
         c, mb = self.cfg, self.cfg.minibatch_size
         r0 = i * mb
-        obs = self.buf["obs"].view(self.N * self.H, NOBS)[r0:r0 + mb]
+        obs = self.buf["obs"].view(self.N * self.H, c.num_obs)[r0:r0 + mb]
         mu, v = self.net.forward(obs)
         mu32, v32 = mu.float().contiguous(), v.float().contiguous()
         native.check(self.lib.dyros_ppo_loss_grad(C.byref(self.pb), r0, mb, self._p(mu32), self._p(v32), self._p(self.net.logstd),
@@ -599,7 +607,9 @@ class PPOTrainer:
         return files
 
     def train_epoch(self) -> Dict[str, float]:
-        """One epoch of ContinuousA2CBase.train (A2C:983-1008): noise schedule, rollout, update. One device->host read."""
+        """One epoch of ContinuousA2CBase.train (A2C:983-1008): noise schedule, rollout, update. One device->host read.
+        With a terrain curriculum, "terrain_level" is the envs' mean level at the end of the rollout (legged_gym's
+        episode log), averaged over ranks."""
         c = self.cfg
         self.epoch += 1
         self.net.update_action_noise((c.max_epochs - self.epoch) / c.max_epochs)  # A2C:985
@@ -607,14 +617,18 @@ class PPOTrainer:
         self.rollout()
         self.update()
         k = c.mini_epochs * self.num_minibatches
-        out = torch.cat([self.stats / k, self.buf["ep_stats"], self.lr[:1]])
+        level = getattr(self.env, "terrain_level_mean", None)
+        out = torch.cat([self.stats / k, self.buf["ep_stats"], self.lr[:1]] + ([level.reshape(1)] if level is not None else []))
         if self.world > 1:
             import torch.distributed as dist
             s = out.clone()
             dist.all_reduce(s)
             out = s / self.world
             out[4:7] = s[4:7]
-        a_loss, c_loss, kl, clip_frac, ep_r, ep_l, ep_n, lr = out.tolist()
-        return {"a_loss": a_loss, "c_loss": c_loss, "kl": kl, "clip_frac": clip_frac, "lr": lr,
-                "mean_reward": ep_r / max(ep_n, 1.0), "mean_length": ep_l / max(ep_n, 1.0), "episodes": ep_n,
-                "frames": self.N * self.H * self.world}
+        a_loss, c_loss, kl, clip_frac, ep_r, ep_l, ep_n, lr, *rest = out.tolist()
+        res = {"a_loss": a_loss, "c_loss": c_loss, "kl": kl, "clip_frac": clip_frac, "lr": lr,
+               "mean_reward": ep_r / max(ep_n, 1.0), "mean_length": ep_l / max(ep_n, 1.0), "episodes": ep_n,
+               "frames": self.N * self.H * self.world}
+        if rest:
+            res["terrain_level"] = rest[0]
+        return res

@@ -1,21 +1,38 @@
 """On-device PPO for a few hundred epochs on one GPU (4096 envs x 128 steps per epoch, the reference's hyper-parameters):
-episode statistics every 20 epochs, plus a finite-state check of the env.   python tools/ppo_learning_curve.py [epochs]"""
-import sys, time, torch
+episode statistics every 20 epochs, plus a finite-state check of the env.
+
+    python tools/ppo_learning_curve.py [epochs] [--terrain]
+
+--terrain trains on the generated sub-terrain grid with its curriculum and the height scan (terrain measure_heights:
+674 observation columns, PPOConfig(num_obs=674)) and adds the mean terrain level to the table."""
+import argparse, sys, time, torch
 sys.path.insert(0, '.')
 from isaacgymdyros_b200 import DyrosDynamicWalk, default_cfg
 from isaacgymdyros_b200.ppo import PPOConfig, PPOTrainer
-E = int(sys.argv[1]) if len(sys.argv) > 1 else 400
-env = DyrosDynamicWalk(default_cfg(4096), "cuda:0", use_cuda_graph=False)
-tr = PPOTrainer(env, PPOConfig())
-print("# On-device PPO, one B200, 4096 envs x 128 steps per epoch (DyrosDynamicWalkPPO.yaml hyper-parameters, self-collision on)\n")
-print("| epoch | frames | mean episode reward | mean episode length | episodes ended | actor loss | critic loss | kl | lr |")
-print("|---|---|---|---|---|---|---|---|---|")
+ap = argparse.ArgumentParser()
+ap.add_argument("epochs", nargs="?", type=int, default=400)
+ap.add_argument("--terrain", action="store_true", help="generated terrain, curriculum and measure_heights")
+args = ap.parse_args()
+E = args.epochs
+cfg = default_cfg(4096)
+if args.terrain:
+    cfg["env"]["terrain"] = {"curriculum": True, "measure_heights": True, "seed": 2}
+env = DyrosDynamicWalk(cfg, "cuda:0", use_cuda_graph=False)
+tr = PPOTrainer(env, PPOConfig(num_obs=env.num_obs))
+where = "curriculum terrain with the height scan" if args.terrain else "the plane"
+print(f"# On-device PPO, one B200, 4096 envs x 128 steps per epoch on {where}, {env.num_obs} observation columns "
+      "(DyrosDynamicWalkPPO.yaml hyper-parameters, self-collision on)\n")
+lvl = args.terrain
+print("| epoch | frames | mean episode reward | mean episode length | episodes ended |" + (" terrain level |" if lvl else "")
+      + " actor loss | critic loss | kl | lr |")
+print("|---|---|---|---|---|" + ("---|" if lvl else "") + "---|---|---|---|")
 t0 = time.time()
 for ep in range(1, E + 1):
     out = tr.train_epoch()
     if ep % 20 == 0 or ep == 1:
         print(f"| {ep} | {ep * 4096 * 128:,} | {out['mean_reward']:.1f} | {out['mean_length']:.1f} | {int(out['episodes'])} | "
-              f"{out['a_loss']:.4f} | {out['c_loss']:.3f} | {out['kl']:.5f} | {out['lr']:.2e} |", flush=True)
+              + (f"{out['terrain_level']:.2f} | " if lvl else "")
+              + f"{out['a_loss']:.4f} | {out['c_loss']:.3f} | {out['kl']:.5f} | {out['lr']:.2e} |", flush=True)
 torch.cuda.synchronize()
 dt = time.time() - t0
 finite = bool(torch.isfinite(env.core.sim_t["root_states"]).all() and torch.isfinite(env.core.sim_t["dof_state"]).all() and torch.isfinite(env.obs_buf).all())
