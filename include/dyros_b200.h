@@ -328,6 +328,26 @@ typedef struct {
   float* measured_heights;   /* (N,P) h_k in m; may be NULL */
 } DyrosHeightScan;
 int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* scan);
+/* Critic states (DESIGN.md section 4, "Critic states"): a privileged row per env for an asymmetric critic, written by
+ * the observation kernels beside the observation row, from the same post-reset root. With P the points of the height
+ * scan (0 without one), row e of `states` (N, S), S = 487 + P + 31, holds
+ *   0..486      the observation row's first 487 columns, bit for bit;
+ *   487..486+P  the height-scan columns clip(root_z - base_offset - h_k, -1, 1) * scale;
+ *   then 31 privileged columns, each clipped to [-5, 5]: root linear velocity (world, no noise) x 2, root angular
+ *   velocity x 0.25, net contact force of the left and right foot x 1e-3, push_force x 1e-2 (these two 0 at an episode
+ *   start, epi_len == 0), motor_constant_scale - 1 (12), total_mass / nominal_mass - 1, the env's ground friction - 1
+ *   (contact_friction[e], else the sim's friction), pd_gain_scale - 1 (2; 0 without the table).
+ * With states set and heights_in_obs == 0, the heights go into the state row ONLY: obs_buf rows (and the rows of
+ * dyros_task_pack_results) are 487 floats wide. With heights_in_obs != 0 they go into both rows (487 + P). `states`
+ * must hold N*S floats for the height scan in force at each launch. Call before a CUDA graph of the step is captured.
+ * NULL, or a NULL `states`, switches the rows off. `states` is caller-owned DEVICE memory that must stay alive while
+ * the task uses it. */
+typedef struct {
+  float* states;             /* (N, 487 + P + 31), 4-byte aligned */
+  int32_t heights_in_obs;    /* 0: the heights go into the state row only */
+  float nominal_mass;        /* > 0: the total mass the model was built with */
+} DyrosCriticStates;
+int dyros_task_set_critic_states(DyrosTask* task, const DyrosCriticStates* states);
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream);      /* VT:307 + T:449-502 */
 /* T:504-530 in one launch: skipframe x (substep torque, gym.simulate, sensor noise); what dyros_task_step uses. */
 int dyros_task_physics(DyrosTask* task, void* stream);
@@ -473,6 +493,19 @@ int dyros_ppo_unpack_grads(const DyrosPpoNet* net, float* flat_grad, float* norm
 int dyros_ppo_adam_packed(const DyrosPpoNet* net, float* params, const float* grads, float* exp_avg, float* exp_avg_sq, float grad_scale,
                           float max_norm, int norm_done, float* norm2_scratch, float* lr_dev, int32_t* step_dev, float beta1, float beta2,
                           float eps, float lr0, float lr_min, int lr_max_steps, void* stream);
+/* Asymmetric critic (DESIGN.md section 9): the same three calls for a critic of input width critic_inputs = Wc wider
+ * than the actor's Wa = net->inputs (0: Wc = Wa, exactly the calls above; otherwise Wc >= Wa, or refused). The flat
+ * master layout then holds the actor's W0 as H x Wa and the critic's as H x Wc; both packed W0 blocks share the leading
+ * dimension K0 = round_up(Wc, 8), so one bf16 input row of width K0 (the state row: its first Wa columns are the
+ * actor's observation) feeds both nets in one batched GEMM. Columns Wa..K0-1 of the actor's W0 are never written and
+ * stay zero: the actor is blind to the critic's extra columns. Run dyros_ppo_cast_obs / dyros_ppo_act with
+ * obs_dim = Wc on the state rows. */
+int dyros_ppo_pack_params_ac(const DyrosPpoNet* net, int critic_inputs, const float* flat, void* stream);
+int dyros_ppo_unpack_grads_ac(const DyrosPpoNet* net, int critic_inputs, float* flat_grad, float* norm2_accum, void* stream);
+int dyros_ppo_adam_packed_ac(const DyrosPpoNet* net, int critic_inputs, float* params, const float* grads, float* exp_avg,
+                             float* exp_avg_sq, float grad_scale, float max_norm, int norm_done, float* norm2_scratch, float* lr_dev,
+                             int32_t* step_dev, float beta1, float beta2, float eps, float lr0, float lr_min, int lr_max_steps,
+                             void* stream);
 
 /* ---- gradient exchange over peer memory (NVLink / NVSwitch): the Horovod all-reduce of AG:161-173 folded into the
  * optimiser's kernels. Every rank allocates two flat gradient buffers of `stride` floats (stride >= n, a multiple of 4,
@@ -501,6 +534,7 @@ int dyros_peer_close(void* ptr);
 int dyros_peer_free(void* ptr);
 /* dyros_ppo_unpack_grads into this rank's buffer of the current parity. */
 int dyros_ppo_unpack_grads_peers(const DyrosPpoNet* net, const DyrosPpoPeers* peers, void* stream);
+int dyros_ppo_unpack_grads_peers_ac(const DyrosPpoNet* net, int critic_inputs, const DyrosPpoPeers* peers, void* stream);
 /* Publishes this rank's buffer, waits for every rank's, and writes the SUM over ranks (in rank order: bit-identical on
  * every rank) to flat_grad_sum (local, n floats); norm2_accum += squared norm of its first n_actor entries. */
 int dyros_ppo_reduce_peers(const DyrosPpoPeers* peers, float* flat_grad_sum, int n, int n_actor, float* norm2_accum, void* stream);

@@ -24,6 +24,7 @@ NOBS = 487  # columns of an observation row without a height scan
 # height scan (legged_gym's measure_heights): obs = clip(root_z - BASE_OFFSET - h, -1, 1) * SCALE
 HEIGHT_SCAN_BASE_OFFSET, HEIGHT_SCAN_SCALE = 0.5, 5.0  # _get_heights / compute_observations, obs_scales.height_measurements
 MAX_HEIGHT_POINTS = 1024
+NPRIV = 31  # privileged columns at the end of a critic state row (DESIGN.md section 4, "Critic states")
 
 # T:58-70 (before the /9 and /3), T:296-301, T:95-100, T:366-371
 KP = [2000.0, 5000.0, 4000.0, 3700.0, 3200.0, 3200.0, 2000.0, 5000.0, 4000.0, 3700.0, 3200.0, 3200.0,
@@ -162,6 +163,11 @@ class CoreConfig:
     # (P, 2) points of the height scan in the base's yaw frame (legged_gym's height_points; DESIGN.md section 4, "Height
     # scan"), or None: each observation row gains P terrain heights around the base, on any ground
     height_scan: Optional[np.ndarray] = None
+    # critic states (DESIGN.md section 4, "Critic states"): task_t["states_buf"] (N, 487 + P + 31) gains a privileged row
+    # per env, written by the observation kernels; the P heights of a height scan then go into it and, only with
+    # critic_heights_in_obs, into the observation row as well
+    critic_states: bool = False
+    critic_heights_in_obs: bool = False
 
 
 def validate_height_points(points) -> np.ndarray:
@@ -305,7 +311,12 @@ class DyrosCore:
                 raise native.DyrosError("height scan: needs the task (its observation kernels measure the heights)")
             self.height_points = validate_height_points(self.cfg.height_scan)
         self.num_height_points = 0 if self.height_points is None else len(self.height_points)
-        self.obs_width = NOBS + self.num_height_points  # columns of obs_buf
+        cs = bool(self.cfg.critic_states)
+        if cs and not with_task:
+            raise native.DyrosError("critic states: need the task (its observation kernels write them)")
+        heights_in_obs = not cs or bool(self.cfg.critic_heights_in_obs)
+        self.obs_width = NOBS + (self.num_height_points if heights_in_obs else 0)  # columns of obs_buf
+        self.states_width = NOBS + self.num_height_points + NPRIV if cs else 0  # columns of states_buf (0: none)
         self.device = torch.device(device)
         self.tables = tables or ModelTables.load(os.path.join(ASSETS, "tocabi_tables.npz"))
         t = self.tables
@@ -367,6 +378,8 @@ class DyrosCore:
             tb["obs_buf"] = z(N, self.obs_width)
             tb["measured_heights"] = z(N, self.num_height_points)
             tb["height_points"] = torch.tensor(self.height_points, device=dev)
+        if self.states_width:
+            tb["states_buf"] = z(N, self.states_width)
         mocap = np.load(os.path.join(ASSETS, "mocap_walk.npy"))
         obs_norm = np.load(os.path.join(ASSETS, "obs_norm.npy"))
         tb["mocap_data"] = torch.tensor(mocap, device=dev).contiguous()
@@ -393,7 +406,8 @@ class DyrosCore:
         if cfg.heightfield is not None:  # start where the first reset puts the root (T:734-735), not above (0, 0)
             s["root_states"][:, 0:3] = tb["env_origins"]
             s["root_states"][:, 2] += cfg.initial_height
-        tb["total_mass"].fill_(float(np.float32(self.tables.total_mass())))
+        self.nominal_mass = float(np.float32(self.tables.total_mass()))  # (critic states: total_mass / nominal - 1)
+        tb["total_mass"].fill_(self.nominal_mass)
         tb["obs_hist_head"].fill_(19)
         tb["act_hist_head"].fill_(19)
 
@@ -426,9 +440,10 @@ class DyrosCore:
         return o.astype(np.float32)
 
     def _pack_state_arena(self):
-        """Moves every per-env buffer except obs_buf and measured_heights (written once per step, never read by the step)
-        into ONE contiguous allocation, 256-byte aligned views: the range dyros_sim_set_l2_persistence can pin in L2."""
-        items = [(d, k) for d in (self.sim_t, self.task_t) for k in d if k not in ("obs_buf", "measured_heights")]
+        """Moves every per-env buffer except obs_buf, states_buf and measured_heights (written once per step, never read
+        by the step) into ONE contiguous allocation, 256-byte aligned views: the range dyros_sim_set_l2_persistence can
+        pin in L2."""
+        items = [(d, k) for d in (self.sim_t, self.task_t) for k in d if k not in ("obs_buf", "states_buf", "measured_heights")]
         al = lambda n: (n + 255) & ~255
         total = sum(al(d[k].numel() * d[k].element_size()) for d, k in items)
         self.state_arena = torch.zeros(total, dtype=torch.uint8, device=self.device)
@@ -528,6 +543,12 @@ class DyrosCore:
             d.base_offset, d.scale = HEIGHT_SCAN_BASE_OFFSET, HEIGHT_SCAN_SCALE
             d.measured_heights = self.task_t["measured_heights"].data_ptr()
             native.check(self.lib.dyros_task_set_height_scan(self.task_handle, C.byref(d)), "dyros_task_set_height_scan")
+        if self.states_width:
+            d = native.DyrosCriticStates()
+            d.states = self.task_t["states_buf"].data_ptr()
+            d.heights_in_obs = int(bool(cfg.critic_heights_in_obs))
+            d.nominal_mass = self.nominal_mass
+            native.check(self.lib.dyros_task_set_critic_states(self.task_handle, C.byref(d)), "dyros_task_set_critic_states")
 
     def close(self):
         if getattr(self, "task_handle", None) and self.task_handle.value:

@@ -476,6 +476,18 @@ int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* sc) {
   t->scan = *sc;
   return 0;
 }
+int dyros_task_set_critic_states(DyrosTask* task, const DyrosCriticStates* cs) {
+  TASK_OR_FAIL("dyros_task_set_critic_states");
+  if (!cs || !cs->states) {
+    t->crit = DyrosCriticStates{};
+    return 0;
+  }
+  REQUIRE((reinterpret_cast<uintptr_t>(cs->states) & 3) == 0, "dyros_task_set_critic_states: states is not 4-byte aligned");
+  REQUIRE(std::isfinite(cs->nominal_mass) && cs->nominal_mass > 0.f,
+          "dyros_task_set_critic_states: nominal_mass must be finite and positive (got %g)", (double)cs->nominal_mass);
+  t->crit = *cs;
+  return 0;
+}
 int dyros_task_prologue(DyrosTask* task, const float* actions, void* stream) {
   TASK_OR_FAIL("dyros_task_prologue");
   if (!actions) {

@@ -123,6 +123,24 @@ struct HeightScan {
   FieldGround f;           // the sim's heightfield when has_field
 };
 
+// The critic's state row (DESIGN.md section 4, "Critic states"), a second compile-time parameter of the same kernels:
+// none, or rows of S = NOBS + P + kPrivCols floats written beside the observation rows: the observation row's NOBS
+// columns, the P heights of a height scan, then the privileged block.
+constexpr int kPrivCols = 31;
+struct NoStates {
+  static constexpr bool kOn = false;
+};
+struct CriticStates {
+  static constexpr bool kOn = true;
+  float* states;           // (N, S) (device memory)
+  int S;                   // NOBS + P + kPrivCols
+  int priv;                // first column of the privileged block: NOBS + P
+  int obs_w;               // columns of the observation row: NOBS, or NOBS + P with the heights in it
+  int heights_in_obs;      // the heights go into the observation row as well
+  float nominal_mass;      // total_mass / nominal_mass - 1 is column priv + 27
+  float mu;                // the sim's friction, for an env without a contact_friction table
+};
+
 struct SimParams {
   int N;
   float dt;       // dt / substeps: the integration step of one sub-step
@@ -189,8 +207,11 @@ struct Task {
   DyrosNoiseInjection inj;
   DyrosTerrainCurriculum cur{};  // dyros_task_set_terrain_curriculum; levels == NULL: off
   DyrosHeightScan scan{};        // dyros_task_set_height_scan; num_points == 0: off
+  DyrosCriticStates crit{};      // dyros_task_set_critic_states; states == NULL: off
   void* dev_blob = nullptr;
-  int obs_width() const { return NOBS + scan.num_points; }
+  // the heights of a height scan go into the observation row unless critic states take them alone
+  int obs_width() const { return NOBS + (!crit.states || crit.heights_in_obs ? scan.num_points : 0); }
+  int states_width() const { return NOBS + scan.num_points + kPrivCols; }
 };
 
 // launchers (task_kernels.cu)

@@ -436,8 +436,10 @@ __global__ void __launch_bounds__(256) k_ppo_loss_grad_packed(DyrosPpoBuffers b,
 }
 
 // master layout of the flat fp32 buffers (ppo.py FlatActorCritic): per net [W0 (H x W), b0 (H), W1 (H x H), b1 (H),
-// Wh (nout x H), bh (nout)], actor (nout 13) then critic (nout 1). The kernels below visit the master block's rows x cols
-// only, so the padding columns W..K0-1 of the packed W0 are never written and stay zero.
+// Wh (nout x H), bh (nout)], actor (nout 13, W = Wa) then critic (nout 1, W = Wc >= Wa: an asymmetric critic reads a
+// wider row). Both W0 blocks share one leading dimension K0 = round_up(Wc, 8). The kernels below visit the master
+// block's rows x cols only, so the columns Wa..K0-1 of the actor's packed W0 and Wc..K0-1 of the critic's are never
+// written and stay zero: the actor is blind to the columns past its own.
 struct PpoSeg {
   int master_off, rows, cols;  // the master block
   int dst_cols;                // leading dimension of the packed matrix (0: a bias vector)
@@ -447,12 +449,12 @@ struct PpoSeg {
 struct PpoSegs {
   PpoSeg s[12];
 };
-static PpoSegs ppo_segments(int hidden, int W) {
+static PpoSegs ppo_segments(int hidden, int Wa, int Wc) {
   PpoSegs S;
   int off = 0, k = 0;
   for (int net = 0; net < 2; ++net) {
-    const int nout = net == 0 ? PPO_NA : 1;
-    S.s[k++] = PpoSeg{off, hidden, W, ppo_padded_width(W), 0, net}; off += hidden * W;
+    const int nout = net == 0 ? PPO_NA : 1, W = net == 0 ? Wa : Wc;
+    S.s[k++] = PpoSeg{off, hidden, W, ppo_padded_width(Wc), 0, net}; off += hidden * W;
     S.s[k++] = PpoSeg{off, 1, hidden, 0, 1, net}; off += hidden;
     S.s[k++] = PpoSeg{off, hidden, hidden, hidden, 2, net}; off += hidden * hidden;
     S.s[k++] = PpoSeg{off, 1, hidden, 0, 3, net}; off += hidden;
@@ -859,20 +861,42 @@ int dyros_ppo_loss_grad_packed(const DyrosPpoBuffers* b, int row0, int mb, const
   DY_LAUNCH_CHECK();
   return 0;
 }
+// The critic's input width Wc of the *_ac entry points: 0 = the actor's (net->inputs); otherwise Wc >= the actor's.
+// Writes dyros_last_error and returns -1 for a bad width.
+static int ppo_critic_width(const DyrosPpoNet* net, int critic_inputs, const char* fn) {
+  if (net->inputs < 0) {
+    dyros::set_error("%s: DyrosPpoNet.inputs < 0 (0 means 487)", fn);
+    return -1;
+  }
+  const int Wa = ppo_width(net->inputs);
+  if (critic_inputs < 0 || (critic_inputs && critic_inputs < Wa)) {
+    dyros::set_error("%s: critic_inputs %d must be 0 (the actor's width) or >= the actor's %d", fn, critic_inputs, Wa);
+    return -1;
+  }
+  return critic_inputs ? critic_inputs : Wa;
+}
 int dyros_ppo_pack_params(const DyrosPpoNet* net, const float* flat, void* stream) {
+  return dyros_ppo_pack_params_ac(net, 0, flat, stream);
+}
+int dyros_ppo_pack_params_ac(const DyrosPpoNet* net, int critic_inputs, const float* flat, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && flat, "dyros_ppo_pack_params: bad argument");
-  PPO_CHECK(net->inputs >= 0, "dyros_ppo_pack_params: DyrosPpoNet.inputs < 0 (0 means 487)");
+  const int Wc = ppo_critic_width(net, critic_inputs, "dyros_ppo_pack_params");
+  if (Wc < 0) return 1;
   if (configure_ppo_kernels()) return 1;
-  k_ppo_pack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, flat);
+  k_ppo_pack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs), Wc), *net, flat);
   DY_LAUNCH_CHECK();
   return 0;
 }
 int dyros_ppo_unpack_grads(const DyrosPpoNet* net, float* flat_grad, float* norm2_accum, void* stream) {
+  return dyros_ppo_unpack_grads_ac(net, 0, flat_grad, norm2_accum, stream);
+}
+int dyros_ppo_unpack_grads_ac(const DyrosPpoNet* net, int critic_inputs, float* flat_grad, float* norm2_accum, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && net->gw0 && net->gw1 && net->gwh && net->gb0 && net->gb1 && net->gbh && flat_grad,
             "dyros_ppo_unpack_grads: bad argument");
-  PPO_CHECK(net->inputs >= 0, "dyros_ppo_unpack_grads: DyrosPpoNet.inputs < 0 (0 means 487)");
+  const int Wc = ppo_critic_width(net, critic_inputs, "dyros_ppo_unpack_grads");
+  if (Wc < 0) return 1;
   if (configure_ppo_kernels()) return 1;
-  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, flat_grad,
+  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs), Wc), *net, flat_grad,
                                                                norm2_accum, nullptr, 0);
   DY_LAUNCH_CHECK();
   return 0;
@@ -881,14 +905,22 @@ int dyros_ppo_unpack_grads(const DyrosPpoNet* net, float* flat_grad, float* norm
 int dyros_ppo_adam_packed(const DyrosPpoNet* net, float* params, const float* grads, float* exp_avg, float* exp_avg_sq, float grad_scale,
                           float max_norm, int norm_done, float* norm2_scratch, float* lr_dev, int32_t* step_dev, float beta1, float beta2,
                           float eps, float lr0, float lr_min, int lr_max_steps, void* stream) {
+  return dyros_ppo_adam_packed_ac(net, 0, params, grads, exp_avg, exp_avg_sq, grad_scale, max_norm, norm_done, norm2_scratch, lr_dev,
+                                  step_dev, beta1, beta2, eps, lr0, lr_min, lr_max_steps, stream);
+}
+int dyros_ppo_adam_packed_ac(const DyrosPpoNet* net, int critic_inputs, float* params, const float* grads, float* exp_avg,
+                             float* exp_avg_sq, float grad_scale, float max_norm, int norm_done, float* norm2_scratch, float* lr_dev,
+                             int32_t* step_dev, float beta1, float beta2, float eps, float lr0, float lr_min, int lr_max_steps,
+                             void* stream) {
   PPO_CHECK(ppo_net_ok(net) && params && grads && exp_avg && exp_avg_sq && norm2_scratch && lr_dev && step_dev, "dyros_ppo_adam_packed: bad argument");
-  PPO_CHECK(net->inputs >= 0, "dyros_ppo_adam_packed: DyrosPpoNet.inputs < 0 (0 means 487)");
+  const int Wc = ppo_critic_width(net, critic_inputs, "dyros_ppo_adam_packed");
+  if (Wc < 0) return 1;
   if (configure_ppo_kernels()) return 1;
   cudaStream_t s = (cudaStream_t)stream;
   const int H = net->hidden, W = ppo_width(net->inputs), n_actor = H * W + H + H * H + H + PPO_NA * H + PPO_NA;
   // norm2 holds the squared norm of the UNSCALED actor gradients (sum over ranks); the kernel scales it
   if (max_norm > 0.f && !norm_done) k_ppo_gradnorm<<<148, 256, 0, s>>>(grads, n_actor, 1.f, norm2_scratch);
-  k_ppo_adam_pack<<<dim3(64, 12), 256, 0, s>>>(ppo_segments(H, W), *net, params, grads, exp_avg, exp_avg_sq, grad_scale, max_norm, norm2_scratch,
+  k_ppo_adam_pack<<<dim3(64, 12), 256, 0, s>>>(ppo_segments(H, W, Wc), *net, params, grads, exp_avg, exp_avg_sq, grad_scale, max_norm, norm2_scratch,
                                               lr_dev, step_dev, beta1, beta2, eps);
   k_ppo_adam_finish<<<1, 1, 0, s>>>(norm2_scratch, step_dev, lr_dev, lr0, lr_min, lr_max_steps);
   DY_LAUNCH_CHECK();
@@ -902,12 +934,16 @@ static bool ppo_peers_ok(const DyrosPpoPeers* p) {
   return true;
 }
 int dyros_ppo_unpack_grads_peers(const DyrosPpoNet* net, const DyrosPpoPeers* peers, void* stream) {
+  return dyros_ppo_unpack_grads_peers_ac(net, 0, peers, stream);
+}
+int dyros_ppo_unpack_grads_peers_ac(const DyrosPpoNet* net, int critic_inputs, const DyrosPpoPeers* peers, void* stream) {
   PPO_CHECK(ppo_net_ok(net) && net->gw0 && net->gw1 && net->gwh && net->gb0 && net->gb1 && net->gbh && ppo_peers_ok(peers),
             "dyros_ppo_unpack_grads_peers: bad argument");
   PPO_CHECK(peers->grad[peers->rank][1] == peers->grad[peers->rank][0] + peers->stride, "dyros_ppo_unpack_grads_peers: the rank's two buffers must be `stride` apart");
-  PPO_CHECK(net->inputs >= 0, "dyros_ppo_unpack_grads_peers: DyrosPpoNet.inputs < 0 (0 means 487)");
+  const int Wc = ppo_critic_width(net, critic_inputs, "dyros_ppo_unpack_grads_peers");
+  if (Wc < 0) return 1;
   if (configure_ppo_kernels()) return 1;
-  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs)), *net, peers->grad[peers->rank][0], nullptr, peers->epoch,
+  k_ppo_unpack<<<dim3(64, 12), 256, 0, (cudaStream_t)stream>>>(ppo_segments(net->hidden, ppo_width(net->inputs), Wc), *net, peers->grad[peers->rank][0], nullptr, peers->epoch,
                                                                (size_t)peers->stride);
   DY_LAUNCH_CHECK();
   return 0;

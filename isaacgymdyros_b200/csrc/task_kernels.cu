@@ -324,9 +324,11 @@ __host__ __device__ inline int obs_width(const HeightScan& sc) { return NOBS + s
 // term of compute_observations), one warp: lane l takes points l, l + 32, ...; the sample gathers of up to kScanBatch
 // points per lane (all of them for P <= 256) are issued before the first is used. (x, y, z) is the root's position,
 // (qz, qw) the z and w components of its quaternion, `ob` the env's observation row (columns NOBS + k are written).
+// kStates: the columns go to the state row `sr` as well, and to `ob` only if it is not NULL.
 constexpr int kScanBatch = 8;
+template <bool kStates = false>
 __device__ __forceinline__ void stage_height_scan(const HeightScan& sc, int e, int lane, float x, float y, float z,
-                                                  float qz, float qw, float* ob) {
+                                                  float qz, float qw, float* ob, float* sr = nullptr) {
   const float n = fmaxf(sqrtf(qz * qz + qw * qw), 1e-9f);  // TU normalize of the quaternion with x = y = 0
   const float yz = qz / n, yw = qw / n;
   const float zb = z - sc.base_offset;
@@ -358,16 +360,44 @@ __device__ __forceinline__ void stage_height_scan(const HeightScan& sc, int e, i
       const int k = k0 + lane + b * kWarp;
       if (k < sc.P) {
         const float h = sc.has_field ? f.oz + f.dz * (float)min(min(s0[b], s1[b]), s2[b]) : 0.0f;  // plane: 0
-        ob[NOBS + k] = fminf(fmaxf(zb - h, -1.0f), 1.0f) * sc.scale;
+        const float v = fminf(fmaxf(zb - h, -1.0f), 1.0f) * sc.scale;
+        if constexpr (kStates) {
+          if (ob) ob[NOBS + k] = v;
+          sr[NOBS + k] = v;
+        } else {
+          ob[NOBS + k] = v;
+        }
         if (mh) mh[k] = h;
       }
     }
   }
 }
 
-// T:750-796 (history kept as rings, see DyrosTaskBuffers), then the height scan if there is one
-template <class Scan>
-__device__ void stage_compute_observations(const TK& k, int e, int lane, const Scan& sc) {
+// Privileged block of the state row (DESIGN.md section 4, "Critic states"): lane c < kPrivCols writes column
+// st.priv + c of `sr` from the post-reset state in global memory; `start`: the env is at an episode start (T:785), where
+// the contact-force and push columns are 0. Every column is clipped to [-5, 5] (fminf / fmaxf: a NaN becomes -5).
+__device__ __forceinline__ void stage_critic_privileged(const TK& k, const CriticStates& st, int e, int lane, bool start,
+                                                        float* sr) {
+  if (lane >= kPrivCols) return;
+  const size_t E = (size_t)e;
+  float v;
+  if (lane < 3) v = __fmul_rn(k.s.root_states[E * 13 + 7 + lane], 2.0f);                  // linear velocity (world)
+  else if (lane < 6) v = __fmul_rn(k.s.root_states[E * 13 + 7 + lane], 0.25f);           // angular velocity (world)
+  else if (lane < 12) {                                                                  // foot contact forces
+    const int b = lane < 9 ? k.p.lfoot : k.p.rfoot, c = lane < 9 ? lane - 6 : lane - 9;
+    v = start ? 0.0f : __fmul_rn(k.s.net_contact_force[(E * NB + b) * 3 + c], 1e-3f);
+  } else if (lane < 15) v = start ? 0.0f : __fmul_rn(k.b.push_force[E * 3 + (lane - 12)], 1e-2f);  // pelvis push
+  else if (lane < 27) v = __fsub_rn(k.b.motor_constant_scale[E * 12 + (lane - 15)], 1.0f);
+  else if (lane == 27) v = __fsub_rn(__fdiv_rn(k.b.total_mass[e], st.nominal_mass), 1.0f);
+  else if (lane == 28) v = __fsub_rn(k.s.contact_friction ? k.s.contact_friction[e] : st.mu, 1.0f);
+  else v = k.b.pd_gain_scale ? __fsub_rn(k.b.pd_gain_scale[E * 2 + (lane - 29)], 1.0f) : 0.0f;
+  sr[st.priv + lane] = fminf(fmaxf(v, -5.0f), 5.0f);
+}
+
+// T:750-796 (history kept as rings, see DyrosTaskBuffers), then the height scan if there is one, then the privileged
+// block of the critic states if they are on
+template <class Scan, class St>
+__device__ void stage_compute_observations(const TK& k, int e, int lane, const Scan& sc, const St& st) {
   const TaskParams& P = k.p;
   const float* root = k.s.root_states + (size_t)e * 13;
   float time = k.b.time[e];
@@ -405,8 +435,11 @@ __device__ void stage_compute_observations(const TK& k, int e, int lane, const S
   __syncwarp();
   if (lane == 0) k.b.obs_hist_head[e] = head;
   float* ob;
-  if constexpr (Scan::kOn) ob = k.b.obs_buf + (size_t)e * obs_width(sc);
+  if constexpr (St::kOn) ob = k.b.obs_buf + (size_t)e * st.obs_w;
+  else if constexpr (Scan::kOn) ob = k.b.obs_buf + (size_t)e * obs_width(sc);
   else ob = k.b.obs_buf + (size_t)e * NOBS;  // (spelt out: the default instantiation keeps its instruction stream)
+  float* sr = nullptr;
+  if constexpr (St::kOn) sr = st.states + (size_t)e * st.S;
   const float* ah = k.b.action_history + (size_t)e * NSLOT * NA;
   int ahead = k.b.act_hist_head[e];
   // gather: all loads first (the compiler cannot reorder them across the stores itself), then the stores
@@ -432,9 +465,18 @@ __device__ void stage_compute_observations(const TK& k, int e, int lane, const S
 #pragma unroll
   for (int it = 0; it < IT; ++it) {
     int o = lane + it * kWarp;
-    if (o < NOBS) ob[o] = vals[it];
+    if (o < NOBS) {
+      ob[o] = vals[it];
+      if constexpr (St::kOn) sr[o] = vals[it];  // the state row's prefix: a second store of the same value
+    }
   }
-  if constexpr (Scan::kOn) stage_height_scan(sc, e, lane, root[0], root[1], root[2], root[5], root[6], ob);
+  if constexpr (Scan::kOn) {
+    if constexpr (St::kOn)
+      stage_height_scan<true>(sc, e, lane, root[0], root[1], root[2], root[5], root[6], st.heights_in_obs ? ob : nullptr, sr);
+    else
+      stage_height_scan(sc, e, lane, root[0], root[1], root[2], root[5], root[6], ob);
+  }
+  if constexpr (St::kOn) stage_critic_privileged(k, st, e, lane, start, sr);
 }
 
 // T:560-563 (loads of all four copies are issued before the first store)
@@ -509,10 +551,10 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_reset_idx(TK k, const i
   if (e < 0 || e >= k.p.N) return;
   stage_reset_env(k, (int)e, lane);
 }
-template <class Scan>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_compute_observations(TK k, Scan sc) {
+template <class Scan, class St>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_compute_observations(TK k, Scan sc, St st) {
   ENV_LANE();
-  stage_compute_observations(k, e, lane, sc);
+  stage_compute_observations(k, e, lane, sc, st);
 }
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_late_update(TK k) {
   ENV_LANE();
@@ -571,10 +613,11 @@ __device__ __forceinline__ bool gate_open(const TaskParams& P, long long s0, lon
 }
 
 // 4 warps per CTA, 7 CTAs per SM: 4096 envs (1024 CTAs) are resident on 148 SMs in ONE wave at <= 73 registers per thread
-// (instantiated without and with the height scan, which runs last, from the post-reset root of the observation stage)
+// (instantiated without and with the height scan, which runs last, from the post-reset root of the observation stage,
+// and without and with the critic states, whose privileged block runs after it)
 constexpr int kPostWarps = 4;
-template <class Scan>
-__global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tail, Scan sc) {
+template <class Scan, class St>
+__global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tail, Scan sc, St st) {
   __shared__ long long gate_acc[2][kPostWarps];
   __shared__ int level_acc[kPostWarps];
   pdl_launch_dependents();
@@ -833,7 +876,9 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
       if (lane == 0) k.b.obs_hist_head[e] = head;
     }
     {
-      float* ob = k.b.obs_buf + E * obs_width(sc);
+      float* ob;                                                                       // (with critic states the heights may
+      if constexpr (St::kOn) ob = k.b.obs_buf + E * st.obs_w;                          //  live in the state row only)
+      else ob = k.b.obs_buf + E * obs_width(sc);
 #pragma unroll
       for (int i = 0; i < NHIS; ++i) {                                                 // T:789-791
         const bool newest = start || i == NHIS - 1;                                    // (T:786-787: at an episode start every slot holds this frame)
@@ -843,6 +888,18 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
 #pragma unroll
       for (int i = 0; i < NHIS - 1; ++i)                                               // T:793-796
         if (lane < NA) ob[NOBS1 * NHIS + NA * i + lane] = hC[i];
+      if constexpr (St::kOn) {  // the state row's prefix: the same registers stored a second time
+        float* sr = st.states + E * st.S;
+#pragma unroll
+        for (int i = 0; i < NHIS; ++i) {
+          const bool newest = start || i == NHIS - 1;
+          sr[NOBS1 * i + lane] = newest ? nvA : hA[i < NHIS - 1 ? i : 0];
+          if (lane < NOBS1 - 32) sr[NOBS1 * i + 32 + lane] = newest ? nvB : hB[i < NHIS - 1 ? i : 0];
+        }
+#pragma unroll
+        for (int i = 0; i < NHIS - 1; ++i)
+          if (lane < NA) sr[NOBS1 * NHIS + NA * i + lane] = hC[i];
+      }
     }
     // ================================================================ late update (T:560-563)
     k.b.pre_joint_velocity_states[E * ND + lane] = in.vel0;
@@ -856,8 +913,14 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     // ================================================================ height scan (DESIGN.md section 4)
     if constexpr (Scan::kOn) {
       const float rx = __shfl_sync(kFull, in.root, 0), ry = __shfl_sync(kFull, in.root, 1), rz = __shfl_sync(kFull, in.root, 2);
-      stage_height_scan(sc, e, lane, rx, ry, rz, quat[2], quat[3], k.b.obs_buf + E * obs_width(sc));
+      if constexpr (St::kOn)
+        stage_height_scan<true>(sc, e, lane, rx, ry, rz, quat[2], quat[3],
+                                st.heights_in_obs ? k.b.obs_buf + E * st.obs_w : nullptr, st.states + E * st.S);
+      else
+        stage_height_scan(sc, e, lane, rx, ry, rz, quat[2], quat[3], k.b.obs_buf + E * obs_width(sc));
     }
+    // ================================================================ privileged block of the critic states (section 4)
+    if constexpr (St::kOn) stage_critic_privileged(k, st, e, lane, start, st.states + E * st.S);
   }
 }
 
@@ -1036,6 +1099,17 @@ static inline HeightScan make_scan(const Task* t) {
   sc.f = t->sim->field;
   return sc;
 }
+static inline CriticStates make_states(const Task* t) {
+  CriticStates st;
+  st.states = t->crit.states;
+  st.S = t->states_width();
+  st.priv = NOBS + t->scan.num_points;
+  st.obs_w = t->obs_width();
+  st.heights_in_obs = t->crit.heights_in_obs ? 1 : 0;
+  st.nominal_mass = t->crit.nominal_mass;
+  st.mu = t->sim->p.mu;
+  return st;
+}
 static inline int env_grid(int N) { return (N + kWarpsPerBlock - 1) / kWarpsPerBlock; }
 #define LAUNCH_ENV(kern, ...)                                                    \
   kern<<<env_grid(t->p.N), kWarpsPerBlock * 32, 0, s>>>(make_tk(t), ##__VA_ARGS__); \
@@ -1049,27 +1123,45 @@ int launch_epilogue(Task* t, cudaStream_t s) { LAUNCH_ENV(k_epilogue) }
 int launch_check_termination(Task* t, cudaStream_t s) { LAUNCH_ENV(k_check_termination) }
 int launch_compute_reward(Task* t, cudaStream_t s) { LAUNCH_ENV(k_compute_reward) }
 int launch_compute_observations(Task* t, cudaStream_t s) {
-  if (t->scan.num_points) { LAUNCH_ENV(k_compute_observations<HeightScan>, make_scan(t)) }
-  LAUNCH_ENV(k_compute_observations<NoScan>, NoScan())
+  if (t->crit.states) {
+    if (t->scan.num_points) { LAUNCH_ENV((k_compute_observations<HeightScan, CriticStates>), make_scan(t), make_states(t)) }
+    LAUNCH_ENV((k_compute_observations<NoScan, CriticStates>), NoScan(), make_states(t))
+  }
+  if (t->scan.num_points) { LAUNCH_ENV((k_compute_observations<HeightScan, NoStates>), make_scan(t), NoStates()) }
+  LAUNCH_ENV((k_compute_observations<NoScan, NoStates>), NoScan(), NoStates())
 }
 int launch_late_update(Task* t, cudaStream_t s) { LAUNCH_ENV(k_late_update) }
 int configure_task_kernels() {
   DY_CUDA(prefer_max_smem_carveout(k_prologue)); DY_CUDA(prefer_max_smem_carveout(k_substep_torque));
   DY_CUDA(prefer_max_smem_carveout(k_sensor_noise)); DY_CUDA(prefer_max_smem_carveout(k_epilogue));
   DY_CUDA(prefer_max_smem_carveout(k_check_termination)); DY_CUDA(prefer_max_smem_carveout(k_compute_reward));
-  DY_CUDA(prefer_max_smem_carveout(k_compute_observations<NoScan>));
-  DY_CUDA(prefer_max_smem_carveout(k_compute_observations<HeightScan>)); DY_CUDA(prefer_max_smem_carveout(k_late_update));
+  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<NoScan, NoStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<HeightScan, NoStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<NoScan, CriticStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<HeightScan, CriticStates>)));
+  DY_CUDA(prefer_max_smem_carveout(k_late_update));
   DY_CUDA(prefer_max_smem_carveout(k_reset_idx)); DY_CUDA(prefer_max_smem_carveout(k_pack_results));
-  DY_CUDA(prefer_max_smem_carveout(k_post_fused<NoScan>)); DY_CUDA(prefer_max_smem_carveout(k_post_fused<HeightScan>));
+  DY_CUDA(prefer_max_smem_carveout((k_post_fused<NoScan, NoStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_post_fused<HeightScan, NoStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_post_fused<NoScan, CriticStates>)));
+  DY_CUDA(prefer_max_smem_carveout((k_post_fused<HeightScan, CriticStates>)));
   DY_CUDA(prefer_max_smem_carveout(k_crossenv));
   return 0;
 }
 int launch_post_fused(Task* t, cudaStream_t s, bool pdl, bool tail) {
   const dim3 grid((t->p.N + kPostWarps - 1) / kPostWarps), block(kPostWarps * 32);
-  if (t->scan.num_points)
-    DY_CUDA(launch_kernel(k_post_fused<HeightScan>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t)));
-  else
-    DY_CUDA(launch_kernel(k_post_fused<NoScan>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan()));
+  if (t->crit.states) {
+    if (t->scan.num_points)
+      DY_CUDA(launch_kernel(k_post_fused<HeightScan, CriticStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t),
+                            make_states(t)));
+    else
+      DY_CUDA(launch_kernel(k_post_fused<NoScan, CriticStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan(),
+                            make_states(t)));
+  } else if (t->scan.num_points) {
+    DY_CUDA(launch_kernel(k_post_fused<HeightScan, NoStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t), NoStates()));
+  } else {
+    DY_CUDA(launch_kernel(k_post_fused<NoScan, NoStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan(), NoStates()));
+  }
   return 0;
 }
 int launch_reset_idx(Task* t, const int64_t* env_ids, int count, cudaStream_t s) {

@@ -105,6 +105,10 @@ class DyrosHeightScan(C.Structure):
                 ("measured_heights", C.c_void_p)]
 
 
+class DyrosCriticStates(C.Structure):
+    _fields_ = [("states", C.c_void_p), ("heights_in_obs", i32), ("nominal_mass", f32)]
+
+
 NOISE_FIELDS = ["qpos_normal", "vel_u", "reset_f", "reset_i", "pert_i", "pert_f", "dr_u"]
 
 
@@ -145,15 +149,20 @@ SIGNATURES = {
     "dyros_ppo_loss_grad_packed": (_INT, [_PB, _INT, _INT, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "dyros_ppo_pack_params": (_INT, [_PN, _VP, _VP]),
     "dyros_ppo_unpack_grads": (_INT, [_PN, _VP, _VP, _VP]),
+    "dyros_ppo_pack_params_ac": (_INT, [_PN, _INT, _VP, _VP]),
+    "dyros_ppo_unpack_grads_ac": (_INT, [_PN, _INT, _VP, _VP, _VP]),
     "dyros_peer_alloc": (_INT, [C.c_size_t, C.POINTER(_VP), C.c_char_p]),
     "dyros_peer_open": (_INT, [C.c_char_p, C.POINTER(_VP)]),
     "dyros_peer_close": (_INT, [_VP]),
     "dyros_peer_free": (_INT, [_VP]),
     "dyros_ppo_unpack_grads_peers": (_INT, [_PN, C.POINTER(DyrosPpoPeers), _VP]),
+    "dyros_ppo_unpack_grads_peers_ac": (_INT, [_PN, _INT, C.POINTER(DyrosPpoPeers), _VP]),
     "dyros_ppo_reduce_peers": (_INT, [C.POINTER(DyrosPpoPeers), _VP, _INT, _INT, _VP, _VP]),
     "dyros_ppo_reduce_scatter_peers": (_INT, [C.POINTER(DyrosPpoPeers), _VP, _INT, _INT, _VP]),
     "dyros_ppo_all_gather_peers": (_INT, [C.POINTER(DyrosPpoPeers), _VP, _INT, _VP, _VP]),
     "dyros_ppo_adam_packed": (_INT, [_PN, _VP, _VP, _VP, _VP, f32, f32, _INT, _VP, _VP, _VP, f32, f32, f32, f32, f32, _INT, _VP]),
+    "dyros_ppo_adam_packed_ac": (_INT, [_PN, _INT, _VP, _VP, _VP, _VP, f32, f32, _INT, _VP, _VP, _VP, f32, f32, f32, f32, f32, _INT,
+                                        _VP]),
     "dyros_last_error": (C.c_char_p, []),
     "dyros_abi_version": (_INT, []),
     "dyros_sim_set_l2_persistence": (_INT, [_VP, _VP, C.c_size_t, _VP, C.POINTER(C.c_size_t)]),
@@ -174,6 +183,7 @@ SIGNATURES = {
     "dyros_task_set_noise_injection": (_INT, [_VP, C.POINTER(DyrosNoiseInjection)]),
     "dyros_task_set_terrain_curriculum": (_INT, [_VP, C.POINTER(DyrosTerrainCurriculum)]),
     "dyros_task_set_height_scan": (_INT, [_VP, C.POINTER(DyrosHeightScan)]),
+    "dyros_task_set_critic_states": (_INT, [_VP, C.POINTER(DyrosCriticStates)]),
     "dyros_task_prologue": (_INT, [_VP, _VP, _VP]),
     "dyros_task_physics": (_INT, [_VP, _VP]),
     "dyros_task_physics_kernel": (_INT, [_VP, _VP]),

@@ -9,10 +9,14 @@ all-reduce of the flat 1.54 MB gradient bucket per minibatch (AG:161-203) plus a
 
 The two W-256-256-{13,1} MLPs are library GEMMs (torch / cuBLAS); parameters, gradients and Adam moments live in flat
 fp32 buffers. W = PPOConfig.num_obs, the env's observation width: the reference's 487, or 674 with the default height scan
-(terrain measure_heights). Both networks see the whole row. Two network paths:
+(terrain measure_heights). Both networks see the whole row, unless PPOConfig.num_states asks for an asymmetric critic:
+the critic then reads the env's critic state row (num_states = Wc columns, DESIGN.md section 4, "Critic states"), whose
+first num_obs columns are the observation row, and the actor reads those first num_obs columns only. Two network
+paths:
   * `mixed_precision="bf16"` (default; the reference trains under fp16 autocast + GradScaler, PPO:59): `PackedNets` --
     actor and critic as ONE batch-2 problem in GEMM layout (bf16 weights, input width padded to K0 = round_up(W, 8):
-    487 -> 488, 674 -> 680), 8 batched
+    487 -> 488, 674 -> 680; with critic states W = Wc, 705 -> 712, and the actor's W0 is zero past its num_obs
+    columns), 8 batched
     GEMMs per minibatch with hand-written backward and the library's own kernels in between (csrc/ppo_kernels.cu,
     "packed bf16 path"): 21 launches per minibatch instead of 79;
   * `mixed_precision="fp32"`: torch autograd on views of the flat buffers (what the tests pin against the oracle)."""
@@ -64,13 +68,17 @@ class PPOConfig:
     graph_span: str = "mini_epoch"          # one CUDA graph per "minibatch" update, or one for all minibatches of a "mini_epoch"
     num_obs: int = NOBS                     # input width of both networks = the env's num_obs (network_builder_dyros.py
                                             # takes it from the observation space); 674 with the default height scan
+    num_states: int = 0                     # > 0: asymmetric critic, whose input is the env's critic state row of this
+                                            # width (= env.num_states, criticStates); 0: the critic reads the observation row
 
 
-def layer_shapes(units=(256, 256), num_obs=NOBS):
-    """(name, out, in) of the actor and the critic (network_builder_dyros.py:129-216, `separate: True`)."""
+def layer_shapes(units=(256, 256), num_obs=NOBS, num_states=0):
+    """(name, out, in) of the actor and the critic (network_builder_dyros.py:129-216, `separate: True`); the critic's
+    input width is num_states if > 0 (asymmetric critic), else num_obs."""
     dims = [num_obs] + list(units)
+    cdims = [num_states or num_obs] + list(units)
     actor = [(f"actor_mlp.{i}", dims[i + 1], dims[i]) for i in range(len(units))] + [("mu", NA, dims[-1])]
-    critic = [(f"critic_mlp.{i}", dims[i + 1], dims[i]) for i in range(len(units))] + [("value", 1, dims[-1])]
+    critic = [(f"critic_mlp.{i}", cdims[i + 1], cdims[i]) for i in range(len(units))] + [("value", 1, cdims[-1])]
     return actor, critic
 
 
@@ -80,7 +88,11 @@ class FlatActorCritic:
 
     def __init__(self, device, cfg: PPOConfig):
         self.cfg, self.device = cfg, torch.device(device)
-        actor, critic = layer_shapes(cfg.units, cfg.num_obs)
+        if cfg.num_states and cfg.num_states < cfg.num_obs:
+            raise ValueError(f"PPOConfig.num_states = {cfg.num_states} < num_obs = {cfg.num_obs}: a critic state row starts "
+                             "with the observation row")
+        actor, critic = layer_shapes(cfg.units, cfg.num_obs, cfg.num_states)
+        self.critic_inputs = cfg.num_states or cfg.num_obs
         self.n_actor = sum(o * i + o for _, o, i in actor)
         self.n = self.n_actor + sum(o * i + o for _, o, i in critic)
         self.flat = torch.zeros(self.n, device=device)
@@ -195,10 +207,11 @@ class FlatActorCritic:
         return F.linear(x, w, b)
 
     def forward(self, obs):
-        """mu (B,13), value (B) -- `mu_activation: None`, value head linear (PPO:17-18)."""
+        """mu (B,13), value (B) -- `mu_activation: None`, value head linear (PPO:17-18). With an asymmetric critic `obs`
+        is a batch of critic state rows: the actor takes their first num_obs columns."""
         amp = self.cfg.mixed_precision == "bf16"
         with torch.autocast("cuda", dtype=torch.bfloat16, enabled=amp and obs.is_cuda):
-            mu = self._mlp(obs, "actor_mlp", "mu")
+            mu = self._mlp(obs[..., :self.cfg.num_obs] if obs.shape[-1] != self.cfg.num_obs else obs, "actor_mlp", "mu")
             v = self._mlp(obs, "critic_mlp", "value")
         return mu, v.squeeze(-1)
 
@@ -206,7 +219,8 @@ class FlatActorCritic:
 class PackedNets:
     """bf16 compute copies of the flat master parameters in GEMM layout (include/dyros_b200.h DyrosPpoNet) and the
     forward / backward of both networks as batch-2 GEMMs. Activations of the last `forward` are kept for `backward`.
-    K0 = round_up(num_obs, 8) is the padded input width of W0 and of the bf16 observation rows (columns num_obs.. zero)."""
+    K0 = round_up(Wc, 8) is the padded input width of W0 and of the bf16 input rows, Wc the critic's input width
+    (num_states, or num_obs): columns num_obs.. of the actor's W0 and Wc.. of the critic's and of the rows are zero."""
     HEAD = 16
 
     def __init__(self, net: FlatActorCritic, lib):
@@ -214,7 +228,8 @@ class PackedNets:
             raise ValueError("the packed path holds two hidden layers of equal width (a multiple of 8), PPO:28-35")
         self.net, self.lib, dev = net, lib, net.device
         Hd = self.hidden = net.cfg.units[0]
-        self.K0 = (net.cfg.num_obs + 7) // 8 * 8
+        self.critic_inputs = net.cfg.num_states  # (0: the actor's width; the *_ac entry points take it)
+        self.K0 = (net.critic_inputs + 7) // 8 * 8
         zb = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)
         zf = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)
         self.w0, self.w1, self.wh = zb(2, Hd, self.K0), zb(2, Hd, Hd), zb(2, self.HEAD, Hd)
@@ -234,10 +249,11 @@ class PackedNets:
         return C.c_void_p(torch.cuda.current_stream(self.net.device).cuda_stream)
 
     def pack(self):
-        native.check(self.lib.dyros_ppo_pack_params(C.byref(self.desc), C.c_void_p(self.net.flat.data_ptr()), self._stream), "pack")
+        native.check(self.lib.dyros_ppo_pack_params_ac(C.byref(self.desc), self.critic_inputs, C.c_void_p(self.net.flat.data_ptr()),
+                                                       self._stream), "pack")
 
     def unpack_grads(self, norm2: Optional[torch.Tensor] = None):
-        native.check(self.lib.dyros_ppo_unpack_grads(C.byref(self.desc), C.c_void_p(self.net.grad.data_ptr()),
+        native.check(self.lib.dyros_ppo_unpack_grads_ac(C.byref(self.desc), self.critic_inputs, C.c_void_p(self.net.grad.data_ptr()),
                                                      C.c_void_p(norm2.data_ptr()) if norm2 is not None else None, self._stream), "unpack")
 
     def _buffers(self, rows: int):
@@ -348,6 +364,12 @@ class PPOTrainer:
             raise ValueError(f"PPOTrainer: the networks take PPOConfig.num_obs = {cfg.num_obs} observation columns; this env "
                              f"has {env.num_obs} (a height scan, terrain measure_heights, adds its heights to each row). "
                              f"Train it with PPOConfig(num_obs={env.num_obs})")
+        if cfg.num_states and (not getattr(env, "critic_states", False) or env.num_states != cfg.num_states):
+            has = getattr(env, "critic_states", False)
+            raise ValueError(f"PPOTrainer: the critic takes PPOConfig.num_states = {cfg.num_states} state columns; this env "
+                             + (f"has critic state rows of {env.num_states}. " if has else
+                                "has no kernel-written critic states (set cfg['env']['criticStates']). ")
+                             + "Train it with PPOConfig(num_states=env.num_states)")
         self.env, self.cfg = env, cfg
         self.rank, self.world = rank, world
         self.lib = native.load()
@@ -368,15 +390,16 @@ class PPOTrainer:
         self.peers: Optional[PeerGrads] = (PeerGrads(self.net.n, dev, rank, world)
                                            if world > 1 and self.packed is not None and c.grad_sync in ("peer", "peer2") else None)
         if self.packed is not None:  # the rollout's observations are kept as the bf16 rows the GEMMs read (N*H x K0)
-            self.x_step = z(N, self.packed.K0, dt=torch.bfloat16)
+            self.x_step = z(N, self.packed.K0, dt=torch.bfloat16)  # (rows of the critic's width: both nets read them)
             self.x_roll = z(N * H, self.packed.K0, dt=torch.bfloat16)
-        self.buf = {"obs": z(N, H, c.num_obs) if self.packed is None else z(1), "actions": z(N, H, NA), "mus": z(N, H, NA), "neglogp": z(N, H), "values": z(N, H),
+        self.W = self.net.critic_inputs  # columns of a stored input row: the state row with an asymmetric critic
+        self.buf = {"obs": z(N, H, self.W) if self.packed is None else z(1), "actions": z(N, H, NA), "mus": z(N, H, NA), "neglogp": z(N, H), "values": z(N, H),
                     "rewards": z(N, H), "dones": z(N, H), "advantages": z(N, H), "returns": z(N, H), "cur_reward": z(N),
                     "cur_length": z(N), "ep_stats": z(3), "step": z(1, dt=torch.int32), "global_step": z(1, dt=torch.int64)}
         pb = native.DyrosPpoBuffers()
         pb.N, pb.H, pb.gamma, pb.tau, pb.e_clip, pb.critic_coef = N, H, c.gamma, c.tau, c.e_clip, c.critic_coef
         pb.reward_scale, pb.value_bootstrap, pb.seed = c.reward_scale, int(c.value_bootstrap), c.seed + 7919 * (rank + 1)
-        pb.obs_dim = c.num_obs
+        pb.obs_dim = self.W
         for k, t in self.buf.items():
             setattr(pb, k, t.data_ptr())
         self.pb = pb
@@ -402,8 +425,13 @@ class PPOTrainer:
         return C.c_void_p(t.data_ptr()) if t is not None else None
 
     # ------------------------------------------------------------------ rollout (A2C:629-703)
+    @property
+    def _input_rows(self) -> torch.Tensor:
+        """What the networks read: the env's critic state rows with an asymmetric critic, else its observation rows."""
+        return self.env.states_buf if self.cfg.num_states else self.env.obs_buf
+
     def _cast_obs(self, into_rollout: bool):
-        native.check(self.lib.dyros_ppo_cast_obs(C.byref(self.pb), self._p(self.env.obs_buf), self._p(self.x_step),
+        native.check(self.lib.dyros_ppo_cast_obs(C.byref(self.pb), self._p(self._input_rows), self._p(self.x_step),
                                                  self._p(self.x_roll) if into_rollout else None, self._stream), "dyros_ppo_cast_obs")
 
     def _rollout_step_packed(self):
@@ -422,9 +450,9 @@ class PPOTrainer:
             return self._rollout_step_packed()
         env = self.env
         with torch.no_grad():
-            mu, v = self.net.forward(env.obs_buf)
+            mu, v = self.net.forward(self._input_rows)
             mu, v = mu.float().contiguous(), v.float().contiguous()
-        native.check(self.lib.dyros_ppo_act(C.byref(self.pb), self._p(mu), self._p(v), self._p(self.net.logstd), self._p(env.obs_buf),
+        native.check(self.lib.dyros_ppo_act(C.byref(self.pb), self._p(mu), self._p(v), self._p(self.net.logstd), self._p(self._input_rows),
                                             self._p(env.reset_buf), self._p(self.actions), self._p(self.inject_normal),
                                             self._stream), "dyros_ppo_act")
         env.core.step(self.actions)  # VecTask.step: 3 launches, reads `actions` in place
@@ -457,7 +485,7 @@ class PPOTrainer:
                 self._cast_obs(False)
                 last_v = self.packed.mu_value(self.packed.forward(self.x_step))[1].contiguous()
             else:
-                _, last_v = self.net.forward(self.env.obs_buf)
+                _, last_v = self.net.forward(self._input_rows)
                 last_v = last_v.float().contiguous()
         native.check(self.lib.dyros_ppo_gae(C.byref(self.pb), self._p(last_v), self._p(self.env.reset_buf), self._stream), "dyros_ppo_gae")
 
@@ -495,7 +523,8 @@ class PPOTrainer:
         if single:
             pk.unpack_grads(self.norm2 if clip > 0 else None)   # (the norm reduction rides along)
         elif self.peers is not None:  # optimizer.synchronize() (AG:161-173) over peer memory: publish, wait, sum in rank order
-            native.check(self.lib.dyros_ppo_unpack_grads_peers(C.byref(pk.desc), C.byref(self.peers.desc), self._stream), "unpack_peers")
+            native.check(self.lib.dyros_ppo_unpack_grads_peers_ac(C.byref(pk.desc), pk.critic_inputs, C.byref(self.peers.desc),
+                                                                  self._stream), "unpack_peers")
             if c.grad_sync == "peer2":
                 native.check(self.lib.dyros_ppo_reduce_scatter_peers(C.byref(self.peers.desc), self._p(n.grad), n.n, n.n_actor,
                                                                      self._stream), "reduce_scatter_peers")
@@ -509,18 +538,18 @@ class PPOTrainer:
             pk.unpack_grads(None)
             dist.all_reduce(n.grad)
             norm_done = False
-        native.check(self.lib.dyros_ppo_adam_packed(C.byref(pk.desc), self._p(n.flat), self._p(n.grad), self._p(n.exp_avg),
-                                                    self._p(n.exp_avg_sq), 1.0 / self.world, clip, int(norm_done), self._p(self.norm2),
-                                                    self._p(self.lr), self._p(self.opt_step), 0.9, 0.999, 1e-8, c.learning_rate,
-                                                    c.learning_rate_min, c.max_epochs if c.lr_schedule == "linear" else 0,
-                                                    self._stream), "dyros_ppo_adam_packed")
+        native.check(self.lib.dyros_ppo_adam_packed_ac(C.byref(pk.desc), pk.critic_inputs, self._p(n.flat), self._p(n.grad), self._p(n.exp_avg),
+                                                       self._p(n.exp_avg_sq), 1.0 / self.world, clip, int(norm_done), self._p(self.norm2),
+                                                       self._p(self.lr), self._p(self.opt_step), 0.9, 0.999, 1e-8, c.learning_rate,
+                                                       c.learning_rate_min, c.max_epochs if c.lr_schedule == "linear" else 0,
+                                                       self._stream), "dyros_ppo_adam_packed")
 
     def _minibatch(self, i: int):
         if self.packed is not None:
             return self._minibatch_packed(i)
         c, mb = self.cfg, self.cfg.minibatch_size
         r0 = i * mb
-        obs = self.buf["obs"].view(self.N * self.H, c.num_obs)[r0:r0 + mb]
+        obs = self.buf["obs"].view(self.N * self.H, self.W)[r0:r0 + mb]
         mu, v = self.net.forward(obs)
         mu32, v32 = mu.float().contiguous(), v.float().contiguous()
         native.check(self.lib.dyros_ppo_loss_grad(C.byref(self.pb), r0, mb, self._p(mu32), self._p(v32), self._p(self.net.logstd),

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from .. import terrain as terrain_gen
-from ..core import NOBS, CoreConfig, DyrosCore, HeightField, TerrainCurriculum
+from ..core import NOBS, NPRIV, CoreConfig, DyrosCore, HeightField, TerrainCurriculum
 from ..native import DyrosError
 from .spaces import Box
 
@@ -65,10 +65,37 @@ def height_scan_points(cfg: Dict[str, Any]) -> Optional[np.ndarray]:
     return None if tr is None else terrain_gen.height_points(terrain_gen.TerrainConfig.from_dict(tr))
 
 
+def critic_states(cfg: Dict[str, Any]) -> Optional[bool]:
+    """cfg["env"]["criticStates"] (ours, not a key of the reference's yaml; DESIGN.md section 4, "Critic states"):
+    None = off (absent or False); otherwise whether the heights of a height scan go into the observation row as well
+    (True: `{"heights_in_obs": True}`; False: `True`, the heights go into the state row only)."""
+    v = cfg["env"].get("criticStates", False)
+    if v is False or v is None:
+        return None
+    if v is True:
+        return False
+    if isinstance(v, dict) and set(v) <= {"heights_in_obs"} and isinstance(v.get("heights_in_obs", False), bool):
+        hio = bool(v.get("heights_in_obs", False))
+        if hio and height_scan_points(cfg) is None:
+            raise ValueError('cfg["env"]["criticStates"]: heights_in_obs needs a height scan (terrain measure_heights)')
+        return hio
+    raise ValueError(f'cfg["env"]["criticStates"]: False, True or {{"heights_in_obs": bool}} (got {v!r})')
+
+
 def num_observations(cfg: Dict[str, Any]) -> int:
-    """Columns of an observation row: the reference's 487 (T:36-44), plus P heights with measure_heights."""
+    """Columns of an observation row: the reference's 487 (T:36-44), plus P heights with measure_heights (unless
+    critic states take the heights alone)."""
     p = height_scan_points(cfg)
-    return NOBS + (0 if p is None else len(p))
+    cs = critic_states(cfg)
+    return NOBS + (0 if p is None or cs is False else len(p))
+
+
+def num_states(cfg: Dict[str, Any]) -> int:
+    """Columns of a critic state row: 487 + P + 31 with criticStates, else cfg["env"]["numStates"] (default 0)."""
+    if critic_states(cfg) is None:
+        return cfg["env"].get("numStates", 0)
+    p = height_scan_points(cfg)
+    return NOBS + (0 if p is None else len(p)) + NPRIV
 
 
 def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generator] = None) -> CoreConfig:
@@ -108,6 +135,9 @@ def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generato
         else:
             _terrain_config(c, tcfg, int(env["numEnvs"]), generator)
         c.height_scan = terrain_gen.height_points(tcfg)  # (any ground, the plane too)
+    cs = critic_states(cfg)
+    if cs is not None:
+        c.critic_states, c.critic_heights_in_obs = True, cs
     ap = task.get("randomization_params", {}).get("actor_params", {}).get("humanoid", {})
     dp = ap.get("dof_properties", {})
     if "damping" in dp:
@@ -155,6 +185,13 @@ class DyrosDynamicWalk:
         if (self.num_single_step_obs, self.num_action, self.num_obs_his, self.num_obs_skip) != (37, 13, 10, 2):
             raise ValueError("the fused observation kernel is specialised to 37/13/10/2 (DyrosDynamicWalk.yaml:15-20)")
         env["numObservations"] = num_observations(cfg)  # + the measured heights (legged_gym's measure_heights)
+        self.critic_states = critic_states(cfg) is not None  # kernel-written privileged rows in states_buf
+        if self.critic_states:
+            ns = num_states(cfg)
+            if "numStates" in env and env["numStates"] != ns:
+                raise ValueError(f'cfg["env"]["numStates"] = {env["numStates"]}, but criticStates makes the state rows {ns} '
+                                 "wide (487 + the heights of a height scan + 31 privileged columns)")
+            env["numStates"] = ns
         # VT:50-97 (Env.__init__)
         dev = sim_device.split(":")
         if dev[0].lower() not in ("cuda", "gpu"):
@@ -187,6 +224,7 @@ class DyrosDynamicWalk:
         self.max_episode_length = self.max_episode_length_s / (self.dt * self.skipframe)  # T:35
         self.core = DyrosCore(self.num_environments, self.device, self.core_cfg, seed=seed, rank=rank)
         assert self.core.obs_width == self.num_observations
+        assert self.core.states_width == (self.num_states if self.critic_states else 0)
         self.num_height_points = self.core.num_height_points
         self._bind_buffers()
         self._initial_randoms()
@@ -226,7 +264,8 @@ class DyrosDynamicWalk:
         t, s, N = self.core.task_t, self.core.sim_t, self.num_envs
         self.obs_buf, self.rew_buf, self.reset_buf = t["obs_buf"], t["rew_buf"], t["reset_buf"]
         self.timeout_buf, self.progress_buf, self.randomize_buf = t["timeout_buf"], t["progress_buf"], t["randomize_buf"]
-        self.states_buf = torch.zeros(N, self.num_states, device=self.device)
+        # critic states (criticStates): the kernels' privileged rows (DESIGN.md section 4); else VecTask's zero buffer
+        self.states_buf = t["states_buf"] if self.critic_states else torch.zeros(N, self.num_states, device=self.device)
         self.root_states = s["root_states"]
         self.dof_state = s["dof_state"]
         self.dof_pos = s["dof_state"].view(N, 33, 2)[..., 0]
@@ -298,6 +337,8 @@ class DyrosDynamicWalk:
         if self.terrain_level_mean is not None:  # legged_gym's episode log; written by the step's kernels
             self.extras.setdefault("episode", {})["terrain_level"] = self.terrain_level_mean
         self.obs_dict["obs"] = self._obs_out()
+        if self.critic_states:  # VT:340-341 (num_states > 0)
+            self.obs_dict["states"] = self.get_state()
         return self.obs_dict, self.rew_buf.to(self.rl_device), self.reset_buf.to(self.rl_device), self.extras
 
     def _obs_out(self) -> torch.Tensor:
@@ -321,6 +362,9 @@ class DyrosDynamicWalk:
         rollout whose actions do not wait for the newest observation runs at max(kernels, PCIe) instead of their sum.
         `self.obs_buf` is not updated by these steps (the observation kernel writes the ticket's block directly); rew_buf,
         reset_buf and the state tensors are. The only host wait is for the slot of step k-async_depth to be free again."""
+        if self.critic_states:
+            raise RuntimeError("step_async: the host pipeline carries obs / rew / reset / time_outs only, no critic states; "
+                               "use step() on an env with criticStates")
         if self._pipe is None:
             self._pipe = _HostPipe(self)
         return self._pipe.submit(actions)
@@ -387,6 +431,8 @@ class DyrosDynamicWalk:
     def reset(self) -> Dict[str, torch.Tensor]:
         """VT:362-374: returns the observation buffer as is (zeros before the first step); resets nothing."""
         self.obs_dict["obs"] = self._obs_out()
+        if self.critic_states:
+            self.obs_dict["states"] = self.get_state()
         return self.obs_dict
 
     def reset_done(self):
@@ -395,6 +441,8 @@ class DyrosDynamicWalk:
         if len(done) > 0:
             self.reset_idx(done)
         self.obs_dict["obs"] = self._obs_out()
+        if self.critic_states:
+            self.obs_dict["states"] = self.get_state()
         return self.obs_dict, done
 
     def reset_idx(self, env_ids: torch.Tensor):

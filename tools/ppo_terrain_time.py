@@ -2,7 +2,11 @@
 (terrain measure_heights, 674 columns), in one process, alternating, split into rollout and update; then the library
 kernels of the first-layer GEMMs of both widths under torch.profiler (source of profiles/ppo_terrain.md).
 
-    python tools/ppo_terrain_time.py [--epochs 10] [--trace-dir DIR]"""
+With --critic-states the two trainers are instead the 674-wide perceptive one (actor and critic read the observation row
+with the heights) and the blind-actor one (criticStates: a 487-input actor, a 705-input critic on the state rows,
+PPOConfig(num_states=705)), both on curriculum terrain.
+
+    python tools/ppo_terrain_time.py [--epochs 10] [--trace-dir DIR] [--critic-states]"""
 import argparse, subprocess, sys, time
 import torch
 sys.path.insert(0, '.')
@@ -12,6 +16,7 @@ from isaacgymdyros_b200.ppo import PPOConfig, PPOTrainer
 ap = argparse.ArgumentParser()
 ap.add_argument("--epochs", type=int, default=10, help="timed epochs per env, alternating")
 ap.add_argument("--trace-dir", default=None, help="also write the torch.profiler traces there")
+ap.add_argument("--critic-states", action="store_true", help="perceptive (674) against blind actor + critic states (487 / 705)")
 args = ap.parse_args()
 N = 4096
 smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
@@ -19,15 +24,18 @@ smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm"
 print(f"GPU: {torch.cuda.get_device_name(0)}; nvidia-smi name, power limit, max SM clock: {smi[0] if smi else 'n/a'}")
 
 
-def make(terrain: bool):
+def make(terrain: bool, states: bool = False):
     cfg = default_cfg(N)
     if terrain:
         cfg["env"]["terrain"] = {"curriculum": True, "measure_heights": True, "seed": 2}
+    if states:
+        cfg["env"]["criticStates"] = True
     env = DyrosDynamicWalk(cfg, "cuda:0", use_cuda_graph=False)
-    return env, PPOTrainer(env, PPOConfig(num_obs=env.num_obs))
+    return env, PPOTrainer(env, PPOConfig(num_obs=env.num_obs, num_states=env.num_states if states else 0))
 
 
-runs = {"plane": make(False), "terrain": make(True)}
+runs = ({"perceptive": make(True), "blind+states": make(True, True)} if args.critic_states
+        else {"plane": make(False), "terrain": make(True)})
 
 
 # ---- the first-layer GEMMs (eager: the same shapes and library calls the CUDA graphs capture)

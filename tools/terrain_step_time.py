@@ -13,7 +13,13 @@ clock64() breakdown of the physics kernel (CTA 0, per role; marks of physics_rol
 and the card's name and power limit, and times the fused post-physics launch alone (dyros_task_post_step, L2 flushed
 before each) for the curriculum and scan rows: the kernel the scan runs in. TOCABI's roles: 0 torso + left arm, 1 head + right arm + base, 2 left leg,
 3 right leg (only the two legs have contact phases).
-Usage: python tools/terrain_step_time.py [--envs 4096] [--steps 60] [--rounds 5] [--out FILE.json]"""
+With --critic-states it times instead, alternating, with the L2 flushed before each timed step and back to back, the
+fused step and the post-physics launch alone of
+  plane         the plane, no critic states
+  plane+states  the plane with criticStates (state rows of 518 floats)
+  scan          the curriculum with the height scan in the observation (rows of 674 floats), no critic states
+  scan+states   the same with criticStates: a blind 487-float observation and state rows of 705 floats
+Usage: python tools/terrain_step_time.py [--envs 4096] [--steps 60] [--rounds 5] [--critic-states] [--out FILE.json]"""
 import argparse
 import json
 import os
@@ -66,10 +72,13 @@ def main():
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=100)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--critic-states", action="store_true", help="time the critic state rows (DESIGN.md section 4)")
     a = ap.parse_args()
     N = a.envs
     name, power = card()
     print(f"card: {name}; power limit, max SM clock: {power}", flush=True)
+    if a.critic_states:
+        return critic_states(a, name, power)
     kinds = ["plane", "flat", "rough", "stairs", "generated", "curriculum", "scan"]
     envs = {}
     for k in kinds:
@@ -142,6 +151,65 @@ def main():
     if a.out:
         with open(a.out, "w") as f:
             json.dump(res, f, indent=1)
+
+
+def critic_states(a, name, power):
+    N = a.envs
+    kinds = {"plane": (None, None), "plane+states": (None, True),
+             "scan": ({"curriculum": True, "measure_heights": True}, None),
+             "scan+states": ({"curriculum": True, "measure_heights": True}, True)}
+    envs = {}
+    for k, (terrain, cs) in kinds.items():
+        cfg = default_cfg(N)
+        if terrain is not None:
+            cfg["env"]["terrain"] = dict(terrain)
+        if cs is not None:
+            cfg["env"]["criticStates"] = cs
+        envs[k] = DyrosDynamicWalk(cfg, "cuda:0")
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda:0")
+    g = torch.Generator(device="cuda:0")
+    g.manual_seed(1)
+    acts = [torch.rand(N, 13, device="cuda:0", generator=g) * 2 - 1 for _ in range(8)]
+    for k in kinds:
+        for i in range(a.warmup):
+            envs[k].step(acts[i % 8])
+    torch.cuda.synchronize()
+    modes = [(what, flushed) for what in ("step", "post") for flushed in (True, False)]
+    times = {(k, w, f): [] for k in kinds for w, f in modes}
+    for r in range(a.rounds):
+        for w, f in modes:
+            for k in kinds:  # alternating
+                env = envs[k]
+                ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.steps)]
+                for i in range(a.steps):
+                    if f:
+                        env.core.flush_l2(flush, i)
+                    ev[i][0].record()
+                    env.step(acts[i % 8]) if w == "step" else env.core.post_step()
+                    ev[i][1].record()
+                torch.cuda.synchronize()
+                times[(k, w, f)] += [e0.elapsed_time(e1) for e0, e1 in ev]
+    res = {"card": name, "power_limit_and_max_sm_clock": power, "envs": N, "steps_per_round": a.steps, "rounds": a.rounds,
+           "widths": {k: {"obs": envs[k].num_obs, "states": envs[k].num_states} for k in kinds}, "ms": {}}
+    print(f"\n| env | obs | states | L2 | step ms (median, p10-p90) | post-physics launch ms (median, p10-p90) |")
+    print("|---|---|---|---|---|---|")
+    for f in (True, False):
+        for k in kinds:
+            row = {}
+            for w in ("step", "post"):
+                t = np.array(times[(k, w, f)])
+                row[w] = {"median": round(float(np.median(t)), 4), "p10": round(float(np.percentile(t, 10)), 4),
+                          "p90": round(float(np.percentile(t, 90)), 4)}
+            res["ms"][f"{k}, {'flushed' if f else 'back to back'}"] = row
+            fmt = lambda d: f"{d['median']:.4f} ({d['p10']:.4f}-{d['p90']:.4f})"
+            print(f"| {k} | {envs[k].num_obs} | {envs[k].num_states} | {'flushed' if f else 'back to back'} | "
+                  f"{fmt(row['step'])} | {fmt(row['post'])} |")
+    print(json.dumps(res, indent=1))
+    if a.out:
+        with open(a.out, "w") as fh:
+            json.dump(res, fh, indent=1)
+    for e in envs.values():
+        e.close()
 
 
 if __name__ == "__main__":
