@@ -1,4 +1,5 @@
-// K2/K3/K4: the bodies of DyrosDynamicWalk's per-step methods as sm_100a kernels (one warp per env).
+// K2/K3/K4: the bodies of DyrosDynamicWalk's per-step methods as sm_100a kernels (one warp per env; the pre-physics
+// stages one CTA per slab of envs, task_stages.cuh).
 //
 // Compiled with -fmad=false: the reference computes every float32 op separately (CPU torch / op-by-op
 // ATen), and parity is judged at 1e-5 relative with bit-exact masks, so no FMA contraction here.
@@ -46,64 +47,145 @@ __device__ __forceinline__ float quat2euler_comp(const float* q, int which) {
   return atan2f(ay, ax);
 }
 
+// ------------------------------------------------------------------ the task's arithmetic, value in and value out:
+// shared by the staged kernels and k_post_fused, which load the inputs and store the results each in its own pattern
+
+// T:532-541, VT:325, T:544-545: the counters after one step. `a12`: the env's last action
+struct EpiCounters {
+  float epi, time;
+  int timeout;
+  long long progress, randomize;
+};
+__device__ __forceinline__ EpiCounters epilogue_counters(const TaskParams& P, float epi_len, float time, float a12,
+                                                        long long progress, long long randomize) {
+  EpiCounters o;
+  o.epi = epi_len + 1.0f;
+  const float t = time + P.dt_policy;
+  o.time = t + P.time_gain * a12;
+  o.timeout = ((float)progress >= P.max_len_m1) ? 1 : 0;
+  o.progress = progress + 1;
+  o.randomize = randomize + 1;
+  return o;
+}
+
+// T:590 / T:937: body b is not a foot and has |F| > 1
+__device__ __forceinline__ bool body_hit(const TaskParams& P, int b, float f0, float f1, float f2) {
+  return b != P.lfoot && b != P.rfoot && sqrtf(f0 * f0 + f1 * f1 + f2 * f2) > 1.0f;
+}
+// T:581-596: the reset flag from the orientation error, the step count after the epilogue and the body-hit test
+__device__ __forceinline__ int termination(const TaskParams& P, float qe, long long progress, bool col) {
+  int reset = (fabsf(qe) > 0.5f) ? 1 : 0;
+  if ((float)progress >= P.max_len_m1) reset = 1;
+  if (col) reset = 1;
+  return reset;
+}
+
+// T:802-947 from the joint sums of T:387-428 and the env's scalars: the 14 terms into r, the total returned
+struct RewardIn {
+  float qe, s_qpos, s_qvel, s_qacc, s_tq, s_tqd;
+  float lf0, lf1, lf2, rf0, rf1, rf2;        // foot contact forces
+  float lfp0, lfp1, lfp2, rfp0, rfp1, rfp2;  // the same, one step before
+  float tvx, tvy, rootvx, rootvy, mass, ft0, ft1;
+  int midx;
+  bool col;
+};
+__device__ __forceinline__ float reward_terms(const TaskParams& P, const RewardIn& in, float (&r)[14]) {
+  r[0] = 0.3f * expf(-13.2f * fabsf(in.qe));                                            // T:835
+  float n;
+  n = sqrtf(in.s_qpos); r[1] = 0.35f * expf(-2.0f * (n * n));                           // T:837
+  n = sqrtf(in.s_qvel); r[2] = 0.05f * expf(-0.01f * (n * n));                          // T:839
+  const float dl0 = in.lf0 - in.lfp0, dl1 = in.lf1 - in.lfp1, dl2 = in.lf2 - in.lfp2;
+  const float dr0 = in.rf0 - in.rfp0, dr1 = in.rf1 - in.rfp1, dr2 = in.rf2 - in.rfp2;
+  r[9] = 0.2f * expf(-0.01f * (sqrtf(dl0 * dl0 + dl1 * dl1 + dl2 * dl2) + sqrtf(dr0 * dr0 + dr1 * dr1 + dr2 * dr2)));  // T:858
+  r[4] = 0.05f * expf(-0.01f * sqrtf(in.s_tq));                                         // T:861
+  r[5] = 0.6f * expf(-0.01f * sqrtf(in.s_tqd));                                         // T:863
+  n = sqrtf(in.s_qacc); r[7] = 0.05f * expf(-20.0f * (n * n));                          // T:865
+  const float vx = in.tvx - in.rootvx, vy = in.tvy - in.rootvy;
+  n = sqrtf(vx * vx + vy * vy); r[6] = 0.3f * expf(-3.0f * (n * n));                    // T:867
+  const bool lc = in.lf2 > 1.0f, rc = in.rf2 > 1.0f;                                    // T:869-870
+  const int idx = in.midx;
+  const bool DSP = ((3300 <= idx) && (idx < 3600)) || (idx < 300) || ((1500 <= idx) && (idx < 2100));
+  const bool RSSP = (300 <= idx) && (idx < 1500);
+  const bool LSSP = (2100 <= idx) && (idx < 3300);
+  const bool sync = (DSP && rc && lc) || (RSSP && rc && !lc) || (LSSP && !rc && lc);  // T:882-889
+  r[8] = sync ? 0.2f : 0.0f;
+  r[10] = 0.0f;                                                                         // T:893
+  const float thr = (float)(1.4 * 9.81) * in.mass;                                      // T:895
+  const bool thres = (in.lf2 > thr) || (in.rf2 > thr);
+  r[11] = thres ? -0.2f : 0.0f;                                                         // T:898
+  const float cl = fmaxf(in.lf2 - thr, 0.0f), cr = fmaxf(in.rf2 - thr, 0.0f);
+  const float pen = 0.1f * expf(-0.007f * (sqrtf(cl * cl) + sqrtf(cr * cr)));           // T:900-901
+  r[3] = thres ? pen : 0.1f;                                                            // T:902
+  const float dthr = (float)(0.2 * 9.81) * in.mass / 1.0f;                              // T:904
+  const bool tdiff = (fabsf(in.lf2 - in.lfp2) > dthr) || (fabsf(in.rf2 - in.rfp2) > dthr);
+  r[12] = tdiff ? -0.05f : 0.0f;                                                        // T:907
+  const float ws = in.mass / 104.48f;                                                   // T:917
+  r[13] = 0.1f * expf(-0.001f * fabsf(in.lf2 + ws * in.ft0)) + 0.1f * expf(-0.001f * fabsf(in.rf2 + ws * in.ft1));  // T:918-919
+  float total = r[0] + r[1] + r[2] + r[3] + r[4] + r[5] + r[6] + r[7] + r[8] + r[9] + r[10] + r[11] + r[12] + r[13];  // T:932-934
+  if (in.col) total = P.death_cost;                                                     // T:942
+  if (fabsf(in.qe) > 0.5f) total = P.death_cost;                                        // T:943
+  return total;
+}
+
+// T:762-763: the angle of the mocap phase at the env's time
+__device__ __forceinline__ float obs_phase_angle(const TaskParams& P, float time, int init_idx) {
+  const float time2idx = py_fmodf(time, P.period) / P.cycle_dt;
+  const float phase = py_fmodf((float)init_idx + time2idx, (float)P.mocap_data_num) / (float)P.mocap_data_num;
+  return (float)(2 * 3.14159265358979) * phase;
+}
+// Component i of the observation frame (T:753-774), normalised (T:776-777), from the sources of that component:
+// i < 3 the root's orientation `quat` and its bias `quatb`; i < 15 the noisy joint angle `qn` and its bias `qb`; i < 27
+// the noisy joint velocity `qv`; 27, 28 the phase angle; i < 31 the target velocity `tv`; i >= 31 the root's velocity
+// `rootv` and the uniform draw `u` of its noise
+__device__ __forceinline__ float obs_component(int i, const float* quat, float quatb, float qn, float qb, float qv,
+                                               float ang, float tv, float rootv, float u, float mean, float var) {
+  float v;
+  if (i < 3) v = quat2euler_comp(quat, i) + quatb;
+  else if (i < 15) v = qn + qb;
+  else if (i < 27) v = qv;
+  else if (i == 27) v = sinf(ang);                                                      // T:764
+  else if (i == 28) v = cosf(ang);                                                      // T:765
+  else if (i < 31) v = tv;
+  else v = rootv + (u * 0.05f - 0.025f);                                                // T:766,774
+  return (v - mean) / sqrtf(var + 1e-8f * 1.0f);
+}
+// T:789-796: ring slots of the history gather, `head` the slot of this step's entry: observation frame i of the gather
+// is at position NSKIP (i + 1) - 1, action i at NSKIP (i + 1)
+__device__ __forceinline__ int obs_hist_slot(int head, int i) { return (head + 1 + NSKIP * (i + 1) - 1) % NSLOT; }
+__device__ __forceinline__ int act_hist_slot(int head, int i) { return (head + 1 + NSKIP * (i + 1)) % NSLOT; }
+
+// ------------------------------------------------------------------ stages (device functions, one warp per env)
+// T:532-541, VT:325, T:544-545
+__device__ void stage_epilogue(const TK& k, int e, int lane) {
+  if (lane != 0) return;
+  const EpiCounters c = epilogue_counters(k.p, k.b.epi_len[e], k.b.time[e], k.b.actions[(size_t)e * NA + NA - 1],
+                                          k.b.progress_buf[e], k.b.randomize_buf[e]);
+  k.b.epi_len[e] = c.epi;
+  k.b.time[e] = c.time;
+  k.b.timeout_buf[e] = c.timeout;
+  k.b.progress_buf[e] = c.progress;
+  k.b.randomize_buf[e] = c.randomize;
+}
+
+// T:590 / T:937 over the bodies of the env (warp-uniform)
 __device__ __forceinline__ bool collision_true(const TK& k, int e, int lane) {
-  // T:590 / T:937: any non-foot body with |F| > 1
   bool hit = false;
   for (int b = lane; b < NB; b += kWarp) {
-    if (b == k.p.lfoot || b == k.p.rfoot) continue;
     const float* f = k.s.net_contact_force + ((size_t)e * NB + b) * 3;
-    float n = sqrtf(f[0] * f[0] + f[1] * f[1] + f[2] * f[2]);
-    hit |= n > 1.0f;
+    hit |= body_hit(k.p, b, f[0], f[1], f[2]);
   }
   return __any_sync(kFull, hit);
 }
 
-// ------------------------------------------------------------------ stages (device functions, one warp per env)
-struct WarpSyncT {
-  __device__ __forceinline__ void operator()() const { __syncwarp(); }
-};
-
-// T:532-541, VT:325, T:544-545
-__device__ void stage_epilogue(const TK& k, int e, int lane) {
-  if (lane != 0) return;
-  k.b.epi_len[e] = k.b.epi_len[e] + 1.0f;
-  float t = k.b.time[e] + k.p.dt_policy;
-  t = t + k.p.time_gain * k.b.actions[(size_t)e * NA + NA - 1];
-  k.b.time[e] = t;
-  long long pr = k.b.progress_buf[e];
-  k.b.timeout_buf[e] = ((float)pr >= k.p.max_len_m1) ? 1 : 0;
-  k.b.progress_buf[e] = pr + 1;
-  k.b.randomize_buf[e] = k.b.randomize_buf[e] + 1;
-}
-
-// T:581-596 ; returns the reset flag (warp-uniform)
-// `shared` (fused kernel): hands the collision flag and the orientation error on to the reward stage, which needs
-// the same two quantities of the same (pre-reset) state.
-struct TermShared {
-  bool col;
-  float qe;
-};
-__device__ int stage_check_termination(const TK& k, int e, int lane, TermShared* shared = nullptr) {
-  float qe = quat_err_identity(k.s.root_states + (size_t)e * 13 + 3);
-  int reset = (fabsf(qe) > 0.5f) ? 1 : 0;
-  if ((float)k.b.progress_buf[e] >= k.p.max_len_m1) reset = 1;
+// T:581-596
+__device__ void stage_check_termination(const TK& k, int e, int lane) {
   const bool col = collision_true(k, e, lane);
-  if (shared) {
-    shared->col = col;
-    shared->qe = qe;
-  }
-  if (col) reset = 1;
-  if (lane == 0) k.b.reset_buf[e] = reset;
-  return reset;
+  if (lane == 0)
+    k.b.reset_buf[e] = termination(k.p, quat_err_identity(k.s.root_states + (size_t)e * 13 + 3), k.b.progress_buf[e], col);
 }
 
-// T:387-428 + T:802-947, in two parts: the warp-wide reductions over the joints, and the scalar terms (one thread per
-// env: the fused kernel runs them for all envs of a CTA side by side in one warp instead of on lane 0 of each).
-struct RewardSums {
-  float s_qpos, s_qvel, s_qacc, s_tq, s_tqd, qe;
-  bool col;
-};
-__device__ RewardSums reward_sums(const TK& k, int e, int lane, const TermShared* shared = nullptr) {
+// T:387-428 + T:802-947: the warp-wide sums over the joints, then the scalar terms on lane 0
+__device__ void stage_compute_reward(const TK& k, int e, int lane) {
   const float* root = k.s.root_states + (size_t)e * 13;
   const float* ds = k.s.dof_state + (size_t)e * ND * 2;
   float s_qpos = 0.f, s_qvel = 0.f, s_qacc = 0.f, s_tq = 0.f, s_tqd = 0.f;
@@ -122,70 +204,25 @@ __device__ RewardSums reward_sums(const TK& k, int e, int lane, const TermShared
     s_tq = t * t;
     s_tqd = td * td;
   }
-  RewardSums o;
-  o.s_qpos = warp_sum(s_qpos);
-  o.s_qvel = warp_sum(s_qvel);
-  o.s_qacc = warp_sum(s_qacc);
-  o.s_tq = warp_sum(s_tq);
-  o.s_tqd = warp_sum(s_tqd);
-  o.col = shared ? shared->col : collision_true(k, e, lane);
-  o.qe = shared ? shared->qe : quat_err_identity(root + 3);
-  return o;
-}
-__device__ void reward_scalar(const TK& k, int e, const RewardSums& in) {
-  const float* root = k.s.root_states + (size_t)e * 13;
-  const float s_qpos = in.s_qpos, s_qvel = in.s_qvel, s_qacc = in.s_qacc, s_tq = in.s_tq, s_tqd = in.s_tqd, qe = in.qe;
-  const bool col = in.col;
-  float r[14];
-  r[0] = 0.3f * expf(-13.2f * fabsf(qe));                                          // T:835
-  float n;
-  n = sqrtf(s_qpos); r[1] = 0.35f * expf(-2.0f * (n * n));                         // T:837
-  n = sqrtf(s_qvel); r[2] = 0.05f * expf(-0.01f * (n * n));                        // T:839
+  s_qpos = warp_sum(s_qpos); s_qvel = warp_sum(s_qvel); s_qacc = warp_sum(s_qacc); s_tq = warp_sum(s_tq); s_tqd = warp_sum(s_tqd);
+  const bool col = collision_true(k, e, lane);
+  if (lane != 0) return;
   const float* F = k.s.net_contact_force + (size_t)e * NB * 3;
   const float* Fp = k.b.contact_forces_pre + (size_t)e * NB * 3;
   const float *lf = F + k.p.lfoot * 3, *rf = F + k.p.rfoot * 3, *lfp = Fp + k.p.lfoot * 3, *rfp = Fp + k.p.rfoot * 3;
-  float dl0 = lf[0] - lfp[0], dl1 = lf[1] - lfp[1], dl2 = lf[2] - lfp[2];
-  float dr0 = rf[0] - rfp[0], dr1 = rf[1] - rfp[1], dr2 = rf[2] - rfp[2];
-  r[9] = 0.2f * expf(-0.01f * (sqrtf(dl0 * dl0 + dl1 * dl1 + dl2 * dl2) + sqrtf(dr0 * dr0 + dr1 * dr1 + dr2 * dr2)));  // T:858
-  r[4] = 0.05f * expf(-0.01f * sqrtf(s_tq));                                        // T:861
-  r[5] = 0.6f * expf(-0.01f * sqrtf(s_tqd));                                        // T:863
-  n = sqrtf(s_qacc); r[7] = 0.05f * expf(-20.0f * (n * n));                        // T:865
-  float vx = k.b.target_vel[(size_t)e * 2] - root[7], vy = k.b.target_vel[(size_t)e * 2 + 1] - root[8];
-  n = sqrtf(vx * vx + vy * vy); r[6] = 0.3f * expf(-3.0f * (n * n));               // T:867
-  bool lc = lf[2] > 1.0f, rc = rf[2] > 1.0f;                                       // T:869-870
-  int idx = k.b.mocap_data_idx[e];
-  bool DSP = ((3300 <= idx) && (idx < 3600)) || (idx < 300) || ((1500 <= idx) && (idx < 2100));
-  bool RSSP = (300 <= idx) && (idx < 1500);
-  bool LSSP = (2100 <= idx) && (idx < 3300);
-  bool sync = (DSP && rc && lc) || (RSSP && rc && !lc) || (LSSP && !rc && lc);     // T:882-889
-  r[8] = sync ? 0.2f : 0.0f;
-  k.b.contact_reward_sum[e] = k.b.contact_reward_sum[e] + r[8];                    // T:891
-  r[10] = 0.0f;                                                                    // T:893
-  float m = k.b.total_mass[e];
-  float thr = (float)(1.4 * 9.81) * m;                                             // T:895
-  bool thres = (lf[2] > thr) || (rf[2] > thr);
-  r[11] = thres ? -0.2f : 0.0f;                                                    // T:898
-  float cl = fmaxf(lf[2] - thr, 0.0f), cr = fmaxf(rf[2] - thr, 0.0f);
-  float pen = 0.1f * expf(-0.007f * (sqrtf(cl * cl) + sqrtf(cr * cr)));            // T:900-901
-  r[3] = thres ? pen : 0.1f;                                                       // T:902
-  float dthr = (float)(0.2 * 9.81) * m / 1.0f;                                     // T:904
-  bool tdiff = (fabsf(lf[2] - lfp[2]) > dthr) || (fabsf(rf[2] - rfp[2]) > dthr);
-  r[12] = tdiff ? -0.05f : 0.0f;                                                   // T:907
-  float ws = m / 104.48f;                                                          // T:917
+  const float* tv = k.b.target_vel + (size_t)e * 2;
   const float* ft = k.b.target_data_force + (size_t)e * 2;
-  r[13] = 0.1f * expf(-0.001f * fabsf(lf[2] + ws * ft[0])) + 0.1f * expf(-0.001f * fabsf(rf[2] + ws * ft[1]));  // T:918-919
-  float total = r[0] + r[1] + r[2] + r[3] + r[4] + r[5] + r[6] + r[7] + r[8] + r[9] + r[10] + r[11] + r[12] + r[13];  // T:932-934
-  if (col) total = k.p.death_cost;                                                 // T:942
-  if (fabsf(qe) > 0.5f) total = k.p.death_cost;                                    // T:943
+  float r[14];
+  const float total = reward_terms(k.p, RewardIn{quat_err_identity(root + 3), s_qpos, s_qvel, s_qacc, s_tq, s_tqd,
+                                                 lf[0], lf[1], lf[2], rf[0], rf[1], rf[2], lfp[0], lfp[1], lfp[2],
+                                                 rfp[0], rfp[1], rfp[2], tv[0], tv[1], root[7], root[8],
+                                                 k.b.total_mass[e], ft[0], ft[1], k.b.mocap_data_idx[e], col}, r);
+  k.b.contact_reward_sum[e] = k.b.contact_reward_sum[e] + r[8];                        // T:891
   k.b.rew_buf[e] = total;
   float* st = k.b.stacked_rewards + (size_t)e * 15;
 #pragma unroll
-  for (int i = 0; i < 14; ++i) st[i] = col ? k.p.death_cost : r[i];                // T:945
-  st[14] = (*k.b.perturb_start) ? 1.0f : 0.0f;                                     // T:415
-}
-__device__ void stage_compute_reward(const TK& k, int e, int lane, const TermShared* shared = nullptr) {
-  RewardSums sums = reward_sums(k, e, lane, shared);
-  if (lane == 0) reward_scalar(k, e, sums);
+  for (int i = 0; i < 14; ++i) st[i] = col ? k.p.death_cost : r[i];                    // T:945
+  st[14] = (*k.b.perturb_start) ? 1.0f : 0.0f;                                         // T:415
 }
 
 // Terrain curriculum of one resetting env (legged_gym _update_terrain_curriculum; DESIGN.md section 4, "Curriculum"),
@@ -400,32 +437,20 @@ template <class Scan, class St>
 __device__ void stage_compute_observations(const TK& k, int e, int lane, const Scan& sc, const St& st) {
   const TaskParams& P = k.p;
   const float* root = k.s.root_states + (size_t)e * 13;
-  float time = k.b.time[e];
-  float time2idx = py_fmodf(time, P.period) / P.cycle_dt;                                           // T:762
-  float phase = py_fmodf((float)k.b.init_mocap_data_idx[e] + time2idx, (float)P.mocap_data_num) / (float)P.mocap_data_num;  // T:763
-  float ang = (float)(2 * 3.14159265358979) * phase;
+  const float ang = obs_phase_angle(P, k.b.time[e], k.b.init_mocap_data_idx[e]);
   int head = (k.b.obs_hist_head[e] + 1) % NSLOT;
   bool start = k.b.epi_len[e] == 0.0f;                                                              // T:785
   float* hist = k.b.obs_history + (size_t)e * NSLOT * NOBS1;
+#pragma unroll 1
   for (int i = lane; i < NOBS1; i += kWarp) {
-    float v;
-    if (i < 3) v = quat2euler_comp(root + 3, i) + k.b.quat_bias[(size_t)e * 3 + i];                 // T:753-757
-    else if (i < 15) v = k.b.qpos_noise[(size_t)e * ND + (i - 3)] + k.b.qpos_bias[(size_t)e * 12 + (i - 3)];
-    else if (i < 27) v = k.b.qvel_noise[(size_t)e * ND + (i - 15)];
-    else if (i == 27) v = sinf(ang);                                                                // T:764
-    else if (i == 28) v = cosf(ang);                                                                // T:765
-    else if (i < 31) v = k.b.target_vel[(size_t)e * 2 + (i - 29)];
-    else {
-      int c = i - 31;
-      float u;
-      if (k.j.vel_u) u = k.j.vel_u[(size_t)e * 6 + c];
-      else {
-        uint4 r = draw4(P.seed, *P.step_counter, e, kSiteVelNoise, c);
-        u = u01(r.x);
-      }
-      v = root[7 + c] + (u * 0.05f - 0.025f);                                                       // T:766,774
-    }
-    float nv = (v - k.b.obs_mean[i]) / sqrtf(k.b.obs_var[i] + 1e-8f * 1.0f);                        // T:776-777
+    // (the sources of component i; the indices of the others are clamped into their rows)
+    const int q = min(max(i - 3, 0), 11), c = max(i - 31, 0);
+    float u = 0.f;
+    if (i >= 31) u = k.j.vel_u ? k.j.vel_u[(size_t)e * 6 + c] : u01(draw4(P.seed, *P.step_counter, e, kSiteVelNoise, c).x);
+    const float nv = obs_component(i, root + 3, k.b.quat_bias[(size_t)e * 3 + min(i, 2)], k.b.qpos_noise[(size_t)e * ND + q],
+                                   k.b.qpos_bias[(size_t)e * 12 + q], k.b.qvel_noise[(size_t)e * ND + min(max(i - 15, 0), 11)],
+                                   ang, k.b.target_vel[(size_t)e * 2 + min(max(i - 29, 0), 1)], root[7 + c], u,
+                                   k.b.obs_mean[i], k.b.obs_var[i]);
     if (start) {
       for (int sl = 0; sl < NSLOT; ++sl) hist[sl * NOBS1 + i] = nv;                                 // T:786-787
     } else {
@@ -452,13 +477,11 @@ __device__ void stage_compute_observations(const TK& k, int e, int lane, const S
     float v;
     if (o < NOBS1 * NHIS) {                                                                         // T:789-791
       int i = o / NOBS1, j = o - i * NOBS1;
-      int pos = NSKIP * (i + 1) - 1;
-      v = hist[((head + 1 + pos) % NSLOT) * NOBS1 + j];
+      v = hist[obs_hist_slot(head, i) * NOBS1 + j];
     } else {                                                                                        // T:793-796
       int q = o - NOBS1 * NHIS;
       int i = q / NA, j = q - i * NA;
-      int pos = NSKIP * (i + 1);
-      v = ah[((ahead + 1 + pos) % NSLOT) * NA + j];
+      v = ah[act_hist_slot(ahead, i) * NA + j];
     }
     vals[it] = v;
   }
@@ -516,19 +539,28 @@ __device__ void stage_late_update(const TK& k, int e, int lane) {
   int e = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);          \
   if (e >= k.p.N) return;
 
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_prologue(TK k, const float* __restrict__ actions) {
+// the pre-physics stages: one CTA of kSlabThreads threads per slab of kSlabMaxEnvs consecutive envs
+#define ENV_SLAB()                                   \
+  const int e0 = blockIdx.x * kSlabMaxEnvs, nenv = min(kSlabMaxEnvs, k.p.N - e0);
+
+__global__ void __launch_bounds__(kSlabThreads) k_prologue(TK k, const float* __restrict__ actions) {
+  __shared__ float pro[kSlabMaxEnvs][8];
   pdl_launch_dependents();
-  ENV_LANE();
-  stage_prologue(k, actions, e, lane);
+  ENV_SLAB();
+  stage_prologue_slab(k, actions, e0, nenv, threadIdx.x, kSlabThreads, pro, [] { __syncthreads(); }, [] {});
 }
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_substep_torque(TK k) {
-  ENV_LANE();
-  WarpSyncT sync;
-  stage_substep_torque<32>(k, e, lane, sync);
+__global__ void __launch_bounds__(kSlabThreads) k_substep_torque(TK k) {
+  ENV_SLAB();
+  const TorqueSlabArgs a = torque_args(k);
+  stage_substep_torque_cta(a, e0, nenv, threadIdx.x, kSlabThreads, [](int, int, float) {},
+                           [&](int le, int d, int which) { return k.s.dof_state[((size_t)(e0 + le) * ND + d) * 2 + which]; });
+  __syncthreads();
+  stage_simul_len_update(a, e0, nenv, threadIdx.x, kSlabThreads);
 }
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) k_sensor_noise(TK k, int substep) {
-  ENV_LANE();
-  stage_sensor_noise<32>(k, substep, e, lane);
+__global__ void __launch_bounds__(kSlabThreads) k_sensor_noise(TK k, int substep) {
+  ENV_SLAB();
+  stage_sensor_noise_cta(noise_args(k), substep, e0, nenv, threadIdx.x, kSlabThreads,
+                         [&](int le, int d) { return k.s.dof_state[((size_t)(e0 + le) * ND + d) * 2]; });
 }
 __global__ void __launch_bounds__(kWarpsPerBlock * 32) k_epilogue(TK k) {
   ENV_LANE();
@@ -598,8 +630,8 @@ __device__ __forceinline__ ObsIn load_obs_in(const TK& k, int e, int lane) {
 // post_physics_step in one launch: epilogue, termination, reward, reset, observations, late update (T:532-563), one
 // warp per env, written as ONE stage: every input of every stage is requested up front (one round of independent,
 // coalesced loads; a second one for the history rows, whose addresses depend on the ring heads), all arithmetic then
-// runs on registers, and the results go out at the end. The arithmetic is that of the staged kernels above, operation
-// for operation (tests/test_env_step_gpu.py pins the two bit for bit). The scalar reward terms are computed by every
+// runs on registers, and the results go out at the end. The arithmetic is the staged kernels' own: both call the helpers
+// at the top of this file (tests/test_env_step_gpu.py pins the two bit for bit). The scalar reward terms are computed by every
 // lane of the warp from broadcast values: no regrouping through shared memory, no CTA barrier.
 // Reward/termination read the pre-reset state, observations the post-reset state (SURVEY A3). Of contact_forces_pre only
 // the two foot rows are maintained here: they are all the reward reads (T:858-859, T:904-907).
@@ -608,8 +640,16 @@ __device__ __forceinline__ ObsIn load_obs_in(const TK& k, int e, int lane) {
 // bits. epi_len_log holds whole numbers (exact at 2^-20), contact_reward_mean lies in [0, 1].
 __device__ __forceinline__ long long gate_term0(float epi_len_log) { return __double2ll_rn((double)epi_len_log * 1048576.0); }
 __device__ __forceinline__ long long gate_term1(float contact_reward_mean) { return __double2ll_rn((double)contact_reward_mean * 1099511627776.0); }
-__device__ __forceinline__ bool gate_open(const TaskParams& P, long long s0, long long s1) {  // T:489
-  return (float)((double)s0 / 1048576.0 / P.N) > P.gate_len && (float)((double)s1 / 1099511627776.0 / P.N) > 0.165f;
+// The last CTA's part of the end-of-step tail (k_post_fused, k_crossenv): the gate decision from the two sums (T:489-490,
+// sticky) and the mean terrain level; the sums are cleared for the next step
+__device__ __forceinline__ void end_step_tail(const TK& k, bool gate, bool lmean) {
+  const TaskParams& P = k.p;
+  if (gate) {
+    const long long s0 = (long long)atomicExch(P.tail + 0, 0ull), s1 = (long long)atomicExch(P.tail + 1, 0ull);
+    if ((float)((double)s0 / 1048576.0 / P.N) > P.gate_len && (float)((double)s1 / 1099511627776.0 / P.N) > 0.165f)
+      *k.b.perturb_start = 1;
+  }
+  if (lmean) *k.c.level_mean = (float)((double)(long long)atomicExch(P.tail + 3, 0ull) / P.N);
 }
 
 // 4 warps per CTA, 7 CTAs per SM: 4096 envs (1024 CTAs) are resident on 148 SMs in ONE wave at <= 73 registers per thread
@@ -666,31 +706,23 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     float hA[NHIS - 1], hB[NHIS - 1], hC[NHIS - 1];
 #pragma unroll
     for (int i = 0; i < NHIS - 1; ++i) {
-      const float* row = hist + ((head + 1 + NSKIP * (i + 1) - 1) % NSLOT) * NOBS1;   // T:789-791, position 2(i+1)-1
+      const float* row = hist + obs_hist_slot(head, i) * NOBS1;
       hA[i] = row[lane];
       hB[i] = row[iB];
-      hC[i] = ah[((ahead + 1 + NSKIP * (i + 1)) % NSLOT) * NA + l13];                 // T:793-796, position 2(i+1)
+      hC[i] = ah[act_hist_slot(ahead, i) * NA + l13];
     }
     // ================================================================ epilogue (T:532-541, VT:325, T:544-545)
-    const float a12 = __shfl_sync(kFull, act, NA - 1);
-    float epi = epi0 + 1.0f;
-    float t = in.time + P.dt_policy;
-    t = t + P.time_gain * a12;
-    const int timeout = ((float)pr >= P.max_len_m1) ? 1 : 0;
-    const long long progress = pr + 1;
-    long long randomize = rnd + 1;
+    const EpiCounters ec = epilogue_counters(P, epi0, in.time, __shfl_sync(kFull, act, NA - 1), pr, rnd);
+    float epi = ec.epi, t = ec.time;
     // ================================================================ termination (T:581-596)
     float quat[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) quat[i] = __shfl_sync(kFull, in.root, 3 + i);
     const float qe = quat_err_identity(quat);
-    int reset = (fabsf(qe) > 0.5f) ? 1 : 0;
-    if ((float)progress >= P.max_len_m1) reset = 1;
-    bool hit = false;                                               // T:590 / T:937: any non-foot body with |F| > 1
-    if (lane != P.lfoot && lane != P.rfoot) hit |= sqrtf(fA0 * fA0 + fA1 * fA1 + fA2 * fA2) > 1.0f;
-    if (lane + 32 < NB && lane + 32 != P.lfoot && lane + 32 != P.rfoot) hit |= sqrtf(fB0 * fB0 + fB1 * fB1 + fB2 * fB2) > 1.0f;
+    bool hit = body_hit(P, lane, fA0, fA1, fA2);
+    if (lane + 32 < NB) hit |= body_hit(P, lane + 32, fB0, fB1, fB2);
     const bool col = __any_sync(kFull, hit);
-    if (col) reset = 1;
+    const int reset = termination(P, qe, ec.progress, col);
     // ================================================================ reward (T:387-428, T:802-947)
     float s_qpos, s_qvel, s_qacc, s_tq = 0.f, s_tqd = 0.f;
     {
@@ -707,48 +739,14 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
       }
     }
     s_qpos = warp_sum(s_qpos); s_qvel = warp_sum(s_qvel); s_qacc = warp_sum(s_qacc); s_tq = warp_sum(s_tq); s_tqd = warp_sum(s_tqd);
-    // the scalar terms, by every lane from broadcast values (reward_scalar, operation for operation)
+    // the scalar terms, by every lane from broadcast values
     const float lf0 = __shfl_sync(kFull, fA0, P.lfoot), lf1 = __shfl_sync(kFull, fA1, P.lfoot), lf2 = __shfl_sync(kFull, fA2, P.lfoot);
     const float rf0 = __shfl_sync(kFull, fA0, P.rfoot), rf1 = __shfl_sync(kFull, fA1, P.rfoot), rf2 = __shfl_sync(kFull, fA2, P.rfoot);
     const float rootvx = __shfl_sync(kFull, in.root, 7), rootvy = __shfl_sync(kFull, in.root, 8);
     const float tvx = __shfl_sync(kFull, in.tv, 0), tvy = __shfl_sync(kFull, in.tv, 1);
     float r[14];
-    float total;
-    {
-      r[0] = 0.3f * expf(-13.2f * fabsf(qe));                                         // T:835
-      float n;
-      n = sqrtf(s_qpos); r[1] = 0.35f * expf(-2.0f * (n * n));                        // T:837
-      n = sqrtf(s_qvel); r[2] = 0.05f * expf(-0.01f * (n * n));                       // T:839
-      const float dl0 = lf0 - lfp0, dl1 = lf1 - lfp1, dl2 = lf2 - lfp2;
-      const float dr0 = rf0 - rfp0, dr1 = rf1 - rfp1, dr2 = rf2 - rfp2;
-      r[9] = 0.2f * expf(-0.01f * (sqrtf(dl0 * dl0 + dl1 * dl1 + dl2 * dl2) + sqrtf(dr0 * dr0 + dr1 * dr1 + dr2 * dr2)));  // T:858
-      r[4] = 0.05f * expf(-0.01f * sqrtf(s_tq));                                       // T:861
-      r[5] = 0.6f * expf(-0.01f * sqrtf(s_tqd));                                       // T:863
-      n = sqrtf(s_qacc); r[7] = 0.05f * expf(-20.0f * (n * n));                       // T:865
-      const float vx = tvx - rootvx, vy = tvy - rootvy;
-      n = sqrtf(vx * vx + vy * vy); r[6] = 0.3f * expf(-3.0f * (n * n));              // T:867
-      const bool lc = lf2 > 1.0f, rc = rf2 > 1.0f;                                    // T:869-870
-      const bool DSP = ((3300 <= midx) && (midx < 3600)) || (midx < 300) || ((1500 <= midx) && (midx < 2100));
-      const bool RSSP = (300 <= midx) && (midx < 1500);
-      const bool LSSP = (2100 <= midx) && (midx < 3300);
-      const bool sync = (DSP && rc && lc) || (RSSP && rc && !lc) || (LSSP && !rc && lc);  // T:882-889
-      r[8] = sync ? 0.2f : 0.0f;
-      r[10] = 0.0f;                                                                   // T:893
-      const float thr = (float)(1.4 * 9.81) * mass;                                   // T:895
-      const bool thres = (lf2 > thr) || (rf2 > thr);
-      r[11] = thres ? -0.2f : 0.0f;                                                   // T:898
-      const float cl = fmaxf(lf2 - thr, 0.0f), cr = fmaxf(rf2 - thr, 0.0f);
-      const float pen = 0.1f * expf(-0.007f * (sqrtf(cl * cl) + sqrtf(cr * cr)));     // T:900-901
-      r[3] = thres ? pen : 0.1f;                                                      // T:902
-      const float dthr = (float)(0.2 * 9.81) * mass / 1.0f;                           // T:904
-      const bool tdiff = (fabsf(lf2 - lfp2) > dthr) || (fabsf(rf2 - rfp2) > dthr);
-      r[12] = tdiff ? -0.05f : 0.0f;                                                  // T:907
-      const float ws = mass / 104.48f;                                                // T:917
-      r[13] = 0.1f * expf(-0.001f * fabsf(lf2 + ws * ft0)) + 0.1f * expf(-0.001f * fabsf(rf2 + ws * ft1));  // T:918-919
-      total = r[0] + r[1] + r[2] + r[3] + r[4] + r[5] + r[6] + r[7] + r[8] + r[9] + r[10] + r[11] + r[12] + r[13];  // T:932-934
-      if (col) total = P.death_cost;                                                  // T:942
-      if (fabsf(qe) > 0.5f) total = P.death_cost;                                     // T:943
-    }
+    const float total = reward_terms(P, RewardIn{qe, s_qpos, s_qvel, s_qacc, s_tq, s_tqd, lf0, lf1, lf2, rf0, rf1, rf2, lfp0, lfp1,
+                                                 lfp2, rfp0, rfp1, rfp2, tvx, tvy, rootvx, rootvy, mass, ft0, ft1, midx, col}, r);
     {
       float stv = col ? P.death_cost : 0.f;                                           // T:945
 #pragma unroll
@@ -760,7 +758,7 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     // ================================================================ stores of the scalar state; reset (T:598-669)
     if (lane == 0) {
       k.b.rew_buf[e] = total;
-      k.b.timeout_buf[e] = timeout;
+      k.b.timeout_buf[e] = ec.timeout;
       k.b.reset_buf[e] = reset;
       k.b.contact_reward_sum[e] = crs + r[8];                                          // T:891
     }
@@ -770,8 +768,8 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
       if (lane == 0) {
         k.b.epi_len[e] = epi;
         k.b.time[e] = t;
-        k.b.progress_buf[e] = progress;
-        k.b.randomize_buf[e] = randomize;
+        k.b.progress_buf[e] = ec.progress;
+        k.b.randomize_buf[e] = ec.randomize;
       }
       __syncwarp();
       stage_reset_env(k, e, lane);
@@ -786,8 +784,8 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     } else if (lane == 0) {
       k.b.epi_len[e] = epi;
       k.b.time[e] = t;
-      k.b.progress_buf[e] = progress;
-      k.b.randomize_buf[e] = randomize;
+      k.b.progress_buf[e] = ec.progress;
+      k.b.randomize_buf[e] = ec.randomize;
     }
     // ================================================================ cross-env pass of the fused step
     // (what k_crossenv does for the staged one, minus the id list): gate sums by 64-bit integer atomics, one pair per
@@ -823,20 +821,14 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
         if (gate || lmean) __threadfence();  // the sums before the ticket
         if (atomicAdd(P.tail + 2, 1ull) == gridDim.x - 1) {  // every CTA has published its sums and taken its epoch copy
           __threadfence();
-          if (gate) {
-            const long long s0 = (long long)atomicExch(P.tail + 0, 0ull), s1 = (long long)atomicExch(P.tail + 1, 0ull);
-            if (gate_open(P, s0, s1)) *k.b.perturb_start = 1;  // T:489-490 (sticky)
-          }
-          if (lmean) *k.c.level_mean = (float)((double)(long long)atomicExch(P.tail + 3, 0ull) / P.N);
+          end_step_tail(k, gate, lmean);
           P.tail[2] = 0;
           *P.step_counter = epoch + 1;
         }
       }
     }
     // ================================================================ observations (T:750-796)
-    const float time2idx = py_fmodf(t, P.period) / P.cycle_dt;                         // T:762
-    const float phase = py_fmodf((float)in.init_idx + time2idx, (float)P.mocap_data_num) / (float)P.mocap_data_num;  // T:763
-    const float ang = (float)(2 * 3.14159265358979) * phase;
+    const float ang = obs_phase_angle(P, t, in.init_idx);
     const bool start = epi == 0.0f;                                                    // T:785
 #pragma unroll
     for (int i = 0; i < 4; ++i) quat[i] = __shfl_sync(kFull, in.root, 3 + i);
@@ -848,20 +840,11 @@ __global__ void __launch_bounds__(kPostWarps * 32, 7) k_post_fused(TK k, int tai
     const float rootv_for_B = __shfl_sync(kFull, in.root, (8 + lane) & 31);  // components 32..36 = root[8..12] (lanes 0..4)
     // T:766: one draw per velocity component c = 0..5, held by lane 31 (component 31) and lanes 0..4 (32..36)
     const int cdraw = lane == 31 ? 0 : (lane < 5 ? lane + 1 : 0);
-    float vnoise = velu;
-    if (!k.j.vel_u) vnoise = u01(draw4(P.seed, epoch, e, kSiteVelNoise, cdraw).x);
-    vnoise = vnoise * 0.05f - 0.025f;
-    float vA, vB = 0.f;
-    if (iA < 3) vA = quat2euler_comp(quat, iA) + in.quatb;                             // T:753-757 (quat_bias[lane], lane < 3)
-    else if (iA < 15) vA = qn_for_A + qb_for_A;
-    else if (iA < 27) vA = qv_for_A;
-    else if (iA == 27) vA = sinf(ang);                                                 // T:764
-    else if (iA == 28) vA = cosf(ang);                                                 // T:765
-    else if (iA < 31) vA = iA == 29 ? tv0n : tv1n;
-    else vA = rootv_for_A + vnoise;                                                    // T:766,774 (component 31)
-    if (lane < NOBS1 - 32) vB = rootv_for_B + vnoise;                                  // components 32..36
-    const float nvA = (vA - meanA) / sqrtf(varA + 1e-8f * 1.0f);                       // T:776-777
-    const float nvB = (vB - meanB) / sqrtf(varB + 1e-8f * 1.0f);
+    float u = velu;
+    if (!k.j.vel_u) u = u01(draw4(P.seed, epoch, e, kSiteVelNoise, cdraw).x);
+    const float nvA = obs_component(iA, quat, in.quatb, qn_for_A, qb_for_A, qv_for_A, ang, iA == 29 ? tv0n : tv1n, rootv_for_A,
+                                    u, meanA, varA);
+    const float nvB = obs_component(iB, quat, in.quatb, qn_for_A, qb_for_A, qv_for_A, ang, tv1n, rootv_for_B, u, meanB, varB);
     {
       float* hw = k.b.obs_history + E * NSLOT * NOBS1;
       if (start) {
@@ -1040,11 +1023,7 @@ __global__ void __launch_bounds__(kScanTile) k_crossenv(TK k, int do_compact, in
       for (int t = 0; t < ntiles; ++t) status[t] = 0u;
       ticket[0] = 0u;
       ticket[1] = 0u;
-      if (gate) {
-        const long long a = (long long)atomicExch(k.p.tail + 0, 0ull), b = (long long)atomicExch(k.p.tail + 1, 0ull);
-        if (gate_open(k.p, a, b)) *k.b.perturb_start = 1;  // T:489-490 (sticky)
-      }
-      if (lmean) *k.c.level_mean = (float)((double)(long long)atomicExch(k.p.tail + 3, 0ull) / N);
+      end_step_tail(k, gate, lmean);
       if (do_bump) *k.p.step_counter = *k.p.step_counter + 1;
     }
   }
@@ -1088,8 +1067,18 @@ __global__ void __launch_bounds__(256) k_pack_results(TK k, float* __restrict__ 
 }
 
 // ------------------------------------------------------------------ launchers
-static inline HeightScan make_scan(const Task* t) {
-  HeightScan sc;
+// Calls f(Scan(), St()) with the types of the observation kernels' instantiation for a task with (`scan`) or without a
+// height scan and with (`states`) or without critic states; kernel_arg(t, sc) / kernel_arg(t, st) are their arguments
+template <class F>
+static int with_scan_states(bool scan, bool states, F f) {
+  if (!scan && !states) return f(NoScan(), NoStates());
+  if (!states) return f(HeightScan(), NoStates());
+  if (!scan) return f(NoScan(), CriticStates());
+  return f(HeightScan(), CriticStates());
+}
+static inline NoScan kernel_arg(const Task*, NoScan sc) { return sc; }
+static inline NoStates kernel_arg(const Task*, NoStates st) { return st; }
+static inline HeightScan kernel_arg(const Task* t, HeightScan sc) {
   sc.points = reinterpret_cast<const float2*>(t->scan.points);
   sc.P = t->scan.num_points;
   sc.base_offset = t->scan.base_offset;
@@ -1099,8 +1088,7 @@ static inline HeightScan make_scan(const Task* t) {
   sc.f = t->sim->field;
   return sc;
 }
-static inline CriticStates make_states(const Task* t) {
-  CriticStates st;
+static inline CriticStates kernel_arg(const Task* t, CriticStates st) {
   st.states = t->crit.states;
   st.S = t->states_width();
   st.priv = NOBS + t->scan.num_points;
@@ -1111,58 +1099,49 @@ static inline CriticStates make_states(const Task* t) {
   return st;
 }
 static inline int env_grid(int N) { return (N + kWarpsPerBlock - 1) / kWarpsPerBlock; }
-#define LAUNCH_ENV(kern, ...)                                                    \
-  kern<<<env_grid(t->p.N), kWarpsPerBlock * 32, 0, s>>>(make_tk(t), ##__VA_ARGS__); \
-  DY_LAUNCH_CHECK();                                                             \
+#define LAUNCH(kern, grid, block, ...)                          \
+  kern<<<grid, block, 0, s>>>(make_tk(t), ##__VA_ARGS__);        \
+  DY_LAUNCH_CHECK();                                            \
   return 0;
+#define LAUNCH_ENV(kern, ...) LAUNCH(kern, env_grid(t->p.N), kWarpsPerBlock * 32, ##__VA_ARGS__)
+#define LAUNCH_SLAB(kern, ...) LAUNCH(kern, (t->p.N + kSlabMaxEnvs - 1) / kSlabMaxEnvs, kSlabThreads, ##__VA_ARGS__)
 
-int launch_prologue(Task* t, const float* actions, cudaStream_t s) { LAUNCH_ENV(k_prologue, actions) }
-int launch_substep_torque(Task* t, cudaStream_t s) { LAUNCH_ENV(k_substep_torque) }
-int launch_sensor_noise(Task* t, int substep, cudaStream_t s) { LAUNCH_ENV(k_sensor_noise, substep) }
+int launch_prologue(Task* t, const float* actions, cudaStream_t s) { LAUNCH_SLAB(k_prologue, actions) }
+int launch_substep_torque(Task* t, cudaStream_t s) { LAUNCH_SLAB(k_substep_torque) }
+int launch_sensor_noise(Task* t, int substep, cudaStream_t s) { LAUNCH_SLAB(k_sensor_noise, substep) }
 int launch_epilogue(Task* t, cudaStream_t s) { LAUNCH_ENV(k_epilogue) }
 int launch_check_termination(Task* t, cudaStream_t s) { LAUNCH_ENV(k_check_termination) }
 int launch_compute_reward(Task* t, cudaStream_t s) { LAUNCH_ENV(k_compute_reward) }
 int launch_compute_observations(Task* t, cudaStream_t s) {
-  if (t->crit.states) {
-    if (t->scan.num_points) { LAUNCH_ENV((k_compute_observations<HeightScan, CriticStates>), make_scan(t), make_states(t)) }
-    LAUNCH_ENV((k_compute_observations<NoScan, CriticStates>), NoScan(), make_states(t))
-  }
-  if (t->scan.num_points) { LAUNCH_ENV((k_compute_observations<HeightScan, NoStates>), make_scan(t), NoStates()) }
-  LAUNCH_ENV((k_compute_observations<NoScan, NoStates>), NoScan(), NoStates())
+  return with_scan_states(t->scan.num_points, t->crit.states, [&](auto sc, auto st) {
+    LAUNCH_ENV((k_compute_observations<decltype(sc), decltype(st)>), kernel_arg(t, sc), kernel_arg(t, st))
+  });
 }
 int launch_late_update(Task* t, cudaStream_t s) { LAUNCH_ENV(k_late_update) }
 int configure_task_kernels() {
   DY_CUDA(prefer_max_smem_carveout(k_prologue)); DY_CUDA(prefer_max_smem_carveout(k_substep_torque));
   DY_CUDA(prefer_max_smem_carveout(k_sensor_noise)); DY_CUDA(prefer_max_smem_carveout(k_epilogue));
   DY_CUDA(prefer_max_smem_carveout(k_check_termination)); DY_CUDA(prefer_max_smem_carveout(k_compute_reward));
-  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<NoScan, NoStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<HeightScan, NoStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<NoScan, CriticStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_compute_observations<HeightScan, CriticStates>)));
   DY_CUDA(prefer_max_smem_carveout(k_late_update));
   DY_CUDA(prefer_max_smem_carveout(k_reset_idx)); DY_CUDA(prefer_max_smem_carveout(k_pack_results));
-  DY_CUDA(prefer_max_smem_carveout((k_post_fused<NoScan, NoStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_post_fused<HeightScan, NoStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_post_fused<NoScan, CriticStates>)));
-  DY_CUDA(prefer_max_smem_carveout((k_post_fused<HeightScan, CriticStates>)));
   DY_CUDA(prefer_max_smem_carveout(k_crossenv));
+  for (int v = 0; v < 4; ++v) {
+    const int err = with_scan_states(v & 1, v & 2, [](auto sc, auto st) {
+      DY_CUDA(prefer_max_smem_carveout(k_compute_observations<decltype(sc), decltype(st)>));
+      DY_CUDA(prefer_max_smem_carveout(k_post_fused<decltype(sc), decltype(st)>));
+      return 0;
+    });
+    if (err) return err;
+  }
   return 0;
 }
 int launch_post_fused(Task* t, cudaStream_t s, bool pdl, bool tail) {
   const dim3 grid((t->p.N + kPostWarps - 1) / kPostWarps), block(kPostWarps * 32);
-  if (t->crit.states) {
-    if (t->scan.num_points)
-      DY_CUDA(launch_kernel(k_post_fused<HeightScan, CriticStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t),
-                            make_states(t)));
-    else
-      DY_CUDA(launch_kernel(k_post_fused<NoScan, CriticStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan(),
-                            make_states(t)));
-  } else if (t->scan.num_points) {
-    DY_CUDA(launch_kernel(k_post_fused<HeightScan, NoStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, make_scan(t), NoStates()));
-  } else {
-    DY_CUDA(launch_kernel(k_post_fused<NoScan, NoStates>, grid, block, 0, s, pdl, make_tk(t), (int)tail, NoScan(), NoStates()));
-  }
-  return 0;
+  return with_scan_states(t->scan.num_points, t->crit.states, [&](auto sc, auto st) {
+    DY_CUDA(launch_kernel(k_post_fused<decltype(sc), decltype(st)>, grid, block, 0, s, pdl, make_tk(t), (int)tail,
+                          kernel_arg(t, sc), kernel_arg(t, st)));
+    return 0;
+  });
 }
 int launch_reset_idx(Task* t, const int64_t* env_ids, int count, cudaStream_t s) {
   if (count == 0) return 0;

@@ -1,7 +1,8 @@
-// Stages of the per-step task logic that run both as their own kernels (task_kernels.cu, one warp per env) and
-// inside the fused physics kernel (physics_kernels.cu, DYROS_LANES lanes per env). Arithmetic uses the
-// non-contracting intrinsics so that both compilation units (with and without -fmad) produce the same bits,
-// and the same float32 results as the reference's op-by-op torch code.
+// The pre-physics stages of the per-step task logic (prologue, sub-step torques, sensor noise), written for a slab of
+// consecutive envs and kSlabThreads cooperating threads. They run as the staged kernels of task_kernels.cu (one CTA per
+// slab) and on the I/O warps of the fused physics kernels (physics_cta.cuh). Arithmetic uses the non-contracting
+// intrinsics so that both compilation units (with and without -fmad) produce the same bits, and the same float32
+// results as the reference's op-by-op torch code.
 #pragma once
 #include "internal.h"
 
@@ -96,55 +97,22 @@ __device__ __forceinline__ void stage_push_schedule(const TK& k, int e) {
   k.b.push_force[(size_t)e * 3 + 2] = 0.f;
 }
 
-// VT:307 clamp + T:449-468 + push schedule T:489-502, T:438-447; one warp per env. Runs as its own kernel
-// (k_prologue) and on the I/O warps of the fused physics kernel.
-__device__ __forceinline__ void stage_prologue(const TK& k, const float* __restrict__ actions_in, int e, int lane) {
-  const TaskParams& P = k.p;
-  float time = k.b.time[e];
-  int init = k.b.init_mocap_data_idx[e];
-  float local_time = py_fmodf(time, P.period);                                                          // T:450
-  float lt_init = py_fmodf(__fadd_rn(local_time, __fmul_rn((float)init, P.cycle_dt)), P.period);        // T:451
-  int idx = (int)(((long long)init + (long long)__fdiv_rn(local_time, P.cycle_dt)) % P.mocap_data_num);  // T:452
-  if (lane == 0) k.b.mocap_data_idx[e] = idx;
-  const float* r0 = k.b.mocap_data + (size_t)idx * 36;
-  const float* r1 = r0 + 36;
-  const CubicKnots kn = cubic_knots(r0[0], r1[0]);
-  for (int c = lane; c < 35; c += 32) {                                           // T:458-461
-    float v = cubic0(lt_init, kn, r0[1 + c], r1[1 + c]);
-    if (c < ND) k.b.target_data_qpos[(size_t)e * ND + c] = v;
-    else k.b.target_data_force[(size_t)e * 2 + (c - ND)] = v;
-  }
-  if (lane < NA) {
-    float a = actions_in[(size_t)e * NA + lane];
-    a = (a < -1.0f) ? -1.0f : ((a > 1.0f) ? 1.0f : a);                            // VT:307 (NaN passes through)
-    if (lane == NA - 1) a = __fmul_rn((a > 0.0f) ? 1.0f : 0.0f, a);               // T:464-465
-    k.b.actions[(size_t)e * NA + lane] = a;
-    int head = (k.b.act_hist_head[e] + 1) % NSLOT;                                // T:466 as a ring push
-    k.b.action_history[((size_t)e * NSLOT + head) * NA + lane] = a;
-    if (lane < 12)                                                                // T:468
-      k.b.action_torque[(size_t)e * 12 + lane] =
-          __fmul_rn(__fmul_rn(a, k.b.motor_constant_scale[(size_t)e * 12 + lane]), P.action_high[lane]);
-    __syncwarp(0x1fffu);
-    if (lane == 0) k.b.act_hist_head[e] = head;
-  }
-  if (lane == 0) stage_push_schedule(k, e);
-}
-
-// The same stage for a contiguous slab of envs [e0, e0 + nenv), thread `tid` of `nthreads` cooperating threads. The
-// warp-per-env form above is a serial chain of dependent loads per env; here the per-env scalars (phase time, mocap
-// row, knot times) are computed once by one thread per env and parked in `pro` (shared memory, 8 words per env), and
-// the (env, column) items of the cubic targets and of the action block then need one batch of independent loads each.
-// Same arithmetic, same bits. `group_sync` is a barrier of the cooperating threads; `after_env_phase` runs at the end,
-// after the push schedule (it stages the push).
+// Envs of a slab, and the thread count (virtual threads in the fused physics kernels) the slab stages are written for
 constexpr int kSlabMaxEnvs = 32;
+constexpr int kSlabThreads = 128;
+
+// VT:307 clamp + T:449-468 + push schedule T:489-502, T:438-447 for a contiguous slab of envs [e0, e0 + nenv), thread
+// `tid` of `nthreads` cooperating threads. The per-env scalars (phase time, mocap row, knot times) are computed once by
+// one thread per env and parked in `pro` (shared memory, 8 words per env), and the (env, column) items of the cubic
+// targets and of the action block then need one batch of independent loads each. `group_sync` is a barrier of the
+// cooperating threads; `after_env_phase` runs at the end, after the push schedule (it stages the push).
 template <class GroupSync, class AfterEnvPhase>
 __device__ __forceinline__ void stage_prologue_slab(const TK& k, const float* __restrict__ actions_in, int e0, int nenv, int tid,
                                                     int nthreads, float (*pro)[8], GroupSync group_sync,
                                                     AfterEnvPhase after_env_phase) {
   const TaskParams& P = k.p;
   const FastDiv d35(35), dNA(NA);
-  constexpr int THREADS = 128;
-  constexpr int IT_A = (kSlabMaxEnvs * NA + THREADS - 1) / THREADS;  // action items per thread
+  constexpr int IT_A = (kSlabMaxEnvs * NA + kSlabThreads - 1) / kSlabThreads;  // action items per thread
   // ---- first round trip: everything that depends on nothing is requested at once: the action block of this thread's
   //      items (VT:307, T:464-468) and, on the per-env threads, the phase time
   float act[IT_A], mcs[IT_A];
@@ -224,93 +192,9 @@ __device__ __forceinline__ void stage_prologue_slab(const TK& k, const float* __
   after_env_phase();
 }
 
-// T:505-520: upper-body PD, actuation-delay ring, the 33 torques of set_dof_actuation_force_tensor.
-// LANES lanes of one env cooperate; `lane` in [0, LANES). Ends with the lanes in sync.
-template <int LANES, class Sync>
-__device__ __forceinline__ void stage_substep_torque(const TK& k, int e, int lane, Sync& sync, bool live = true) {
-  const float* ds = k.s.dof_state + (size_t)e * ND * 2;
-  float* out = k.s.dof_actuation_force + (size_t)e * ND;
-  {  // T:506; loads of all iterations are issued before the first use (trip count is a compile-time constant)
-    constexpr int IT = (ND - 12 + LANES - 1) / LANES;
-    float pos[IT], vel[IT], tgt[IT], kp[IT], kv[IT];
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      int d = 12 + lane + it * LANES;
-      int dc = d < ND ? d : ND - 1;
-      pos[it] = ds[2 * dc];
-      vel[it] = ds[2 * dc + 1];
-      tgt[it] = k.b.target_data_qpos[(size_t)e * ND + dc];
-      // optional per-env gain scales (DR of the PD gains); a scale of 1 leaves the reference's product unchanged
-      kp[it] = k.b.pd_gain_scale ? __fmul_rn(k.p.kp[dc], k.b.pd_gain_scale[(size_t)e * 2]) : k.p.kp[dc];
-      kv[it] = k.b.pd_gain_scale ? __fmul_rn(k.p.kv[dc], k.b.pd_gain_scale[(size_t)e * 2 + 1]) : k.p.kv[dc];
-    }
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      int d = 12 + lane + it * LANES;
-      if (d < ND && live) out[d] = __fadd_rn(__fmul_rn(kp[it], __fsub_rn(tgt[it], pos[it])), __fmul_rn(kv[it], -vel[it]));
-    }
-  }
-  int sl = k.b.simul_len[e] + 1;                                                  // T:513-514
-  sl = sl > LOG_DEPTH ? LOG_DEPTH : (sl < 0 ? 0 : sl);
-  int dl = k.b.delay_idx[e];
-  for (int j = lane; j < 12; j += LANES) {
-    float* lg = k.b.action_log + (size_t)e * LOG_DEPTH * 12 + j;
-    float v[LOG_DEPTH];
-#pragma unroll
-    for (int i = 0; i < LOG_DEPTH - 1; ++i) v[i] = lg[(i + 1) * 12];              // T:511
-    v[LOG_DEPTH - 1] = k.b.action_torque[(size_t)e * 12 + j];                     // T:512
-#pragma unroll
-    for (int i = 0; i < LOG_DEPTH; ++i)
-      if (live) lg[i * 12] = v[i];
-    int pick = (sl > dl) ? dl : (LOG_DEPTH - sl);                                 // T:515-519
-    float r = v[0];
-#pragma unroll
-    for (int i = 1; i < LOG_DEPTH; ++i) r = (pick == i) ? v[i] : r;
-    if (live) out[j] = r;                                                         // T:520
-  }
-  sync();
-  if (lane == 0 && live) k.b.simul_len[e] = sl;
-}
-
-// T:528-530
-template <int LANES>
-__device__ __forceinline__ void stage_sensor_noise(const TK& k, int substep, int e, int lane, bool live = true) {
-  const float* ds = k.s.dof_state + (size_t)e * ND * 2;
-  constexpr int IT = (ND + LANES - 1) / LANES;
-  float pos[IT], pre[IT], nz[IT];
-  const bool inject = k.j.qpos_normal != nullptr;
-  const uint64_t epoch = inject ? 0 : *k.p.step_counter;
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {  // all loads first
-    int d = lane + it * LANES;
-    int dc = d < ND ? d : ND - 1;
-    pos[it] = ds[2 * dc];
-    pre[it] = k.b.qpos_pre[(size_t)e * ND + dc];
-    nz[it] = inject ? k.j.qpos_normal[((size_t)substep * k.p.N + e) * ND + dc] : 0.f;
-  }
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {
-    int d = lane + it * LANES;
-    if (d < ND && live) {
-      float n = nz[it];
-      if (!inject) {
-        uint4 r = draw4(k.p.seed, epoch, e, kSiteQposNoise, substep * 64 + (d >> 1));  // one draw per pair of DOFs
-        float2 nn = normal01_pair(r.x, r.y);
-        n = __fmul_rn((d & 1) ? nn.y : nn.x, k.p.noise_std);
-      }
-      n = (n < -0.00016f) ? -0.00016f : ((n > 0.00016f) ? 0.00016f : n);
-      float qn = __fadd_rn(pos[it], n);
-      size_t i = (size_t)e * ND + d;
-      k.b.qvel_noise[i] = __fdiv_rn(__fsub_rn(qn, pre[it]), k.p.dt);
-      k.b.qpos_noise[i] = qn;
-      k.b.qpos_pre[i] = qn;
-    }
-  }
-}
-
-// ---- CTA-cooperative variants for a contiguous slab of envs [e0, e0 + nenv): thread `tid` of `nthreads`, one
-//      element per thread and iteration, so every global access is coalesced; the loads of all iterations are issued
-//      before the first use (MAXE bounds the slab). Same arithmetic, same bits as the per-env variants.
+// ---- T:505-520 and T:528-530 for a contiguous slab of envs [e0, e0 + nenv): thread `tid` of `nthreads`, one element
+//      per thread and iteration, so every global access is coalesced; the loads of all iterations are issued before the
+//      first use (kSlabMaxEnvs bounds the slab).
 //      `tau_sink(le, d, v)` additionally receives every torque (the fused kernel feeds its scratch blocks with it).
 struct TorqueSlabArgs {  // the handful of pointers the torque stage touches (passed by value to a non-inlined function)
   const float* dof_state;
@@ -342,17 +226,19 @@ __device__ __forceinline__ NoiseSlabArgs noise_args(const TK& k) {
   return NoiseSlabArgs{k.j.qpos_normal, k.b.qpos_pre, k.b.qvel_noise, k.b.qpos_noise, k.p.step_counter, k.p.seed,
                        k.p.noise_std, k.p.dt, k.p.N};
 }
+// T:505-520: upper-body PD, actuation-delay ring, the 33 torques of set_dof_actuation_force_tensor.
 // `state_of(le, d, which)` supplies the joint angle (which = 0) / velocity (1): global dof_state or the fused kernel's
 // scratch blocks.
 // Split in two: the part below reads simul_len, stage_simul_len_update (after a barrier of the cooperating threads)
-// advances it. `tid` of `nthreads` = 128 VIRTUAL threads: a single warp runs it as four chunks of 32.
+// advances it. In the fused physics kernels `tid` of `nthreads` = kSlabThreads are virtual threads: a single warp runs them
+// as four chunks of 32.
 template <class Sink, class StateFn>
 __device__ __forceinline__ void stage_substep_torque_cta(const TorqueSlabArgs& k, int e0, int nenv, int tid, int nthreads,
                                                          Sink tau_sink, StateFn state_of) {
   constexpr int NU = ND - 12;
-  constexpr int THREADS = 128;
   const FastDiv dNU(NU), d12(12);
-  constexpr int IT_PD = (kSlabMaxEnvs * NU + THREADS - 1) / THREADS, IT_RG = (kSlabMaxEnvs * 12 + THREADS - 1) / THREADS;
+  constexpr int IT_PD = (kSlabMaxEnvs * NU + kSlabThreads - 1) / kSlabThreads;
+  constexpr int IT_RG = (kSlabMaxEnvs * 12 + kSlabThreads - 1) / kSlabThreads;
   {
     float pos[IT_PD], vel[IT_PD], tgt[IT_PD], kp[IT_PD], kv[IT_PD];
 #pragma unroll
@@ -423,13 +309,13 @@ __device__ __forceinline__ void stage_simul_len_update(const TorqueSlabArgs& k, 
   }
 }
 
-// T:528-530 for a slab; `pos_of(le, d)` supplies the fresh joint angle (from shared memory in the fused kernel).
+// T:528-530 for a slab; `pos_of(le, d)` supplies the fresh joint angle (global dof_state, or shared memory in the fused
+// kernel).
 // One thread handles a pair of DOFs (one Philox draw and one Box-Muller transform per pair).
 template <class PosFn>
 __device__ __forceinline__ void stage_sensor_noise_cta(const NoiseSlabArgs& k, int substep, int e0, int nenv, int tid, int nthreads, PosFn pos_of) {
-  constexpr int THREADS = 128;
   constexpr int NP = (ND + 1) / 2;
-  constexpr int IT = (kSlabMaxEnvs * NP + THREADS - 1) / THREADS;
+  constexpr int IT = (kSlabMaxEnvs * NP + kSlabThreads - 1) / kSlabThreads;
   const FastDiv dNP(NP);
   const bool inject = k.qpos_normal != nullptr;
   const uint64_t epoch = inject ? 0 : *k.step_counter;
