@@ -287,6 +287,28 @@ typedef struct {
 } DyrosHeightField;
 int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* field);
 
+/* gym.add_triangle_mesh (legged_gym terrain, mesh_type 'trimesh'): the ground of the sim becomes a triangle mesh. Vertex v
+ * sits at vertices[v] + origin (only a translation, as for the heightfield); triangle (a, b, c) has the face normal
+ * normalize((b - a) x (c - a)), its front the counter-clockwise side. A sphere of centre c and radius r (r = 0 for box
+ * corners and cylinder rim points) touches the nearest triangle (ties: the lowest index) with gap s - r, s the distance
+ * signed by the face normal; a point farther than the query margin M = contact_offset + the model's largest point radius
+ * + 0.1 m from every triangle has no ground (DESIGN.md section 4, "Triangle-mesh ground"). The library copies the mesh
+ * into its own device memory and builds a bucket grid over it; zero-area triangles are dropped. One ground per sim: a sim
+ * with a heightfield refuses a mesh and the other way round. The lanes program (physics_program 1) has no mesh ground.
+ * NULL switches back to the plane z = 0, frees the mesh and restores DyrosSimDesc.friction. While the mesh is set, the
+ * contact friction of envs without a contact_friction table is dynamic_friction. */
+typedef struct {
+  const float* vertices;      /* (num_vertices, 3) HOST array */
+  const uint32_t* triangles;  /* (num_triangles, 3) HOST array of vertex indices */
+  int64_t num_vertices, num_triangles;
+  float origin[3];            /* TriangleMeshParams.transform.p */
+  float dynamic_friction;     /* TriangleMeshParams.dynamic_friction, >= 0 */
+} DyrosTriangleMesh;
+int dyros_sim_set_triangle_mesh(DyrosSim* sim, const DyrosTriangleMesh* mesh);
+/* The sim's mesh ground: out[0] device bytes allocated, out[1] zero-area triangles dropped, out[2] triangles kept,
+ * out[3] buckets of the grid (all 0 without a mesh). */
+int dyros_sim_triangle_mesh_info(DyrosSim* sim, int64_t out[4]);
+
 /* --- task level (bodies of DyrosDynamicWalk methods) --- */
 int dyros_task_create(DyrosSim* sim, const DyrosTaskDesc* desc, const DyrosTaskBuffers* buf, DyrosTask** out);
 int dyros_task_destroy(DyrosTask* task);
@@ -326,6 +348,10 @@ typedef struct {
   float base_offset;         /* 0.5 */
   float scale;               /* obs_scales.height_measurements, 5.0 */
   float* measured_heights;   /* (N,P) h_k in m; may be NULL */
+  /* the samples h_k is read from: NULL = the sim's heightfield at each launch (0 on the plane); non-NULL = this field
+   * (validated and copied at this call; its samples stay caller-owned device memory), e.g. the samples a triangle-mesh
+   * ground was made from (legged_gym reads height_samples with mesh_type 'trimesh') */
+  const DyrosHeightField* field;
 } DyrosHeightScan;
 int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* scan);
 /* Critic states (DESIGN.md section 4, "Critic states"): a privileged row per env for an asymmetric critic, written by

@@ -89,6 +89,74 @@ class HeightField:
 
 
 @dataclass
+class TriangleMesh:
+    """Triangle-mesh ground (gym.add_triangle_mesh; DESIGN.md section 4, "Triangle-mesh ground"): vertex v sits at
+    origin + vertices[v]; triangle (a, b, c) faces the side from which a, b, c run counter-clockwise. A point touches the
+    nearest triangle; one farther than the query margin from every triangle has no ground.
+    friction: the ground's coefficient in place of CoreConfig.friction (None: keep it).
+    env_origins: (N, 3) world origins of the envs (None: the usual grid, T:709-718, with z the highest mesh surface there).
+    scan_field: the heightfield the mesh was made from; the height scan reads its samples (legged_gym's trimesh reads
+    height_samples). None: the scan reads 0, as on the plane."""
+    vertices: np.ndarray
+    triangles: np.ndarray
+    origin: tuple = (0.0, 0.0, 0.0)
+    friction: Optional[float] = None
+    env_origins: Optional[np.ndarray] = None
+    scan_field: Optional[HeightField] = None
+
+    def validate(self):
+        v, t = self.vertices, self.triangles
+        if not isinstance(v, np.ndarray) or v.dtype != np.float32 or v.ndim != 2 or v.shape[1] != 3 or len(v) < 3:
+            raise native.DyrosError("triangle mesh: vertices must be a (V, 3) float32 array with V >= 3 (got "
+                                    f"{getattr(v, 'dtype', type(v))} {getattr(v, 'shape', '')})")
+        if not isinstance(t, np.ndarray) or t.dtype != np.uint32 or t.ndim != 2 or t.shape[1] != 3 or len(t) < 1:
+            raise native.DyrosError("triangle mesh: triangles must be a (T, 3) uint32 array with T >= 1 (got "
+                                    f"{getattr(t, 'dtype', type(t))} {getattr(t, 'shape', '')})")
+        if not np.all(np.isfinite(v)):
+            raise native.DyrosError("triangle mesh: vertices must be finite")
+        if t.max() >= len(v):
+            raise native.DyrosError(f"triangle mesh: vertex index {int(t.max())} out of range (V = {len(v)})")
+        if len(self.origin) != 3 or not np.all(np.isfinite(self.origin)):
+            raise native.DyrosError(f"triangle mesh: origin must be 3 finite numbers (got {self.origin})")
+        if self.friction is not None and not (np.isfinite(self.friction) and self.friction >= 0):
+            raise native.DyrosError(f"triangle mesh: friction must be >= 0 (got {self.friction})")
+        if self.scan_field is not None:
+            self.scan_field.validate()
+
+    def height_at(self, x, y):
+        """Highest mesh surface above world points (x, y) and whether any triangle lies under them (host, float64).
+        The triangles are sorted by their lowest x once; a point tests only those whose x range can hold it (O(T)
+        memory, whatever the triangle sizes)."""
+        x, y = np.atleast_1d(np.asarray(x, np.float64)), np.atleast_1d(np.asarray(y, np.float64))
+        V = self.vertices.astype(np.float64) + np.asarray(self.origin, np.float64)
+        T = self.triangles.astype(np.int64)
+        vx, vy = V[:, 0][T], V[:, 1][T]  # (T, 3) each
+        lo_x, hi_x = vx.min(1), vx.max(1)
+        lo_y, hi_y = vy.min(1), vy.max(1)
+        order = np.argsort(lo_x, kind="stable")
+        lo_sorted = lo_x[order]
+        width = float((hi_x - lo_x).max())
+        z = np.full(x.shape, -np.inf)
+        for e in range(len(x)):
+            cand = order[np.searchsorted(lo_sorted, x[e] - width):np.searchsorted(lo_sorted, x[e], "right")]
+            cand = cand[(hi_x[cand] >= x[e]) & (lo_y[cand] <= y[e]) & (hi_y[cand] >= y[e])]
+            if len(cand) == 0:
+                continue
+            P = V[T[cand]]
+            a, b, c = P[:, 0], P[:, 1], P[:, 2]
+            d = (b[:, 0] - a[:, 0]) * (c[:, 1] - a[:, 1]) - (c[:, 0] - a[:, 0]) * (b[:, 1] - a[:, 1])
+            ok = np.abs(d) > 1e-12  # (vertical and zero-area triangles cover no x-y area)
+            d = np.where(ok, d, 1.0)
+            u = ((b[:, 0] - x[e]) * (c[:, 1] - y[e]) - (c[:, 0] - x[e]) * (b[:, 1] - y[e])) / d
+            v = ((c[:, 0] - x[e]) * (a[:, 1] - y[e]) - (a[:, 0] - x[e]) * (c[:, 1] - y[e])) / d
+            w = 1 - u - v
+            inside = ok & (u >= -1e-9) & (v >= -1e-9) & (w >= -1e-9)
+            if inside.any():
+                z[e] = (u * a[:, 2] + v * b[:, 2] + w * c[:, 2])[inside].max()
+        return z, np.isfinite(z)
+
+
+@dataclass
 class TerrainCurriculum:
     """Envs on a grid of sub-terrains and the terrain curriculum (legged_gym's _update_terrain_curriculum; DESIGN.md
     section 4, "Curriculum"): env e starts at origins[levels[e], types[e]]. With `curriculum`, every reset moves it one
@@ -159,6 +227,7 @@ class CoreConfig:
     physics_program: str = "roles"       # "roles": one lane per env, warp per role (default); "lanes": 8 lanes per env
     self_collision: bool = True          # create_actor(..., filter 0), T:354: the actor's shapes collide with each other
     heightfield: Optional[HeightField] = None  # ground: None = the plane z = 0 (gym.add_ground), else gym.add_heightfield
+    triangle_mesh: Optional[TriangleMesh] = None  # ground: gym.add_triangle_mesh (exclusive with heightfield)
     terrain_curriculum: Optional[TerrainCurriculum] = None  # env origins on sub-terrains (+ level updates on reset)
     # (P, 2) points of the height scan in the base's yaw frame (legged_gym's height_points; DESIGN.md section 4, "Height
     # scan"), or None: each observation row gains P terrain heights around the base, on any ground
@@ -300,6 +369,16 @@ class DyrosCore:
                                         "program is plane only)")
             if hf.friction is not None:
                 self.cfg = replace(self.cfg, friction=float(hf.friction))
+        tm = self.cfg.triangle_mesh
+        if tm is not None:
+            if hf is not None:
+                raise native.DyrosError("triangle mesh: the config already has a heightfield ground (one ground per sim)")
+            tm.validate()
+            if self.cfg.physics_program != "roles":
+                raise native.DyrosError("triangle mesh: only the roles physics program has a triangle-mesh ground (the "
+                                        "lanes program is plane only)")
+            if tm.friction is not None:
+                self.cfg = replace(self.cfg, friction=float(tm.friction))
         tc = self.cfg.terrain_curriculum
         if tc is not None:
             if not with_task:
@@ -403,7 +482,8 @@ class DyrosCore:
             if tc.curriculum:
                 tb["terrain_level_mean"] = torch.tensor(float(np.mean(tc.levels)), dtype=torch.float32, device=dev)
         tb["env_origins"].copy_(torch.tensor(self._env_origins()))
-        if cfg.heightfield is not None:  # start where the first reset puts the root (T:734-735), not above (0, 0)
+        if cfg.heightfield is not None or cfg.triangle_mesh is not None:  # start where the first reset puts the root
+            # (T:734-735), not above (0, 0)
             s["root_states"][:, 0:3] = tb["env_origins"]
             s["root_states"][:, 2] += cfg.initial_height
         self.nominal_mass = float(np.float32(self.tables.total_mass()))  # (critic states: total_mass / nominal - 1)
@@ -412,31 +492,36 @@ class DyrosCore:
         tb["act_hist_head"].fill_(19)
 
     def _env_origins(self) -> np.ndarray:
-        """T:709-718; on a heightfield the given origins, or the grid with z the terrain height there; with a terrain
-        curriculum origins[levels, types] (every sub-terrain origin must then lie on the field)."""
-        hf, tc = self.cfg.heightfield, self.cfg.terrain_curriculum
+        """T:709-718; on a heightfield or a triangle mesh the given origins, or the grid with z the terrain height there
+        (on a mesh the highest surface); with a terrain curriculum origins[levels, types] (every sub-terrain origin must
+        then lie on the ground)."""
+        tc = self.cfg.terrain_curriculum
+        g = self.cfg.heightfield if self.cfg.heightfield is not None else self.cfg.triangle_mesh
+        what = "heightfield" if self.cfg.heightfield is not None else "triangle mesh"
         if tc is not None:
             table = np.asarray(tc.origins, np.float32)
-            if hf is not None:
-                inside = hf.height_at(table[..., 0], table[..., 1])[1]
+            if g is not None:
+                inside = g.height_at(table[..., 0].ravel(), table[..., 1].ravel())[1].reshape(table.shape[:2])
                 if not inside.all():
                     l, t = np.argwhere(~inside)[0]
-                    raise native.DyrosError(f"terrain curriculum: the origin of sub-terrain ({l}, {t}) lies outside the field")
+                    where = "the field" if what == "heightfield" else "the mesh"
+                    raise native.DyrosError(f"terrain curriculum: the origin of sub-terrain ({l}, {t}) lies outside {where}")
             return table[np.asarray(tc.levels), np.asarray(tc.types)]
-        if hf is None:
+        if g is None:
             return env_origins(self.N, self.cfg.env_spacing)
-        if hf.env_origins is not None:
-            o = np.asarray(hf.env_origins, np.float64)
+        if g.env_origins is not None:
+            o = np.asarray(g.env_origins, np.float64)
             if o.shape != (self.N, 3) or not np.all(np.isfinite(o)):
-                raise native.DyrosError(f"heightfield: env_origins must be a finite ({self.N}, 3) array (got {o.shape})")
+                raise native.DyrosError(f"{what}: env_origins must be a finite ({self.N}, 3) array (got {o.shape})")
+            inside = g.height_at(o[:, 0], o[:, 1])[1]
         else:
             o = env_origins(self.N, self.cfg.env_spacing).astype(np.float64)
-            o[:, 2] = hf.height_at(o[:, 0], o[:, 1])[0]
-        inside = hf.height_at(o[:, 0], o[:, 1])[1]
+            o[:, 2], inside = g.height_at(o[:, 0], o[:, 1])
         if not inside.all():
             e = int(np.flatnonzero(~inside)[0])
-            raise native.DyrosError(f"heightfield: the origin of env {e} ({o[e, 0]:.3f}, {o[e, 1]:.3f}) lies outside the "
-                                    f"field; {int((~inside).sum())} of {self.N} envs do")
+            where = "outside the field" if what == "heightfield" else "where no triangle is under it"
+            raise native.DyrosError(f"{what}: the origin of env {e} ({o[e, 0]:.3f}, {o[e, 1]:.3f}) lies {where}; "
+                                    f"{int((~inside).sum())} of {self.N} envs do")
         return o.astype(np.float32)
 
     def _pack_state_arena(self):
@@ -489,6 +574,30 @@ class DyrosCore:
             d.row_scale, d.column_scale, d.vertical_scale = hf.row_scale, hf.column_scale, hf.vertical_scale
             d.origin = (C.c_float * 3)(*hf.origin)
             native.check(self.lib.dyros_sim_set_heightfield(self.sim_handle, C.byref(d)), "dyros_sim_set_heightfield")
+        tm = self.cfg.triangle_mesh
+        self.mesh_info = None
+        if tm is not None:
+            v = np.ascontiguousarray(tm.vertices, np.float32)
+            t = np.ascontiguousarray(tm.triangles, np.uint32)
+            d = native.DyrosTriangleMesh()
+            d.vertices, d.triangles = v.ctypes.data, t.ctypes.data
+            d.num_vertices, d.num_triangles = len(v), len(t)
+            d.origin = (C.c_float * 3)(*tm.origin)
+            d.dynamic_friction = self.cfg.friction
+            native.check(self.lib.dyros_sim_set_triangle_mesh(self.sim_handle, C.byref(d)), "dyros_sim_set_triangle_mesh")
+            out = (C.c_int64 * 4)()
+            native.check(self.lib.dyros_sim_triangle_mesh_info(self.sim_handle, C.byref(out)), "dyros_sim_triangle_mesh_info")
+            # device bytes of the mesh and its grid, zero-area triangles dropped, triangles kept, buckets
+            self.mesh_info = dict(zip(("bytes", "dropped", "triangles", "buckets"), (int(x) for x in out)))
+            if tm.scan_field is not None and self.height_points is not None:
+                sf = tm.scan_field
+                self.scan_samples = torch.tensor(np.ascontiguousarray(sf.samples), dtype=torch.int16, device=self.device)
+                self.scan_field_desc = native.DyrosHeightField()
+                fd = self.scan_field_desc
+                fd.samples = self.scan_samples.data_ptr()
+                fd.num_rows, fd.num_columns = sf.samples.shape
+                fd.row_scale, fd.column_scale, fd.vertical_scale = sf.row_scale, sf.column_scale, sf.vertical_scale
+                fd.origin = (C.c_float * 3)(*sf.origin)
 
     def _create_task(self, seed: int):
         t, cfg = self.tables, self.cfg
@@ -542,6 +651,8 @@ class DyrosCore:
             d.points, d.num_points = self.task_t["height_points"].data_ptr(), self.num_height_points
             d.base_offset, d.scale = HEIGHT_SCAN_BASE_OFFSET, HEIGHT_SCAN_SCALE
             d.measured_heights = self.task_t["measured_heights"].data_ptr()
+            if getattr(self, "scan_field_desc", None) is not None:  # (a mesh made from a heightfield: its samples)
+                d.field = C.pointer(self.scan_field_desc)
             native.check(self.lib.dyros_task_set_height_scan(self.task_handle, C.byref(d)), "dyros_task_set_height_scan")
         if self.states_width:
             d = native.DyrosCriticStates()

@@ -11,6 +11,7 @@
 
 #include "host_model.h"
 #include "internal.h"
+#include "mesh_grid.h"
 
 namespace dyros {
 
@@ -46,6 +47,8 @@ static int build_sim(const DyrosSimDesc* d, const DyrosModelDesc* m, const Dyros
   sim->device = d->device;
   sim->program = d->physics_program;
   fill_sim_params(d, sim->p);
+  sim->desc_mu = sim->p.mu;
+  for (int i = 0; i < m->num_points; ++i) sim->max_radius = std::max(sim->max_radius, (float)m->pt_radius[i]);
   sim->b = *b;
   Blob bl;
   ModelOffsets off;
@@ -217,6 +220,7 @@ int dyros_sim_destroy(DyrosSim* sim) {
   Sim* s = reinterpret_cast<Sim*>(sim);
   if (!s) return 0;
   if (s->dev_blob) cudaFree(s->dev_blob);
+  if (s->mesh_blob) cudaFree(s->mesh_blob);
   delete s;
   return 0;
 }
@@ -359,6 +363,7 @@ int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* f) {
   }
   REQUIRE(s->program == 0, "dyros_sim_set_heightfield: the lanes physics program (physics_program 1) has no heightfield "
                            "ground; use the roles program (0)");
+  REQUIRE(!s->has_mesh, "dyros_sim_set_heightfield: the sim already has a triangle-mesh ground (one ground per sim)");
   REQUIRE(f->samples, "dyros_sim_set_heightfield: samples is NULL");
   REQUIRE(f->num_rows >= 2 && f->num_columns >= 2, "dyros_sim_set_heightfield: need at least 2 x 2 samples (got %d x %d)",
           f->num_rows, f->num_columns);
@@ -398,6 +403,68 @@ int dyros_sim_set_heightfield(DyrosSim* sim, const DyrosHeightField* f) {
   g.cull = (float)std::sqrt(1 + gmax) * (1 + 1e-5f);                 // 1 / smallest n_z
   s->has_field = true;  // (same launch geometry as the plane: the env scratch block is the same size)
   s->field = g;
+  return 0;
+}
+
+static void free_mesh(Sim* s) {
+  if (s->mesh_blob) cudaFree(s->mesh_blob);
+  s->mesh_blob = nullptr;
+  s->has_mesh = false;
+  s->mesh = MeshGround{};
+  s->mesh_bytes = 0;
+  s->mesh_dropped = 0;
+  s->mesh_kept = 0;
+  s->p.mu = s->desc_mu;
+}
+
+// Copies the mesh and builds its bucket grid (mesh_grid.h), then uploads both in one allocation.
+int dyros_sim_set_triangle_mesh(DyrosSim* sim, const DyrosTriangleMesh* mesh) {
+  SIM_OR_FAIL("dyros_sim_set_triangle_mesh");
+  if (!mesh) {
+    DY_CUDA(cudaSetDevice(s->device));
+    free_mesh(s);
+    return 0;
+  }
+  REQUIRE(s->program == 0, "dyros_sim_set_triangle_mesh: the lanes physics program (physics_program 1) has no "
+                           "triangle-mesh ground; use the roles program (0)");
+  REQUIRE(!s->has_field, "dyros_sim_set_triangle_mesh: the sim already has a heightfield ground (one ground per sim)");
+  MeshGrid mg;
+  const std::string err = build_mesh_grid(mesh, (double)s->p.contact_offset + s->max_radius + kMeshDepthAllowance, mg);
+  REQUIRE(err.empty(), "dyros_sim_set_triangle_mesh: %s", err.c_str());
+  const size_t b_tri = mg.tri.size() * sizeof(float4), b_cell = mg.cell.size() * sizeof(int4), b_list = mg.list.size() * sizeof(int);
+  DY_CUDA(cudaSetDevice(s->device));
+  free_mesh(s);
+  void* blob = nullptr;
+  DY_CUDA(cudaMalloc(&blob, b_tri + b_cell + b_list));
+  char* base = static_cast<char*>(blob);
+  cudaError_t e = cudaMemcpy(base, mg.tri.data(), b_tri, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(base + b_tri, mg.cell.data(), b_cell, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && b_list) e = cudaMemcpy(base + b_tri + b_cell, mg.list.data(), b_list, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    cudaFree(blob);
+    set_error("dyros_sim_set_triangle_mesh: CUDA error while uploading the mesh: %s", cudaGetErrorString(e));
+    return 1;
+  }
+  MeshGround g = mg.g;
+  g.tri = reinterpret_cast<const float4*>(base);
+  g.cell = reinterpret_cast<const int4*>(base + b_tri);
+  g.list = reinterpret_cast<const int*>(base + b_tri + b_cell);
+  s->mesh_blob = blob;
+  s->mesh_bytes = b_tri + b_cell + b_list;
+  s->mesh_dropped = mg.dropped;
+  s->mesh_kept = mg.kept;
+  s->mesh = g;
+  s->has_mesh = true;  // (same launch geometry as the plane: the env scratch block is the same size)
+  s->p.mu = mesh->dynamic_friction;
+  return 0;
+}
+int dyros_sim_triangle_mesh_info(DyrosSim* sim, int64_t out[4]) {
+  SIM_OR_FAIL("dyros_sim_triangle_mesh_info");
+  REQUIRE(out, "dyros_sim_triangle_mesh_info: out is NULL");
+  out[0] = (int64_t)s->mesh_bytes;
+  out[1] = s->mesh_dropped;
+  out[2] = s->mesh_kept;
+  out[3] = s->has_mesh ? (int64_t)s->mesh.gx * s->mesh.gy : 0;
   return 0;
 }
 
@@ -461,6 +528,7 @@ int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* sc) {
   TASK_OR_FAIL("dyros_task_set_height_scan");
   if (!sc) {
     t->scan = DyrosHeightScan{};
+    t->scan_own_field = false;
     return 0;
   }
   REQUIRE(sc->points && (reinterpret_cast<uintptr_t>(sc->points) & 7) == 0,
@@ -473,7 +541,28 @@ int dyros_task_set_height_scan(DyrosTask* task, const DyrosHeightScan* sc) {
   DY_CUDA(cudaSetDevice(t->sim->device));
   DY_CUDA(cudaMemcpy(pts.data(), sc->points, pts.size() * sizeof(float), cudaMemcpyDeviceToHost));
   for (float v : pts) REQUIRE(std::isfinite(v), "dyros_task_set_height_scan: points must be finite");
+  FieldGround g{};
+  if (const DyrosHeightField* f = sc->field) {
+    REQUIRE(f->samples && f->num_rows >= 2 && f->num_columns >= 2,
+            "dyros_task_set_height_scan: field needs samples of at least 2 x 2");
+    REQUIRE(f->row_scale > 0 && f->column_scale > 0 && f->vertical_scale > 0 && std::isfinite(f->row_scale) &&
+                std::isfinite(f->column_scale) && std::isfinite(f->vertical_scale) && std::isfinite(f->origin[0]) &&
+                std::isfinite(f->origin[1]) && std::isfinite(f->origin[2]),
+            "dyros_task_set_height_scan: field scales must be positive and its origin finite");
+    g.s = f->samples;
+    g.nr = f->num_rows;
+    g.nc = f->num_columns;
+    g.ox = f->origin[0];
+    g.oy = f->origin[1];
+    g.oz = f->origin[2];
+    g.dx = f->row_scale;
+    g.dy = f->column_scale;
+    g.dz = f->vertical_scale;
+  }
   t->scan = *sc;
+  t->scan.field = nullptr;  // (copied into scan_field: the caller's struct need not outlive this call)
+  t->scan_own_field = sc->field != nullptr;
+  t->scan_field = g;
   return 0;
 }
 int dyros_task_set_critic_states(DyrosTask* task, const DyrosCriticStates* cs) {

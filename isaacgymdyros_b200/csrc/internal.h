@@ -93,18 +93,47 @@ struct DevModel {
 };
 
 // The ground of the physics kernels' role program (physics_roles.cuh), a compile-time parameter: the plane z = 0 with
-// normal +z, or a heightfield (DESIGN.md section 4).
+// normal +z, a heightfield or a triangle mesh (DESIGN.md section 4). kField: contacts carry their own ground normal
+// (heightfield and mesh); kMesh: the normal and gap come from the mesh narrow phase (mesh_query).
 struct PlaneGround {
   static constexpr bool kField = false;
+  static constexpr bool kMesh = false;
 };
 struct FieldGround {
   static constexpr bool kField = true;
+  static constexpr bool kMesh = false;
   const int16_t* s;        // (nr, nc) samples, row-major: row i along x, column j along y (device memory)
   int nr, nc;              // >= 2 each
   float ox, oy, oz;        // transform.p
   float dx, dy, dz;        // row_scale, column_scale, vertical_scale
   float zmax;              // height of the highest vertex
   float cull;              // 1 / (smallest n_z of any triangle) >= 1: see link_ext_wrench
+};
+// Triangle mesh (dyros_sim_set_triangle_mesh): a uniform x-y bucket grid in CSR form, built on the host. Bucket (bx, by)
+// covers [x0 + bx B, x0 + (bx + 1) B) x [y0 + by B, ...) and lists, in ascending order, every triangle whose x-y bounds
+// dilated by the query margin overlap it: a point reads exactly one bucket.
+constexpr float kMeshBucket = 0.1f;       // B, m
+constexpr int kMeshBucketCap = 1024;      // triangles of one bucket
+constexpr long long kMeshMaxCells = 1ll << 27;
+constexpr float kMeshDepthAllowance = 0.1f;  // D: the query margin is contact_offset + largest radius + D
+struct MeshGround {
+  static constexpr bool kField = true;
+  static constexpr bool kMesh = true;
+  const float4* tri;       // (T, 3): vertex a (world), b - a, c - a; the w components hold the unit face normal
+  const int4* cell;        // (gx * gy) first list entry, entry count, sign bound, top (float bits). top: the highest
+                           // vertex of the bucket's triangles (rounded up); a point with c.z - top > margin is farther
+                           // than the margin from all of them, on any mesh. sign bound: top, or +inf when one of the
+                           // triangles does not face up (n_z < 1e-6); a point with c.z - r > bound + contact_offset
+                           // cannot touch on a height-function mesh (each vertical line meets its up-facing surface once,
+                           // as on legged_gym's meshes: the nearest triangle is a tread, nearer or tied, and s > 0). On
+                           // other meshes, e.g. above the top edge of a steep face and behind it, s can be negative
+                           // there: that cull assumes a height-function mesh (DESIGN.md section 4)
+  const int* list;         // triangle indices, bucket after bucket
+  int gx, gy;
+  float x0, y0, inv_b;     // grid origin and 1 / B
+  float margin;            // M
+  float ztop;              // the whole mesh's highest vertex (rounded up): see link_ext_wrench
+  float zmax;              // ztop, or +inf when a triangle is not facing up: see link_ext_wrench
 };
 
 // The height scan of the observation kernels (DESIGN.md section 4, "Height scan"), a compile-time parameter of
@@ -120,7 +149,7 @@ struct HeightScan {
   float base_offset, scale;
   float* measured;         // (N, P) heights in m, or NULL
   int has_field;           // 0: the plane z = 0 (every height 0)
-  FieldGround f;           // the sim's heightfield when has_field
+  FieldGround f;           // the samples when has_field: DyrosHeightScan.field, else the sim's heightfield
 };
 
 // The critic's state row (DESIGN.md section 4, "Critic states"), a second compile-time parameter of the same kernels:
@@ -198,6 +227,14 @@ struct Sim {
   size_t phys_smem = 0;      // dynamic shared memory of one physics CTA
   bool has_field = false;    // ground: false = the plane z = 0, true = the heightfield `field` (dyros_sim_set_heightfield)
   FieldGround field{};
+  bool has_mesh = false;     // ground: the triangle mesh `mesh` (dyros_sim_set_triangle_mesh); exclusive with has_field
+  MeshGround mesh{};
+  void* mesh_blob = nullptr; // device memory of the mesh's triangles and grid (owned)
+  size_t mesh_bytes = 0;
+  long long mesh_dropped = 0;  // zero-area triangles left out of the mesh
+  long long mesh_kept = 0;     // triangles of the mesh
+  float max_radius = 0;      // largest penalty / sole-sphere radius of the model (query margin)
+  float desc_mu = 0;         // DyrosSimDesc.friction (p.mu is the mesh's dynamic_friction while a mesh is set)
 };
 
 struct Task {
@@ -208,6 +245,8 @@ struct Task {
   DyrosTerrainCurriculum cur{};  // dyros_task_set_terrain_curriculum; levels == NULL: off
   DyrosHeightScan scan{};        // dyros_task_set_height_scan; num_points == 0: off
   DyrosCriticStates crit{};      // dyros_task_set_critic_states; states == NULL: off
+  bool scan_own_field = false;   // the height scan reads scan_field (DyrosHeightScan.field) instead of the sim's ground
+  FieldGround scan_field{};
   void* dev_blob = nullptr;
   // the heights of a height scan go into the observation row unless critic states take them alone
   int obs_width() const { return NOBS + (!crit.states || crit.heights_in_obs ? scan.num_points : 0); }

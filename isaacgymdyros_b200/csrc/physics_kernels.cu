@@ -89,7 +89,7 @@ __device__ __forceinline__ EnvIO env_io(const DevModel& m, const DyrosSimBuffers
   return io;
 }
 
-// (both kernels are instantiated for each ground, PlaneGround and FieldGround: physics_roles.cuh)
+// (both kernels are instantiated for each ground, PlaneGround, FieldGround and MeshGround: physics_roles.cuh)
 template <class Ground>
 __global__ void __launch_bounds__(kPhysThreads) k_simulate(DevModel m, SimParams p, DyrosSimBuffers b, const float* __restrict__ push,
                                                            int apply_wrench, int epb, int es, Ground gnd) {
@@ -150,13 +150,18 @@ static int physics_configure_roles(Sim* sim) {
   DY_CUDA(cudaFuncSetAttribute(k_step_physics<PlaneGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
   DY_CUDA(cudaFuncSetAttribute(k_simulate<FieldGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
   DY_CUDA(cudaFuncSetAttribute(k_step_physics<FieldGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_simulate<MeshGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
+  DY_CUDA(cudaFuncSetAttribute(k_step_physics<MeshGround>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPhysSmem));
   return 0;
 }
 
 static int launch_simulate_roles(Sim* sim, int apply_wrench, const float* push, cudaStream_t s) {
   const int epb = sim->envs_per_block;
   const int grid = (sim->p.N + epb - 1) / epb;
-  if (sim->has_field)
+  if (sim->has_mesh)
+    k_simulate<<<grid, kPhysThreads, sim->phys_smem, s>>>(sim->m, sim->p, sim->b, push, apply_wrench, epb, env_scratch_floats(sim->m.nl, sim->m.nb),
+                                                     sim->mesh);
+  else if (sim->has_field)
     k_simulate<<<grid, kPhysThreads, sim->phys_smem, s>>>(sim->m, sim->p, sim->b, push, apply_wrench, epb, env_scratch_floats(sim->m.nl, sim->m.nb),
                                                      sim->field);
   else
@@ -170,7 +175,10 @@ static int launch_task_physics_roles(Task* t, cudaStream_t s, long long* trace, 
   Sim* sim = t->sim;
   const int epb = sim->envs_per_block;
   const int grid = (sim->p.N + epb - 1) / epb;
-  if (sim->has_field)
+  if (sim->has_mesh)
+    DY_CUDA(launch_kernel(k_step_physics<MeshGround>, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p,
+                          make_tk(t), epb, env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions, sim->mesh));
+  else if (sim->has_field)
     DY_CUDA(launch_kernel(k_step_physics<FieldGround>, dim3(grid), dim3(kStepThreads), sim->phys_smem, s, pdl, sim->m, sim->p,
                           make_tk(t), epb, env_scratch_floats(sim->m.nl, sim->m.nb), trace, actions, sim->field));
   else

@@ -22,6 +22,7 @@
 // three tree passes and the whole contact stage while the arm roles are still in theirs.
 // The same source is compiled for the host by tests/native/hostemu.cu (one thread per role, atomics for the flags).
 #pragma once
+#include <string.h>
 #include "internal.h"
 #include "phys_math.cuh"
 
@@ -159,6 +160,120 @@ HD void field_tangents(V3 n, V3& t1, V3& t2) {
   t1 = v3(n.z * inv, 0, -n.x * inv);
   t2 = cross(n, t1);
 }
+// Mesh: the same rule, and t1 = normalize(0, n_z, -n_y) where n_x^2 + n_z^2 < 1e-6 (a wall facing +-y, such as a riser
+// of legged_gym's trimesh stairs, where the heightfield rule divides by zero).
+HD void mesh_tangents(V3 n, V3& t1, V3& t2) {
+  const real q = n.z * n.z + n.x * n.x;
+  if (q < (real)1e-6) {
+    const real inv = 1 / sqrt(n.z * n.z + n.y * n.y);
+    t1 = v3(0, n.z * inv, -n.y * inv);
+  } else {
+    const real inv = 1 / sqrt(q);
+    t1 = v3(n.z * inv, 0, -n.x * inv);
+  }
+  t2 = cross(n, t1);
+}
+
+HD float4 mesh_ld(const float4* p) {
+#ifdef __CUDA_ARCH__
+  return __ldg(p);  // read-only path: the mesh is shared by every env and stays in L2
+#else
+  return *p;
+#endif
+}
+HD int4 mesh_ld(const int4* p) {
+#ifdef __CUDA_ARCH__
+  return __ldg(p);
+#else
+  return *p;
+#endif
+}
+HD float mesh_bound(int bits) {  // the height bound of a bucket, stored as the bits of a float
+#ifdef __CUDA_ARCH__
+  return __int_as_float(bits);
+#else
+  float f;
+  memcpy(&f, &bits, 4);
+  return f;
+#endif
+}
+HD int mesh_ld(const int* p) {
+#ifdef __CUDA_ARCH__
+  return __ldg(p);
+#else
+  return *p;
+#endif
+}
+
+// Mesh narrow phase (DESIGN.md section 4, "Triangle-mesh ground") for a sphere of centre c and radius r: the triangle T*
+// nearest to c (ties: the lowest index), the signed distance s = +-|c - p| (the sign of (c - p) . n_f(T*)) and the unit
+// normal n = sign (c - p) / |c - p|, or n_f(T*) below 1e-6 m. False (no ground) off the grid, farther than the margin
+// from every triangle, and after one load of the bucket where c.z - top > margin (farther than the margin from every
+// listed triangle) or c.z - r > sign bound + contact_offset (neither a sole point, phi >= contact_offset, nor a penalty
+// sphere, depth <= 0, can touch a height-function mesh: MeshGround.cell). Closest points are formed relative to vertex
+// a (coordinates reach ~200 m).
+HD bool mesh_query(const MeshGround& g, V3 c, real r, real contact_offset, real& s, V3& n) {
+  const real u = (c.x - g.x0) * g.inv_b, v = (c.y - g.y0) * g.inv_b;
+  if (!(u >= 0 && v >= 0 && u < (real)g.gx && v < (real)g.gy)) return false;
+  const int4 cell = mesh_ld(g.cell + (size_t)(int)v * g.gx + (int)u);
+  if (c.z - r > (real)mesh_bound(cell.z) + contact_offset || c.z - (real)mesh_bound(cell.w) > (real)g.margin) return false;
+  real best = (real)g.margin * (real)g.margin;
+  bool hit = false;
+  V3 bd = v3(0, 0, 0), bn = v3(0, 0, 1);
+  bool interior = false;
+#pragma unroll 1
+  for (int k = 0; k < cell.y; ++k) {
+    const float4* t = g.tri + 3 * (size_t)mesh_ld(g.list + cell.x + k);
+    const float4 A = mesh_ld(t), B = mesh_ld(t + 1), C = mesh_ld(t + 2);
+    const V3 q = v3(c.x - A.x, c.y - A.y, c.z - A.z), e1 = v3(B.x, B.y, B.z), e2 = v3(C.x, C.y, C.z);
+    const V3 nf = v3(A.w, B.w, C.w);
+    // closest point p (relative to a) by the Voronoi regions of the triangle
+    const real d1 = dot(e1, q), d2 = dot(e2, q);
+    V3 p;
+    bool in = false;
+    if (d1 <= 0 && d2 <= 0) {
+      p = v3(0, 0, 0);
+    } else {
+      const V3 qb = q - e1;
+      const real d3 = dot(e1, qb), d4 = dot(e2, qb);
+      const V3 qc = q - e2;
+      const real d5 = dot(e1, qc), d6 = dot(e2, qc);
+      const real vc = d1 * d4 - d3 * d2, vb = d5 * d2 - d1 * d6, va = d3 * d6 - d5 * d4;
+      if (d3 >= 0 && d4 <= d3) p = e1;
+      else if (d6 >= 0 && d5 <= d6) p = e2;
+      else if (vc <= 0 && d1 >= 0 && d3 <= 0) p = (d1 / (d1 - d3)) * e1;
+      else if (vb <= 0 && d2 >= 0 && d6 <= 0) p = (d2 / (d2 - d6)) * e2;
+      else if (va <= 0 && d4 - d3 >= 0 && d5 - d6 >= 0) p = e1 + ((d4 - d3) / ((d4 - d3) + (d5 - d6))) * (e2 - e1);
+      else {
+        p = v3(0, 0, 0);
+        in = true;
+      }
+    }
+    V3 d;
+    real d2s;
+    if (in) {  // inside the face: c - p is along n_f
+      const real h = dot(q, nf);
+      d = h * nf;
+      d2s = h * h;
+    } else {
+      d = q - p;
+      d2s = dot(d, d);
+    }
+    if (d2s < best) {
+      best = d2s;
+      hit = true;
+      bd = d;
+      bn = nf;
+      interior = in;
+    }
+  }
+  if (!hit) return false;
+  const real dd = sqrt(best);
+  const real sg = dot(bd, bn) >= 0 ? (real)1 : (real)-1;
+  s = sg * dd;
+  n = (interior || dd < (real)1e-6) ? bn : (sg / dd) * bd;
+  return true;
+}
 
 // Heightfield: the active sole points of foot g (X_PTS, at most MAX_ACTIVE_PTS) from the start-of-step foot pose
 // (X_FOOTPOSE); returns their number and the foot's world rotation. Gap phi = (z_c - h) n_z - r of a candidate sphere
@@ -190,12 +305,42 @@ HD int field_select(const FieldGround& gnd, const DevModel& m, const SimParams& 
   return nact;
 }
 
+// Mesh: the same selection with phi = s - r from mesh_query.
+HD int field_select(const MeshGround& gnd, const DevModel& m, const SimParams& p, real* sm, real* X, int g, real inv_dt,
+                    M3& Rwf) {
+  Rwf = ld_m3(X + X_FOOTPOSE + 12 * g);
+  const V3 pf = ld3(X + X_FOOTPOSE + 12 * g + 9);
+  real* const pts = X + X_PTS + g * MAX_ACTIVE_PTS * PT_WORDS;
+  int nact = 0;
+  real sd;
+  V3 n;
+#pragma unroll 1
+  for (int k = 0; k < m.foot_npts[g]; ++k) {
+    const V3 c = pf + mul(Rwf, v3(m.foot_pt_pos[g][k][0], m.foot_pt_pos[g][k][1], m.foot_pt_pos[g][k][2]));
+    const real rad = m.foot_pt_radius[g][k];
+    if (!mesh_query(gnd, c, rad, p.contact_offset, sd, n)) continue;
+    real phi = sd - rad;
+    if (phi < p.contact_offset && nact < MAX_ACTIVE_PTS) {
+      real* pt = pts + nact * PT_WORDS;
+      reinterpret_cast<int*>(pt)[0] = k;
+      pt[1] = phi >= 0 ? -phi * inv_dt : fmin_r(-p.erp * phi * inv_dt, p.max_depen_vel);
+      pt[2] = pt[3] = pt[4] = 0;
+      st3(BLK(m.chain[g][nact]) + LS_WP, n);
+      ++nact;
+    }
+  }
+  return nact;
+}
+
 // Heightfield: active sole point `a` of foot g -> its contact location relative to the foot origin, world axes (the
 // sphere's point along -n), and its row directions n, t1, t2.
+// (mesh: the same, with mesh_tangents)
+template <class Ground>
 HD void field_sole_point(const DevModel& m, const real* sm, const real* X, const M3& Rwf, int g, int a, V3& xa, V3* dirs) {
   const int k = reinterpret_cast<const int*>(X + X_PTS + (g * MAX_ACTIVE_PTS + a) * PT_WORDS)[0];
   dirs[0] = ld3(BLK(m.chain[g][a]) + LS_WP);
-  field_tangents(dirs[0], dirs[1], dirs[2]);
+  if constexpr (Ground::kMesh) mesh_tangents(dirs[0], dirs[1], dirs[2]);
+  else field_tangents(dirs[0], dirs[1], dirs[2]);
   xa = mul(Rwf, v3(m.foot_pt_pos[g][k][0], m.foot_pt_pos[g][k][1], m.foot_pt_pos[g][k][2])) - m.foot_pt_radius[g][k] * dirs[0];
 }
 
@@ -287,7 +432,39 @@ HD SV link_ext_wrench(const EnvIO& io, const real* X, const float* hot, const De
       fext.v = fext.v + F;
     }
   }
-  if constexpr (Ground::kField) {
+  if constexpr (Ground::kMesh) {
+    // Culls: every sphere centre and rim point of the link lies at most reach below the link origin. So with
+    // pw.z >= ztop + reach + margin all are farther than the margin from the mesh (any mesh); and on a height-function
+    // mesh with every triangle facing up (zmax finite), nothing can touch with pw.z >= zmax + reach (s >= height above
+    // the vertices).
+    if (pw.z - gnd.zmax < R[R_REACH] && pw.z - gnd.ztop < R[R_REACH] + gnd.margin) {
+      const real mu = X[X_MU];
+      real sd;
+      V3 n;
+#pragma unroll 1
+      for (int k = RI(R, R_PT0); k < RI(R, R_PT1); ++k) {
+        const V3 xw = mul(Rw, ld3_f(m.pt_pos + 3 * k));
+        const real rad = m.pt_radius[k];
+        if (!mesh_query(gnd, pw + xw, rad, p.contact_offset, sd, n)) continue;
+        penalty_point_n(p, mu, v, xw - rad * n, n, rad - sd, io.contact + 3 * m.pt_body[k], io.live, fext);
+      }
+#pragma unroll 1
+      for (int k = RI(R, R_CYL0); k < RI(R, R_CYL1); ++k) {  // the rim point lowest in WORLD z, as for the plane
+        V3 c = ld3_f(m.cyl_center + 3 * k), a = ld3_f(m.cyl_axis + 3 * k);
+        real rad = m.cyl_size[2 * k], hh = m.cyl_size[2 * k + 1];
+        real az = dot(nrm, a);
+        real s = az >= 0 ? (real)-1 : (real)1;
+        V3 d = neg(nrm - az * a);
+        real dn = sqrt(dot(d, d));
+        V3 rim = c + (s * hh) * a;
+        if (dn > (real)1e-6) rim = rim + (rad / dn) * d;
+        const V3 xw = mul(Rw, rim);
+        if (!mesh_query(gnd, pw + xw, (real)0, p.contact_offset, sd, n)) continue;
+        penalty_point_n(p, mu, v, xw, n, -sd, io.contact + 3 * m.cyl_body[k], io.live, fext);
+      }
+    }
+    return fext;
+  } else if constexpr (Ground::kField) {
     // Cull: a sphere of radius r <= reach touches where (h - z_c) n_z + r > 0, i.e. z_c < h + r / n_z, and its centre is
     // at most reach - r below the link origin; a cylinder's rim point at most reach below it. So nothing of this link
     // can touch unless pw.z < zmax + reach * cull.
@@ -384,7 +561,7 @@ HD void env_store_outputs(const EnvIO& io, const real* sm, const float* hot, con
 // with `io_async` the per-sub-step inputs are staged concurrently by another warp, which publishes F_IO_PRE (push,
 // zeroed contact forces: needed by the force loop), F_IO_TAU (torque, damping, armature: needed by pass 2) and
 // F_IO_DONE (it has finished reading the joint angles, which the last pass overwrites).
-// `gnd`: the ground (PlaneGround or FieldGround).
+// `gnd`: the ground (PlaneGround, FieldGround or MeshGround).
 template <class Sync, class Ground = PlaneGround>
 HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const float* hot, const DevModel& m,
                          const SimParams& p, int role, Sync& sync, bool io_async = false, const Ground& gnd = Ground()) {
@@ -716,7 +893,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
 #pragma unroll 1
       for (int a = 0; a < nact; ++a) {
         V3 xa, dirs[3];
-        field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+        field_sole_point<Ground>(m, sm, X, Rwf, g, a, xa, dirs);
 #pragma unroll
         for (int d = 0; d < 3; ++d) {
           SV J{cross(xa, dirs[d]), dirs[d]};
@@ -753,7 +930,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
         for (int a = 0; a < nact; ++a) {
           real* pt = pts + a * PT_WORDS;
           V3 xa, dirs[3];
-          field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+          field_sole_point<Ground>(m, sm, X, Rwf, g, a, xa, dirs);
           const real bias = pt[1];
           real lam[3] = {pt[2], pt[3], pt[4]};
 #pragma unroll
@@ -841,7 +1018,7 @@ HD void env_substep_role(const EnvIO& io, real* sm, int* flags, int epoch, const
         float* cf = io.contact + 3 * m.foot_pt_body[g][reinterpret_cast<const int*>(pt)[0]];
         if constexpr (Ground::kField) {  // (lam_n n + lam_1 t1 + lam_2 t2) / dt
           V3 xa, dirs[3];
-          field_sole_point(m, sm, X, Rwf, g, a, xa, dirs);
+          field_sole_point<Ground>(m, sm, X, Rwf, g, a, xa, dirs);
           const V3 F = (pt[2] * inv_dt) * dirs[0] + (pt[3] * inv_dt) * dirs[1] + (pt[4] * inv_dt) * dirs[2];
           cf[0] += (float)F.x;
           cf[1] += (float)F.y;

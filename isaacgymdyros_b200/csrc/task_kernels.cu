@@ -1084,8 +1084,9 @@ static inline HeightScan kernel_arg(const Task* t, HeightScan sc) {
   sc.base_offset = t->scan.base_offset;
   sc.scale = t->scan.scale;
   sc.measured = t->scan.measured_heights;
-  sc.has_field = t->sim->has_field ? 1 : 0;  // the sim's ground at this launch (dyros_sim_set_heightfield)
-  sc.f = t->sim->field;
+  // DyrosHeightScan.field, else the sim's ground at this launch (dyros_sim_set_heightfield; 0 on a plane or a mesh)
+  sc.has_field = t->scan_own_field || t->sim->has_field ? 1 : 0;
+  sc.f = t->scan_own_field ? t->scan_field : t->sim->field;
   return sc;
 }
 static inline CriticStates kernel_arg(const Task* t, CriticStates st) {

@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import native
-from .core import ARMATURE, ASSETS, CoreConfig, DyrosCore, HeightField, stable_penalty
+from .core import ARMATURE, ASSETS, CoreConfig, DyrosCore, HeightField, TriangleMesh, stable_penalty
 from .model.mjcf import load_mjcf
 from .model.tables import ModelTables, build_tables
 
@@ -240,7 +240,8 @@ class Sim:
     def __init__(self, compute_device: int, params: SimParams):
         self.compute_device, self.params = compute_device, params
         self.plane: Optional[PlaneParams] = None
-        self.heightfield: Optional[HeightField] = None  # add_heightfield (a sim has one ground: plane or heightfield)
+        self.heightfield: Optional[HeightField] = None  # add_heightfield (a sim has one ground: plane, heightfield or mesh)
+        self.triangle_mesh: Optional[TriangleMesh] = None  # add_triangle_mesh
         self.asset: Optional[Asset] = None
         self.envs: List[Env] = []
         self.start_poses: List[Transform] = []
@@ -274,6 +275,11 @@ def _cfg_from_sim(sim: Sim) -> CoreConfig:
         pos = np.array([[tf.p.x, tf.p.y, 0.0] for tf in sim.start_poses], np.float64).reshape(-1, 3)
         pos[:, 2] = sim.heightfield.height_at(pos[:, 0], pos[:, 1])[0]
         cfg.heightfield = replace(sim.heightfield, env_origins=pos)
+    if sim.triangle_mesh is not None:
+        cfg.friction = float(sim.triangle_mesh.friction)
+        pos = np.array([[tf.p.x, tf.p.y, 0.0] for tf in sim.start_poses], np.float64).reshape(-1, 3)
+        pos[:, 2] = sim.triangle_mesh.height_at(pos[:, 0], pos[:, 1])[0]
+        cfg.triangle_mesh = replace(sim.triangle_mesh, env_origins=pos)
     if sim.asset is not None:
         cfg.max_angular_velocity = float(sim.asset.options.max_angular_velocity)
     return cfg
@@ -302,6 +308,8 @@ class Gym:
     def add_ground(self, sim: Sim, params: PlaneParams):
         if sim.heightfield is not None:
             raise native.DyrosError("add_ground: the sim already has a heightfield ground (one ground per sim)")
+        if sim.triangle_mesh is not None:
+            raise native.DyrosError("add_ground: the sim already has a triangle-mesh ground (one ground per sim)")
         n = params.normal
         if (round(n.x, 6), round(n.y, 6), round(n.z, 6)) != (0.0, 0.0, 1.0) or params.distance != 0.0:
             raise native.DyrosError("add_ground: only the z = 0 plane with normal +z is implemented (T:227-235)")
@@ -310,9 +318,9 @@ class Gym:
     def add_heightfield(self, sim: Sim, heightSamples, params: HeightFieldParams):
         """The ground of the sim becomes a heightfield (legged_gym terrain, mesh_type 'heightfield'): int16 samples of
         shape (nbRows, nbColumns), or their row-major flattening. Outside the field there is no ground."""
-        if sim.plane is not None or sim.heightfield is not None:
-            raise native.DyrosError("add_heightfield: the sim already has a ground (one ground per sim: a plane or a "
-                                    "heightfield)")
+        if sim.plane is not None or sim.heightfield is not None or sim.triangle_mesh is not None:
+            raise native.DyrosError("add_heightfield: the sim already has a ground (one ground per sim: a plane, a "
+                                    "heightfield or a triangle mesh)")
         if sim.core is not None:
             raise native.DyrosError("add_heightfield: call it before prepare_sim")
         r = params.transform.r
@@ -331,8 +339,31 @@ class Gym:
         sim.heightfield = hf
 
     def add_triangle_mesh(self, sim: Sim, vertices, triangles, params: "TriangleMeshParams"):
-        raise native.DyrosError("add_triangle_mesh: triangle-mesh ground is not implemented (it needs a general mesh "
-                                "narrow phase); use add_heightfield (mesh_type 'heightfield') or add_ground")
+        """The ground of the sim becomes a triangle mesh (legged_gym terrain, mesh_type 'trimesh'): float32 vertices
+        (nb_vertices, 3) and uint32 triangles (nb_triangles, 3), or their row-major flattenings, placed at transform.p.
+        A point farther than the query margin from every triangle has no ground (DESIGN.md section 4)."""
+        if sim.plane is not None or sim.heightfield is not None or sim.triangle_mesh is not None:
+            raise native.DyrosError("add_triangle_mesh: the sim already has a ground (one ground per sim: add_ground, "
+                                    "add_heightfield or add_triangle_mesh)")
+        if sim.core is not None:
+            raise native.DyrosError("add_triangle_mesh: call it before prepare_sim")
+        r = params.transform.r
+        if (round(r.x, 6), round(r.y, 6), round(r.z, 6), round(abs(r.w), 6)) != (0.0, 0.0, 0.0, 1.0):
+            raise native.DyrosError("add_triangle_mesh: only an identity transform.r is implemented (the mesh is not rotated)")
+        v, t = np.asarray(vertices), np.asarray(triangles)
+        if v.dtype != np.float32:
+            raise native.DyrosError(f"add_triangle_mesh: vertices must be float32 (got {v.dtype})")
+        if t.dtype != np.uint32:
+            raise native.DyrosError(f"add_triangle_mesh: triangles must be uint32 (got {t.dtype})")
+        nv, nt = int(params.nb_vertices), int(params.nb_triangles)
+        if v.size != 3 * nv or t.size != 3 * nt:
+            raise native.DyrosError(f"add_triangle_mesh: {v.size} vertex and {t.size} triangle values for nb_vertices = "
+                                    f"{nv} and nb_triangles = {nt} (3 each)")
+        p = params.transform.p
+        tm = TriangleMesh(np.ascontiguousarray(v.reshape(nv, 3)), np.ascontiguousarray(t.reshape(nt, 3)), (p.x, p.y, p.z),
+                          friction=float(params.dynamic_friction))
+        tm.validate()
+        sim.triangle_mesh = tm
 
     def load_asset(self, sim: Sim, rootpath: str, filename: str, options: Optional[AssetOptions] = None):
         options = options or AssetOptions()
@@ -481,7 +512,8 @@ class Gym:
         sim.shape_friction[env.index] = mu
         if sim.core is not None and "contact_friction" in sim.core.sim_t:
             ground = sim.heightfield.friction if sim.heightfield is not None else (
-                sim.plane.dynamic_friction if sim.plane is not None else 1.0)
+                sim.triangle_mesh.friction if sim.triangle_mesh is not None else (
+                    sim.plane.dynamic_friction if sim.plane is not None else 1.0))
             plane = float(ground)
             sim.core.sim_t["contact_friction"][env.index] = plane * mu
         return True
@@ -543,8 +575,8 @@ class Gym:
         """vec_task.py:196: allocate the tensor-API buffers and build the native sim."""
         if sim.core is not None:
             return True
-        if sim.asset is None or not sim.envs or (sim.plane is None and sim.heightfield is None):
-            print("*** prepare_sim: need a ground (plane or heightfield), an asset and at least one env")
+        if sim.asset is None or not sim.envs or (sim.plane is None and sim.heightfield is None and sim.triangle_mesh is None):
+            print("*** prepare_sim: need a ground (plane, heightfield or triangle mesh), an asset and at least one env")
             return False
         N = len(sim.envs)
         if any(len(e.actor_names) != 1 for e in sim.envs):

@@ -49,6 +49,11 @@ class DyrosHeightField(C.Structure):
                 ("column_scale", f32), ("vertical_scale", f32), ("origin", f32 * 3)]
 
 
+class DyrosTriangleMesh(C.Structure):
+    _fields_ = [("vertices", C.c_void_p), ("triangles", C.c_void_p), ("num_vertices", C.c_int64),
+                ("num_triangles", C.c_int64), ("origin", f32 * 3), ("dynamic_friction", f32)]
+
+
 class DyrosSimBuffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in SIM_BUFFERS]
 
@@ -102,7 +107,7 @@ class DyrosTerrainCurriculum(C.Structure):
 
 class DyrosHeightScan(C.Structure):
     _fields_ = [("points", C.c_void_p), ("num_points", i32), ("base_offset", f32), ("scale", f32),
-                ("measured_heights", C.c_void_p)]
+                ("measured_heights", C.c_void_p), ("field", C.POINTER(DyrosHeightField))]
 
 
 class DyrosCriticStates(C.Structure):
@@ -178,6 +183,8 @@ SIGNATURES = {
     "dyros_flush_l2": (_INT, [C.c_void_p, C.c_size_t, _INT, C.c_void_p]),
     "dyros_sim_launch_info": (_INT, [_VP, C.POINTER(C.c_int32 * 4)]),
     "dyros_sim_set_heightfield": (_INT, [_VP, C.POINTER(DyrosHeightField)]),
+    "dyros_sim_set_triangle_mesh": (_INT, [_VP, C.POINTER(DyrosTriangleMesh)]),
+    "dyros_sim_triangle_mesh_info": (_INT, [_VP, C.POINTER(C.c_int64 * 4)]),
     "dyros_task_create": (_INT, [_VP, C.POINTER(DyrosTaskDesc), C.POINTER(DyrosTaskBuffers), C.POINTER(_VP)]),
     "dyros_task_destroy": (_INT, [_VP]),
     "dyros_task_set_noise_injection": (_INT, [_VP, C.POINTER(DyrosNoiseInjection)]),

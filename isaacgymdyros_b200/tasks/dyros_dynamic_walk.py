@@ -126,6 +126,13 @@ def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generato
     # (not a key of the reference's yaml either: its TerrainCfg, terrain_cfg.py:2-21, switched on. DESIGN.md section 4,
     # "Curriculum")
     tr = env.get("terrain")
+    # (ours: legged_gym's default mesh_type 'trimesh', where risers are vertical walls. DESIGN.md section 4,
+    # "Triangle-mesh ground")
+    mesh = env.get("terrainMesh", False)
+    if not isinstance(mesh, bool):
+        raise ValueError(f'cfg["env"]["terrainMesh"]: True or False (got {mesh!r})')
+    if mesh and hf is not None:
+        raise DyrosError('cfg["env"]["terrainMesh"]: makes the generated "terrain" the ground; it cannot go with "heightfield"')
     if tr is not None:
         tcfg = terrain_gen.TerrainConfig.from_dict(tr)
         if tcfg.mesh_type in ("plane", "none"):
@@ -134,7 +141,13 @@ def core_config_from_cfg(cfg: Dict[str, Any], generator: Optional[torch.Generato
             raise DyrosError('cfg["env"]: give either "heightfield" or "terrain", not both')
         else:
             _terrain_config(c, tcfg, int(env["numEnvs"]), generator)
+            if mesh:  # the field's trimesh is the ground; its samples still drive the height scan
+                c.triangle_mesh = terrain_gen.trimesh_from_field(c.heightfield, tcfg.slope_treshold)
+                c.heightfield = None
         c.height_scan = terrain_gen.height_points(tcfg)  # (any ground, the plane too)
+    if mesh and c.triangle_mesh is None:
+        raise DyrosError('cfg["env"]["terrainMesh"]: needs a generated terrain (cfg["env"]["terrain"] with mesh_type '
+                         "'heightfield')")
     cs = critic_states(cfg)
     if cs is not None:
         c.critic_states, c.critic_heights_in_obs = True, cs

@@ -13,7 +13,7 @@ from typing import List, Optional
 
 import numpy as np
 
-from .core import HeightField
+from .core import HeightField, TriangleMesh
 from .native import DyrosError
 
 
@@ -42,6 +42,10 @@ class TerrainConfig:
     measured_points_y: List[float] = field(default_factory=lambda: [-0.5, -0.4, -0.3, -0.2, -0.1, 0., 0.1, 0.2, 0.3,
                                                                     0.4, 0.5])
     seed: int = 0
+    # legged_gym's key (and spelling): convert_heightfield_to_trimesh moves vertices where neighbouring samples differ by
+    # more than this slope, so that risers become vertical walls; None: no moves. Used only for a mesh ground
+    # (cfg["env"]["terrainMesh"])
+    slope_treshold: Optional[float] = 0.75
 
     @classmethod
     def from_dict(cls, d: dict) -> "TerrainConfig":
@@ -139,10 +143,59 @@ def height_points(cfg: TerrainConfig) -> Optional[np.ndarray]:
     return np.ascontiguousarray(np.stack([gx.ravel(), gy.ravel()], 1), np.float32)
 
 
+def convert_heightfield_to_trimesh(height_field_raw, horizontal_scale, vertical_scale, slope_threshold=None):
+    """isaacgym's terrain_utils.convert_heightfield_to_trimesh -> (vertices (R*C, 3) float32, triangles
+    (2 (R-1)(C-1), 3) uint32). Vertex r*C + c sits at (r hs, c hs, vs h[r, c]); with slope_threshold, a vertex moves one
+    horizontal step along x (y) toward a neighbour higher by more than slope_threshold * hs / vs sample units, and along
+    the diagonal where it moved along neither, so that steep steps become vertical walls. Cell (i, j) gives the
+    triangles (i,j),(i+1,j+1),(i,j+1) and (i,j),(i+1,j),(i+1,j+1), in that order: the heightfield's diagonal split,
+    facing up."""
+    hf = np.asarray(height_field_raw).astype(np.int64)
+    nr, nc = hf.shape
+    hs = float(horizontal_scale)
+    yy, xx = np.meshgrid(np.linspace(0, (nc - 1) * hs, nc), np.linspace(0, (nr - 1) * hs, nr))
+    if slope_threshold is not None:
+        t = slope_threshold * hs / vertical_scale
+        move_x, move_y, move_c = (np.zeros((nr, nc)) for _ in range(3))
+        move_x[:nr - 1, :] += hf[1:, :] - hf[:nr - 1, :] > t
+        move_x[1:, :] -= hf[:nr - 1, :] - hf[1:, :] > t
+        move_y[:, :nc - 1] += hf[:, 1:] - hf[:, :nc - 1] > t
+        move_y[:, 1:] -= hf[:, :nc - 1] - hf[:, 1:] > t
+        move_c[:nr - 1, :nc - 1] += hf[1:, 1:] - hf[:nr - 1, :nc - 1] > t
+        move_c[1:, 1:] -= hf[:nr - 1, :nc - 1] - hf[1:, 1:] > t
+        xx = xx + (move_x + move_c * (move_x == 0)) * hs
+        yy = yy + (move_y + move_c * (move_y == 0)) * hs
+    vertices = np.zeros((nr * nc, 3), np.float32)
+    vertices[:, 0] = xx.ravel()
+    vertices[:, 1] = yy.ravel()
+    vertices[:, 2] = hf.ravel() * vertical_scale
+    i, j = np.meshgrid(np.arange(nr - 1), np.arange(nc - 1), indexing="ij")
+    i0 = (i * nc + j).ravel()
+    i1, i2 = i0 + 1, i0 + nc
+    i3 = i2 + 1
+    triangles = np.empty((2 * len(i0), 3), np.uint32)
+    triangles[0::2] = np.stack([i0, i3, i1], 1)
+    triangles[1::2] = np.stack([i0, i2, i3], 1)
+    return vertices, triangles
+
+
+def trimesh_from_field(hf: HeightField, slope_threshold) -> TriangleMesh:
+    """legged_gym's trimesh terrain: the mesh of a generated field (equal row and column scales) at the field's origin,
+    with the field's friction, and the field as the samples of the height scan."""
+    if hf.row_scale != hf.column_scale:
+        raise DyrosError(f"terrain: a trimesh needs equal row and column scales (legged_gym's horizontal_scale; got "
+                         f"{hf.row_scale}, {hf.column_scale})")
+    v, t = convert_heightfield_to_trimesh(hf.samples, hf.row_scale, hf.vertical_scale, slope_threshold)
+    return TriangleMesh(v, t, origin=tuple(hf.origin), friction=hf.friction, scan_field=hf)
+
+
 def validate(cfg: TerrainConfig):
     if cfg.mesh_type == "trimesh":
-        raise DyrosError("terrain: mesh_type 'trimesh' is not built (a triangle-mesh ground needs a general mesh narrow "
-                         "phase); use mesh_type 'heightfield'")
+        raise DyrosError("terrain: mesh_type 'trimesh' is not accepted here; use mesh_type 'heightfield' (for legged_gym's "
+                         "trimesh ground, set cfg[\"env\"][\"terrainMesh\"] = True beside it)")
+    st = cfg.slope_treshold
+    if st is not None and not (isinstance(st, (int, float)) and not isinstance(st, bool) and np.isfinite(st) and st >= 0):
+        raise DyrosError(f"terrain: slope_treshold must be a number >= 0 or None (got {st!r})")
     if cfg.mesh_type != "heightfield":
         raise DyrosError(f"terrain: nothing to generate for mesh_type {cfg.mesh_type!r} (only 'heightfield')")
     p = np.asarray(cfg.terrain_proportions, np.float64)
